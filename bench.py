@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the sampling hot path: sampled ligands/sec, 1000-step DDPM.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one complete pass of the hot path over one batch: the 1000 reverse-diffusion steps of
 KeypointDiffusion.sample_from_encoded_receptors for the workload's complexes (graph build + denoiser + posterior step
@@ -222,6 +222,38 @@ def oracle_step_time(sd, arch, kw, rec_nf, pocket, n_lig, n_timed, threads, T=10
     return total / len(timed), sum(e_ll) / max(len(e_ll), 1)
 
 
+DUMP_LIMIT_BYTES = 64_000_000          # all files of a dump, .npy headers included
+NPY_HEADER_BYTES = 1024                 # allowance per file (np.save writes 128 B for these shapes)
+
+
+def dump_outputs(out_dir, result, strong):
+    """What a caller of the timed path receives from its last timed step, as float32 .npy files in out_dir: the sampled
+    ligands' positions [atoms, 3] and atom features [atoms, F], concatenated in the order the call returns them
+    (rank-major for a weak-scaling run, receptor-major for a strong-scaling one).  The inputs depend only on the
+    arguments, so two builds run with the same arguments (--warmup and --steps included: every call writes its keypoint
+    positions back into the input graph) can be compared array for array.  Where the files would exceed
+    DUMP_LIMIT_BYTES, a fixed seeded sample of atom rows is written instead, with its row indices (rows.npy, float64)."""
+    import numpy as np
+    if strong:
+        pos = [p for rec in result for p in rec["positions"]]
+        feat = [f for rec in result for f in rec["features"]]
+    else:
+        pos, feat = result[0], result[1]
+    arrays = {"positions": torch.cat([p.cpu() for p in pos]).float(),
+              "features": torch.cat([f.cpu() for f in feat]).float()}
+    n = arrays["positions"].shape[0]
+    row_bytes = sum(a[0].numel() * 4 for a in arrays.values())
+    if n * row_bytes + 2 * NPY_HEADER_BYTES > DUMP_LIMIT_BYTES:
+        k = (DUMP_LIMIT_BYTES - 3 * NPY_HEADER_BYTES) // (row_bytes + 8)
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.double()
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a.numpy())
+
+
 def git_head():
     try:
         return subprocess.run(["git", "-C", str(ROOT), "rev-parse", "--short", "HEAD"], capture_output=True, text=True,
@@ -230,7 +262,7 @@ def git_head():
         return None
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=3)
@@ -254,7 +286,21 @@ def main():
                          "GVP only, ~2e-3)")
     ap.add_argument("--no-mode-blocks", action="store_true",
                     help="skip the separately-reported measurements of the other precision modes")
-    args = ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ligands the timed path returned in its last timed step to DIR/<name>.npy")
+    args = ap.parse_args(argv)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path; the reference arm only times fast-forwarded CPU steps")
+    if args.dump_outputs:
+        # relative to where the caller ran it: build_model() changes into the repository root before the dump
+        args.dump_outputs = str(Path(args.dump_outputs).resolve())
+    return args
+
+
+def main():
+    args = parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -338,12 +384,13 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, k):
+        """k calls of fn -> (device seconds, wall seconds, what the last call returned)."""
         barrier()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0 = time.perf_counter()
         ev0.record()
         for _ in range(k):
-            fn()
+            res = fn()
         ev1.record()
         torch.cuda.synchronize()
         wall = time.perf_counter() - t0
@@ -354,7 +401,7 @@ def main():
         if world > 1:
             import torch.distributed as dist
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t[0]), float(t[1])
+        return float(t[0]), float(t[1]), res
 
     if strong:
         # ONE fixed job: `pockets` encoded pockets x ligands/pockets sizes, dealt to the ranks by KeypointDiffusion.sample_sharded
@@ -408,8 +455,10 @@ def main():
         one_sample_device()
     clocks = ClockSampler(local_rank)
     clocks.start()
-    dt, wall = timed(one_sample_device, args.steps)
+    dt, wall, last = timed(one_sample_device, args.steps)
     clk = clocks.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, strong)     # now: the legs below re-run the samplers that own these buffers
     if strong:
         dt = max(dt, wall)          # the call ends with the gather + D2H of every rank's ligands: wall clock >= device time
     value = work * args.steps / dt
@@ -423,7 +472,7 @@ def main():
         e2e_value = value
     else:
         one_sample_e2e()
-        dt_e, wall_e = timed(one_sample_e2e, args.steps)
+        dt_e, wall_e, _ = timed(one_sample_e2e, args.steps)
         e2e_value = work * args.steps / max(dt_e, wall_e)
 
     out = {"metric": metric, "value": value, "unit": "ligands/s", "n_gpus": world, "steps": args.steps,
@@ -555,7 +604,7 @@ def main():
             k = 1 if p == "fp32" else args.steps            # the SIMT mode is slow: one timed sample
             for _ in range(1 if p == "fp32" else 2):
                 one_sample_device()
-            dtp, _ = timed(one_sample_device, k)
+            dtp, _, _ = timed(one_sample_device, k)
             out["modes"][p] = {"value": work * k / dtp, "unit": "ligands/s", "ms_per_step": dtp / k * 1e3, "steps": k,
                                "dtype": DTYPES[p], "accuracy": acc[p]}
         model.dynamics.set_precision(args.precision)
@@ -573,7 +622,7 @@ def main():
 
         for _ in range(2):
             shipped_sample()
-        dts, _ = timed(shipped_sample, args.steps)
+        dts, _, _ = timed(shipped_sample, args.steps)
         out["shipped_ll_cutoff"] = {"value": work * args.steps / dts, "unit": "ligands/s", "ms_per_step": dts / args.steps * 1e3,
                                     "ll_cutoff": cfg_s["graph"]["graph_cutoffs"]["ll"],
                                     "note": "same workload and weights at the shipped ll cutoff: the untrained model lets the "
@@ -610,4 +659,7 @@ def main():
 
 
 if __name__ == "__main__":
+    # the benchmark writes nothing into the tree: without this, importing the tests/ helpers creates tests/__pycache__
+    # (build() imports every other module it loads); set here, not at import, so that importing bench leaves the flag alone
+    sys.dont_write_bytecode = True
     main()
