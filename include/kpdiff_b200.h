@@ -142,10 +142,14 @@ typedef struct kpd_egnn_model kpd_egnn_model;
 int kpd_egnn_create(const kpd_egnn_config* cfg, const float* blob, const int64_t* offsets,
                     int32_t n_offsets, kpd_egnn_model** out);
 void kpd_egnn_destroy(kpd_egnn_model* m);
-/* Tensor-core mode of the EGNN ("bf16x3": split (hi, lo) bf16 operands on tcgen05, all four products, fp32
- * accumulation in TMEM -- inside the 1e-4 parity bar): the per-node first-layer products and the node MLPs run
- * through kpd_tc_linear(nsplit = 2), the edge stage through the warp-specialised kernel of csrc/egnn_ws.inl.
- * tc_blob / byte_offsets from pack.pack_egnn_tc.  mode: 0 = fp32 SIMT (default), 2 = bf16x3. */
+/* Tensor-core modes of the EGNN: the per-node first-layer products and the node MLPs run through
+ * kpd_tc_linear(nsplit = 2), the edge stage through the warp-specialised kernel of csrc/egnn_ws.inl.
+ *   nsplit = 2: "bf16x3", split (hi, lo) bf16 operands, all four products, fp32 accumulation in TMEM -- inside the
+ *               1e-4 parity bar -> mode 2;
+ *   nsplit = 1: "bf16", plain bf16 operands in the edge kernel (one M = 64 MMA per k-step, one-MUFU activations;
+ *               within 3e-2 of the output scale) -> mode 1, which needs the nsplit = 2 pack as well (node GEMMs).
+ * tc_blob / byte_offsets from pack.pack_egnn_tc(split = nsplit == 2); both packs stay attached side by side.
+ * mode: 0 = fp32 SIMT (default), 1 = bf16, 2 = bf16x3. */
 int kpd_egnn_attach_tc(kpd_egnn_model* m, const void* tc_blob, const int64_t* byte_offsets, int32_t n,
                        int32_t nsplit);
 int kpd_egnn_set_mode(kpd_egnn_model* m, int32_t mode);

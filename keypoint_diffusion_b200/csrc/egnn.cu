@@ -30,6 +30,7 @@
 #include "ws_common.cuh"
 #include "tc_gemm.cuh"
 #include <string.h>
+#include <type_traits>
 #include <vector>
 
 namespace kpd {
@@ -315,8 +316,8 @@ struct EgnnLayerW {
     const float* watt[4]; const float* batt[4]; const float* w3c[4];
     const float* Wn1T[2]; const float* bn1[2]; const float* Wn2T[2]; const float* bn2[2];
     const float* lnw[2]; const float* lnb[2];
-    // tensor-core mode (kpd_egnn_attach_tc): packed k-step slabs
-    const void* WpreP[2]; const uint4* W2P[4][2]; const void* Wn1P[2]; const void* Wn2P[2];
+    // tensor-core modes (kpd_egnn_attach_tc): packed k-step slabs, [nsplit - 1] = bf16 | bf16x3
+    struct Tc { const void* WpreP[2]; const uint4* W2P[4][2]; const void* Wn1P[2]; const void* Wn2P[2]; } tc[2];
 };
 
 struct kpd_egnn_model {
@@ -325,9 +326,9 @@ struct kpd_egnn_model {
     int n_et, n_upd, nslot[2];
     const float* lig_enc[4]; const float* rec_enc[4]; const float* dec[4];
     std::vector<EgnnLayerW> layers;
-    size_t edge_smem, edge_smem_ws;
-    int mode;          // 0 = fp32 SIMT, 2 = bf16x3 tcgen05 (split operands, fp32-grade)
-    bool tc2_ready;
+    size_t edge_smem, edge_smem_ws[2];      // edge_smem_ws[nsplit - 1]
+    int mode;          // 0 = fp32 SIMT, 1 = bf16 tcgen05 (plain operands), 2 = bf16x3 tcgen05 (split operands, fp32-grade)
+    bool tc_ready[2];  // [nsplit - 1]
 };
 
 struct EgnnWs {
@@ -410,39 +411,48 @@ extern "C" int kpd_egnn_create(const kpd_egnn_config* cfg, const float* blob, co
     cudaError_t e = cudaFuncSetAttribute(egnn_edge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->edge_smem);
     if (e != cudaSuccess) { const size_t sm = m->edge_smem; delete m; KPD_REQUIRE(false, "kpd_egnn_create: cannot set %zu B shared memory: %s", sm, cudaGetErrorString(e)); }
     m->mode = 0;
-    m->tc2_ready = false;
-    m->edge_smem_ws = egws::smem_bytes(2 * cdiv(m->H, 16));
+    m->tc_ready[0] = m->tc_ready[1] = false;
+    m->edge_smem_ws[0] = egws::smem_bytes<1>(2 * cdiv(m->H, 16));
+    m->edge_smem_ws[1] = egws::smem_bytes<2>(2 * cdiv(m->H, 16));
     *out = m;
     return 0;
 }
 
 extern "C" void kpd_egnn_destroy(kpd_egnn_model* m) { delete m; }
 
-// Tensor-core mode ("bf16x3": split (hi, lo) bf16 operands, fp32-grade): tc_blob holds, per layer, the packed
-// (pack.pack_tc_weight(split=True)) weights  Wpre[lig], Wpre[kp]; per edge type W2 of edge_mlp and coord_mlp (rows
-// [0, nmain)); per updated node type node_mlp.0 and node_mlp.2 -- pack.pack_egnn_tc.
+// Tensor-core modes (nsplit = 1: "bf16", plain bf16 operands; nsplit = 2: "bf16x3", split (hi, lo) bf16 operands,
+// fp32-grade): tc_blob holds, per layer, the packed (pack.pack_tc_weight(split = nsplit == 2)) weights  Wpre[lig],
+// Wpre[kp]; per edge type W2 of edge_mlp and coord_mlp (rows [0, nmain)); per updated node type node_mlp.0 and
+// node_mlp.2 -- pack.pack_egnn_tc.  The two packs are kept side by side: set_mode switches between them.
 extern "C" int kpd_egnn_attach_tc(kpd_egnn_model* m, const void* tc_blob, const int64_t* byte_offsets, int32_t n, int32_t nsplit) {
     KPD_REQUIRE(m && tc_blob && byte_offsets, "kpd_egnn_attach_tc: null argument");
-    KPD_REQUIRE(nsplit == 2, "kpd_egnn_attach_tc: only nsplit = 2 (bf16x3) is implemented for the EGNN");
+    KPD_REQUIRE(nsplit == 1 || nsplit == 2, "kpd_egnn_attach_tc: nsplit must be 1 (bf16) or 2 (bf16x3)");
     const int per_layer = 2 + m->n_et * 2 + m->n_upd * 2;
     KPD_REQUIRE(n == m->cfg.n_layers * per_layer, "kpd_egnn_attach_tc: expected %d offsets, got %d", m->cfg.n_layers * per_layer, n);
     KPD_REQUIRE((reinterpret_cast<uintptr_t>(tc_blob) & 127) == 0, "kpd_egnn_attach_tc: blob must be 128-byte aligned");
     KPD_REQUIRE(m->nmain % 8 == 0 && m->H <= 257, "kpd_egnn_attach_tc: hidden width %d unsupported by the tensor-core tiles", m->H);
-    KPD_REQUIRE(m->edge_smem_ws <= 227 * 1024, "kpd_egnn_attach_tc: tile needs %zu B of shared memory", m->edge_smem_ws);
+    const size_t smem = m->edge_smem_ws[nsplit - 1];
+    KPD_REQUIRE(smem <= 227 * 1024, "kpd_egnn_attach_tc: tile needs %zu B of shared memory", smem);
     const char* base = static_cast<const char*>(tc_blob);
     int i = 0;
     auto P = [&](void) -> const void* { return base + byte_offsets[i++]; };
     for (int l = 0; l < m->cfg.n_layers; ++l) {
-        EgnnLayerW& L = m->layers[l];
-        for (int nt = 0; nt < 2; ++nt) L.WpreP[nt] = P();
+        EgnnLayerW::Tc& T = m->layers[l].tc[nsplit - 1];
+        for (int nt = 0; nt < 2; ++nt) T.WpreP[nt] = P();
         for (int e = 0; e < m->n_et; ++e)
-            for (int br = 0; br < 2; ++br) L.W2P[e][br] = static_cast<const uint4*>(P());
-        for (int nt = 0; nt < m->n_upd; ++nt) { L.Wn1P[nt] = P(); L.Wn2P[nt] = P(); }
+            for (int br = 0; br < 2; ++br) T.W2P[e][br] = static_cast<const uint4*>(P());
+        for (int nt = 0; nt < m->n_upd; ++nt) { T.Wn1P[nt] = P(); T.Wn2P[nt] = P(); }
     }
-    cudaError_t e = cudaFuncSetAttribute(egnn_edge_ws_kernel<257>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->edge_smem_ws);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(egnn_edge_ws_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->edge_smem_ws);
-    KPD_REQUIRE(e == cudaSuccess, "kpd_egnn_attach_tc: cannot set %zu B shared memory: %s", m->edge_smem_ws, cudaGetErrorString(e));
-    m->tc2_ready = true;
+    cudaError_t e;
+    if (nsplit == 1) {
+        e = cudaFuncSetAttribute(egnn_edge_ws_kernel<257, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(egnn_edge_ws_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    } else {
+        e = cudaFuncSetAttribute(egnn_edge_ws_kernel<257, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(egnn_edge_ws_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    }
+    KPD_REQUIRE(e == cudaSuccess, "kpd_egnn_attach_tc: cannot set %zu B shared memory: %s", smem, cudaGetErrorString(e));
+    m->tc_ready[nsplit - 1] = true;
     return 0;
 }
 
@@ -459,8 +469,9 @@ extern "C" int kpd_debug_eg_times(unsigned long long* out16) {
 
 extern "C" int kpd_egnn_set_mode(kpd_egnn_model* m, int32_t mode) {
     KPD_REQUIRE(m, "kpd_egnn_set_mode: null model");
-    KPD_REQUIRE(mode == 0 || mode == 2, "kpd_egnn_set_mode: mode must be 0 (fp32 SIMT) or 2 (bf16x3 tensor cores)");
-    KPD_REQUIRE(mode != 2 || m->tc2_ready, "kpd_egnn_set_mode: call kpd_egnn_attach_tc first");
+    KPD_REQUIRE(mode >= 0 && mode <= 2, "kpd_egnn_set_mode: mode must be 0 (fp32 SIMT), 1 (bf16) or 2 (bf16x3 tensor cores)");
+    KPD_REQUIRE(mode == 0 || (m->tc_ready[mode - 1] && m->tc_ready[1]),
+                "kpd_egnn_set_mode: mode %d needs kpd_egnn_attach_tc(nsplit = 2)%s first", mode, mode == 1 ? " and (nsplit = 1)" : "");
     m->mode = mode;
     return 0;
 }
@@ -535,13 +546,18 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
 
     for (int l = 0; l < m->cfg.n_layers; ++l) {
         const EgnnLayerW& W = m->layers[l];
+        // edge kernel: the mode's own pack (nsplit = mode).  Node GEMMs: split operands in both tensor-core modes --
+        // tc_linear<1> takes 128 rows per CTA, half the CTAs of tc_linear<2>, and at a sampling batch's node counts
+        // that left the GPU idle (egnn_20kp 72 -> 49 ligands/s on B200 with nsplit = 1 here, DESIGN.md 4.1)
+        const EgnnLayerW::Tc& T = W.tc[m->mode == 1 ? 0 : 1];
+        const EgnnLayerW::Tc& TN = W.tc[1];
         prof_begin(PROF_EGNN_PRE, st);
-        if (m->mode == 2) {       // both node types in one launch
+        if (m->mode != 0) {       // both node types in one launch
             TcLinBatch TB;
             memset(&TB, 0, sizeof(TB));
             for (int nt = 0; nt < 2; ++nt) {
                 const int ncol = m->nslot[nt] * Hp;
-                TB.p[nt] = tc_problem(w.h[nt], Hp, W.WpreP[nt], W.bpre[nt], nullptr, 0, w.P[nt], ncol, N[nt], H, ncol, 0);
+                TB.p[nt] = tc_problem(w.h[nt], Hp, TN.WpreP[nt], W.bpre[nt], nullptr, 0, w.P[nt], ncol, N[nt], H, ncol, 0);
             }
             KPD_TRY(launch_tc_batch(TB, 2, 2, st));
         } else {
@@ -566,17 +582,24 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
             a.hn = w.hn[e]; a.xn = w.xn[e]; a.part = w.part[e];
         }
         prof_begin(PROF_EGNN_EDGE, st);
-        if (m->mode == 2) {
+        if (m->mode != 0) {
             EgnnWsLaunch WL;
             memset(&WL, 0, sizeof(WL));
             WL.L = L;
             WL.kch = 2 * cdiv(H, 16);
             for (int e = 0; e < m->n_et; ++e)
-                for (int br = 0; br < 2; ++br) WL.t[e].W2P[br] = W.W2P[e][br];
+                for (int br = 0; br < 2; ++br) WL.t[e].W2P[br] = T.W2P[e][br];
             for (int e = 0; e < 4; ++e) WL.tile_off[e + 1] = WL.tile_off[e] + (e < m->n_et ? cdiv(caps[e] > 0 ? caps[e] : 1, egws::R) : 0);
             // (the constants the kernel derives from HS = 257 are exactly what this function passes for H = 257)
-            if (H == 257) egnn_edge_ws_kernel<257><<<dim3(WL.tile_off[4]), egws::NT, m->edge_smem_ws, st>>>(WL);
-            else egnn_edge_ws_kernel<0><<<dim3(WL.tile_off[4]), egws::NT, m->edge_smem_ws, st>>>(WL);
+            const dim3 grid(WL.tile_off[4]);
+            const size_t smem = m->edge_smem_ws[m->mode - 1];
+            if (m->mode == 1) {
+                if (H == 257) egnn_edge_ws_kernel<257, 1><<<grid, egws::NT, smem, st>>>(WL);
+                else egnn_edge_ws_kernel<0, 1><<<grid, egws::NT, smem, st>>>(WL);
+            } else {
+                if (H == 257) egnn_edge_ws_kernel<257, 2><<<grid, egws::NT, smem, st>>>(WL);
+                else egnn_edge_ws_kernel<0, 2><<<grid, egws::NT, smem, st>>>(WL);
+            }
             KPD_TRY(check_launch("egnn_edge_ws_kernel"));
         } else {
             egnn_edge_kernel<<<dim3(max_tiles, m->n_et), NT, m->edge_smem, st>>>(L);
@@ -586,7 +609,7 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
         prof_begin(PROF_EGNN_NODE, st);
 
         // tensor-core mode: h_neigh starts at the 4-aligned column Hp of the cat row (zero gap [H, Hp))
-        const int off_neigh = m->mode == 2 ? Hp : H;
+        const int off_neigh = m->mode != 0 ? Hp : H;
         const int ldcat = (off_neigh + H + 3) & ~3;
         EgnnNodePrepPair NP;
         memset(&NP, 0, sizeof(NP));
@@ -604,12 +627,12 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
             a.z_const = m->cfg.message_norm;
             a.node_batch = nt == 0 ? b->lig_batch : b->kp_batch;
             a.ptr = nt == 0 ? b->lig_ptr : b->kp_ptr;
-            if (a.n > 0 && m->mode != 2) {
+            if (a.n > 0 && m->mode == 0) {
                 egnn_node_prep_kernel<<<a.n, 128, 0, st>>>(a);
                 KPD_TRY(check_launch("egnn_node_prep_kernel"));
             }
         }
-        if (m->mode == 2) {
+        if (m->mode != 0) {
             const int blocks0 = cdiv(NP.a[0].n > 0 ? NP.a[0].n : 0, 8), blocks1 = m->n_upd > 1 ? cdiv(NP.a[1].n > 0 ? NP.a[1].n : 0, 8) : 0;
             if (blocks0 + blocks1 > 0) {
                 egnn_node_prep_pair_kernel<<<blocks0 + blocks1, 256, 0, st>>>(NP, off_neigh, blocks0);
@@ -617,27 +640,27 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
             }
         }
         // node_mlp = Linear(2H,H), SiLU, Linear(H,H); residual; LayerNorm  (:202-205)
-        if (m->mode == 2) {       // all updated node types in one launch per Linear
+        if (m->mode != 0) {       // all updated node types in one launch per Linear
             TcLinBatch T1, T2;
             memset(&T1, 0, sizeof(T1));
             memset(&T2, 0, sizeof(T2));
             for (int nt = 0; nt < m->n_upd; ++nt) {
-                T1.p[nt] = tc_problem(w.cat[nt], ldcat, W.Wn1P[nt], W.bn1[nt], nullptr, 0, w.tmp1[nt], Hp, N[nt], off_neigh + H, H, 1);
-                T2.p[nt] = tc_problem(w.tmp1[nt], Hp, W.Wn2P[nt], W.bn2[nt], w.h[nt], Hp, w.y[nt], Hp, N[nt], H, H, 0);
+                T1.p[nt] = tc_problem(w.cat[nt], ldcat, TN.Wn1P[nt], W.bn1[nt], nullptr, 0, w.tmp1[nt], Hp, N[nt], off_neigh + H, H, 1);
+                T2.p[nt] = tc_problem(w.tmp1[nt], Hp, TN.Wn2P[nt], W.bn2[nt], w.h[nt], Hp, w.y[nt], Hp, N[nt], H, H, 0);
             }
             KPD_TRY(launch_tc_batch(T1, m->n_upd, 2, st));
             KPD_TRY(launch_tc_batch(T2, m->n_upd, 2, st));
         }
         for (int nt = 0; nt < m->n_upd; ++nt) {
-            if (m->mode != 2) {
+            if (m->mode == 0) {
                 KPD_TRY(launch_linear(w.cat[nt], ldcat, W.Wn1T[nt], Hp, W.bn1[nt], nullptr, 0, w.tmp1[nt], Hp, N[nt], 2 * H, H, 1, st));
                 KPD_TRY(launch_linear(w.tmp1[nt], Hp, W.Wn2T[nt], Hp, W.bn2[nt], w.h[nt], Hp, w.y[nt], Hp, N[nt], H, H, 0, st));
             }
-            if (m->cfg.norm && m->mode == 2) continue;      // (one launch for all node types below)
+            if (m->cfg.norm && m->mode != 0) continue;      // (one launch for all node types below)
             if (m->cfg.norm) KPD_TRY(launch_layernorm(w.y[nt], Hp, w.h[nt], Hp, N[nt], H, W.lnw[nt], W.lnb[nt], st));
             else KPD_TRY(launch_copy_rows(w.y[nt], Hp, w.h[nt], Hp, N[nt], H, st));
         }
-        if (m->cfg.norm && m->mode == 2) {
+        if (m->cfg.norm && m->mode != 0) {
             const bool two = m->n_upd > 1;
             KPD_TRY(launch_layernorm_pair(w.y[0], w.h[0], N[0], W.lnw[0], W.lnb[0], two ? w.y[1] : nullptr, two ? w.h[1] : nullptr,
                                           two ? N[1] : 0, two ? W.lnw[1] : nullptr, two ? W.lnb[1] : nullptr, Hp, Hp, H, st));

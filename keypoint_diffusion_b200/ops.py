@@ -246,6 +246,7 @@ class EgnnModel(_Model):
             raise RuntimeError("EgnnModel needs a CUDA device (no CPU fallback)")
         self.update_kp_feat = bool(update_kp_feat)
         self.atom_nf, self.rec_nf, self.hidden_nf = atom_nf, rec_nf, hidden_nf
+        self.n_layers = n_layers
         has_rec = "rec_encoder.0.weight" in sd
         self.blob, offs = pack.pack_egnn(sd, atom_nf=atom_nf, rec_nf=rec_nf, hidden_nf=hidden_nf, n_layers=n_layers,
                                          update_kp_feat=update_kp_feat, norm=norm, device=self.device)
@@ -255,21 +256,33 @@ class EgnnModel(_Model):
         arr = (C.c_int64 * len(offs))(*offs)
         check(lib.kpd_egnn_create(C.byref(cfg), ptr(self.blob), arr, len(offs), C.byref(self.handle)), "kpd_egnn_create")
         self.precision = "fp32"
-        self.tc_blob2 = None
+        self.tc_blob = self.tc_blob2 = None
+        self._sd_bf16 = None
         H = hidden_nf + 1
         if (min(H, 256) // 4 * 4) % 8 == 0 and H <= 257:
-            self.tc_blob2, toffs = pack.pack_egnn_tc(sd, hidden_nf=hidden_nf, n_layers=n_layers,
-                                                     update_kp_feat=update_kp_feat, device=self.device, split=True)
-            tarr = (C.c_int64 * len(toffs))(*toffs)
-            check(lib.kpd_egnn_attach_tc(self.handle, ptr(self.tc_blob2), tarr, len(toffs), 2), "kpd_egnn_attach_tc")
+            self.tc_blob2 = self._attach_tc(sd, split=True)
+            # the plain-bf16 pack is built on the first set_precision('bf16') (from a reference to sd, not a copy): a
+            # model that never uses that mode costs no more to create and holds no more packed weights
+            self._sd_bf16 = sd
 
-    PRECISIONS = {"fp32": 0, "bf16x3": 2}
+    PRECISIONS = {"fp32": 0, "bf16": 1, "bf16x3": 2}
+
+    def _attach_tc(self, sd, split: bool) -> torch.Tensor:
+        blob, toffs = pack.pack_egnn_tc(sd, hidden_nf=self.hidden_nf, n_layers=self.n_layers,
+                                        update_kp_feat=self.update_kp_feat, device=self.device, split=split)
+        tarr = (C.c_int64 * len(toffs))(*toffs)
+        check(lib.kpd_egnn_attach_tc(self.handle, ptr(blob), tarr, len(toffs), 2 if split else 1), "kpd_egnn_attach_tc")
+        return blob
 
     def set_precision(self, precision: str):
-        """'fp32' (SIMT, the reference's arithmetic) or 'bf16x3' (tcgen05 tensor cores with split bf16 operands:
-        fp32-grade, inside the 1e-4 parity bar)."""
+        """'fp32' (SIMT, the reference's arithmetic), 'bf16x3' (tcgen05 tensor cores with split bf16 operands:
+        fp32-grade, inside the 1e-4 parity bar) or 'bf16' (tcgen05, plain bf16 operands in the edge kernel: faster,
+        within 3e-2 of the fp32 output scale)."""
         if precision not in self.PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(self.PRECISIONS)}, got {precision!r}")
+        if precision == "bf16" and self.tc_blob is None and self.tc_blob2 is not None:
+            self.tc_blob = self._attach_tc(self._sd_bf16, split=False)
+            self._sd_bf16 = None
         check(lib.kpd_egnn_set_mode(self.handle, self.PRECISIONS[precision]), "kpd_egnn_set_mode")
         self.precision = precision
 
