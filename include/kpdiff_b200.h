@@ -208,7 +208,9 @@ int kpd_gvp_dims(const kpd_gvp_model* m, int* n_kp_scalars, int* vector_size);
  *               operands, meets the 1e-4 parity bar on the tensor cores.  The edge kernel keeps hi and lo PLANES of a
  *               128-row tile and issues THREE MMAs per k-step (hi*hi + lo*hi + hi*lo); the node / head kernels stack the
  *               hi and lo rows of 64 tile rows into one 128-row operand and issue TWO (x W_hi, x W_lo: all four
- *               products).  KPD_GVP_EDGE=stack at model creation selects the stacked layout for the edge kernel too.
+ *               products).  When the edge tile of hi / lo planes does not fit in 227 KB of shared memory, the
+ *               edge kernel uses the stacked layout too; of the accepted configurations only n_hidden_scalars = 256,
+ *               vector_size = 16, rbf_dim = 32 (a 305-column first message GVP input) is that wide.
  * mode: 0 = fp32 SIMT (reference arithmetic), 1 = bf16, 2 = bf16x3. */
 int kpd_gvp_attach_tc(kpd_gvp_model* m, const void* tc_blob, const int64_t* byte_offsets, int32_t n,
                       int32_t nsplit);

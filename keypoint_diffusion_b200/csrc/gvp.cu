@@ -384,25 +384,17 @@ __global__ void __launch_bounds__(NT, 1) gvp_head_kernel(const GvpHeadArgs a) {
 
 using namespace kpd;
 
-// launch with thread-block clusters of `cl` CTAs along x (grid.x is rounded up to a multiple of cl)
+// launch, optionally with the highest stream priority as a launch attribute
 template <typename Arg>
-static void launch_clustered(void (*kernel)(Arg), dim3 grid, int threads, size_t smem, cudaStream_t st, int cl, const Arg& arg,
-                             bool high_priority = false) {
-    grid.x = (grid.x + cl - 1) / cl * cl;
+static void launch_with_priority(void (*kernel)(Arg), dim3 grid, int threads, size_t smem, cudaStream_t st, const Arg& arg,
+                                 bool high_priority = false) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(threads);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     int na = 0;
-    if (cl > 1) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = cl;
-        attr[na].val.clusterDim.y = 1;
-        attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
     if (high_priority) {        // explicit, so that a captured kernel node carries it whatever the stream's priority
         int pr_lo = 0, pr_hi = 0;
         cudaDeviceGetStreamPriorityRange(&pr_lo, &pr_hi);
@@ -430,9 +422,8 @@ struct kpd_gvp_model {
     GvpW head[MAXG];
     const float* WoT; const float* bo;
     size_t smem, smem_node, smem_ws1, smem_ws2, smem_ws1n, smem_ks;
-    bool edge_ks;       // bf16x3: the edge kernel keeps (hi, lo) planes of 128-row tiles (WsKS); KPD_GVP_EDGE=stack selects the
-                        // 64-row stacked-operand kernel (WsSplit) instead
-    bool edge_pair;     // bf16x3: the edge kernel runs as CTA pairs (message GVP weights pair-packed, pack.pack_gvp_tc)
+    bool edge_ks;       // bf16x3: the edge kernel keeps (hi, lo) planes of 128-row tiles (WsKS) when that tile fits in 227 KB
+                        // of shared memory, and runs the 64-row stacked-operand kernel (WsSplit) otherwise
     int kch;           // k-chunks of the bf16 tile (tensor-core mode)
     int mode;          // 0 = fp32 SIMT, 1 = bf16 tcgen05, 2 = bf16x3 tcgen05 (split operands, fp32-grade)
     bool tc_ready, tc2_ready;
@@ -553,14 +544,9 @@ extern "C" int kpd_gvp_create(const kpd_gvp_config* cfg, const float* blob, cons
         m->kch = 2 * ((wmax + 15) / 16);
         m->smem_ws1 = ws::smem_bytes<WsBf16>(m->kch);
         m->smem_ws2 = ws::smem_bytes<WsSplit>(m->kch);
-#ifdef KPD_EDGE_PAIR      // experimental (slower, see DESIGN.md 4.3): needs pack_gvp_tc(..., pair=True), i.e. KPD_EDGE_PAIR=1 at run time
-        m->edge_pair = m->cfg.n_hidden_scalars % 32 == 0;
-#else
-        m->edge_pair = false;
-#endif
         m->smem_ws1n = ws::smem_bytes<WsBf16N>(m->kch);
         m->smem_ks = ws::smem_bytes<WsKS>(m->kch);
-        { const char* e = getenv("KPD_GVP_EDGE"); m->edge_ks = !(e && e[0] == 's') && m->smem_ks <= 227 * 1024 && !m->edge_pair; }
+        m->edge_ks = m->smem_ks <= 227 * 1024;
         m->mode = 0;
         m->tc_ready = false;
         m->tc2_ready = false;
@@ -634,7 +620,6 @@ extern "C" int kpd_gvp_attach_tc(kpd_gvp_model* m, const void* tc_blob, const in
     }
     if (nsplit == 2) {
         cudaError_t e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsSplit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsSplitPair>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
         if (e == cudaSuccess && m->edge_ks) e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsKS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ks);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_node_ws_kernel<WsSplit, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_head_ws_kernel<WsSplit, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
@@ -790,7 +775,7 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
     // 650 edge tiles are 4.4 waves of one CTA per SM and its node tiles a fifth of a wave; as separate launches their
     // tails leave SMs idle, as a graph the tail of one kernel is filled with the CTAs of the next ready one.
     // The CUDA-event profiler (bench.py's roofline leg) and KPD_GVP_SERIAL=1 use the serial path below.
-    const bool dag = m->mode != 0 && !m->serial && !prof_enabled() && !m->edge_pair;
+    const bool dag = m->mode != 0 && !m->serial && !prof_enabled();
     if (dag) KPD_TRY(gvp_dag_init(m));       // normally done by kpd_gvp_attach_tc, outside any stream capture
     // stream of edge type e (ll, kl, lk, kk) and of node type nt
     cudaStream_t es[4] = {st, st, st, st}, ns[2] = {st, st};
@@ -812,10 +797,9 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
         a.sm = w.sm[cur][e]; a.vm = w.vm[cur][e]; a.part = w.part[cur][e];
     };
     auto launch_edge_ws = [&](const GvpEdgeLaunch& L, int tiles, int n_et, cudaStream_t s_) -> int {
-        if (m->mode == 1) launch_clustered(gvp_edge_ws_kernel<WsBf16>, dim3(tiles, n_et), WsBf16::NT, m->smem_ws1, s_, WsBf16::CL, L);
-        else if (m->edge_ks) launch_clustered(gvp_edge_ws_kernel<WsKS>, dim3(tiles, n_et), WsKS::NT, m->smem_ks, s_, 1, L);
-        else if (m->edge_pair) launch_clustered(gvp_edge_ws_kernel<WsSplitPair>, dim3(tiles, n_et), WsSplitPair::NT, m->smem_ws2, s_, 2, L);
-        else launch_clustered(gvp_edge_ws_kernel<WsSplit>, dim3(tiles, n_et), WsSplit::NT, m->smem_ws2, s_, WsSplit::CL, L);
+        if (m->mode == 1) launch_with_priority(gvp_edge_ws_kernel<WsBf16>, dim3(tiles, n_et), WsBf16::NT, m->smem_ws1, s_, L);
+        else if (m->edge_ks) launch_with_priority(gvp_edge_ws_kernel<WsKS>, dim3(tiles, n_et), WsKS::NT, m->smem_ks, s_, L);
+        else launch_with_priority(gvp_edge_ws_kernel<WsSplit>, dim3(tiles, n_et), WsSplit::NT, m->smem_ws2, s_, L);
         return check_launch("gvp_edge_ws_kernel");
     };
     auto fill_node = [&](GvpNodeLaunch& NL, int slot, int nt, const GvpLayerW& W, int cur, int nxt) {
@@ -844,11 +828,11 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
     auto launch_node_ws = [&](const GvpNodeLaunch& NL, int max_n, int n_dst, cudaStream_t s_) -> int {
         const dim3 grid(cdiv(max_n, node_rows), n_dst);
         if (m->mode == 1) {
-            if (full_node_tiles) launch_clustered(gvp_node_ws_kernel<WsBf16N, NODE_ROWS_FULL>, grid, WsBf16N::NT, m->smem_ws1n, s_, WsBf16N::CL, NL, dag);
-            else launch_clustered(gvp_node_ws_kernel<WsBf16N, NODE_ROWS>, grid, WsBf16N::NT, m->smem_ws1n, s_, WsBf16N::CL, NL, dag);
+            if (full_node_tiles) launch_with_priority(gvp_node_ws_kernel<WsBf16N, NODE_ROWS_FULL>, grid, WsBf16N::NT, m->smem_ws1n, s_, NL, dag);
+            else launch_with_priority(gvp_node_ws_kernel<WsBf16N, NODE_ROWS>, grid, WsBf16N::NT, m->smem_ws1n, s_, NL, dag);
         } else {
-            if (full_node_tiles) launch_clustered(gvp_node_ws_kernel<WsSplit, NODE_ROWS_FULL>, grid, WsSplit::NT, m->smem_ws2, s_, WsSplit::CL, NL, dag);
-            else launch_clustered(gvp_node_ws_kernel<WsSplit, NODE_ROWS>, grid, WsSplit::NT, m->smem_ws2, s_, WsSplit::CL, NL, dag);
+            if (full_node_tiles) launch_with_priority(gvp_node_ws_kernel<WsSplit, NODE_ROWS_FULL>, grid, WsSplit::NT, m->smem_ws2, s_, NL, dag);
+            else launch_with_priority(gvp_node_ws_kernel<WsSplit, NODE_ROWS>, grid, WsSplit::NT, m->smem_ws2, s_, NL, dag);
         }
         return check_launch("gvp_node_ws_kernel");
     };
@@ -946,12 +930,12 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
             prof_begin(PROF_GVP_HEAD, st);
             a.kch = m->kch;
             if (m->mode == 1) {
-                if (full_node_tiles) launch_clustered(gvp_head_ws_kernel<WsBf16N, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, WsBf16N::CL, a);
-                else launch_clustered(gvp_head_ws_kernel<WsBf16N, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, WsBf16N::CL, a);
+                if (full_node_tiles) launch_with_priority(gvp_head_ws_kernel<WsBf16N, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, a);
+                else launch_with_priority(gvp_head_ws_kernel<WsBf16N, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, a);
                 KPD_TRY(check_launch("gvp_head_ws_kernel"));
             } else if (m->mode == 2) {
-                if (full_node_tiles) launch_clustered(gvp_head_ws_kernel<WsSplit, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, WsSplit::CL, a);
-                else launch_clustered(gvp_head_ws_kernel<WsSplit, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, WsSplit::CL, a);
+                if (full_node_tiles) launch_with_priority(gvp_head_ws_kernel<WsSplit, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, a);
+                else launch_with_priority(gvp_head_ws_kernel<WsSplit, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, a);
                 KPD_TRY(check_launch("gvp_head_ws_kernel"));
             } else {
                 gvp_head_kernel<<<cdiv(a.n, TN), NT, m->smem_node, st>>>(a);

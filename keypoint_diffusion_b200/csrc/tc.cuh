@@ -58,37 +58,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                  : "memory");
 }
 
-// ------------------------------------------------------------------ thread-block clusters
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-// all threads of all CTAs of the cluster
-__device__ __forceinline__ void cluster_sync() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// address of the same shared-memory location in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t map_to_cta(const void* p, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
-    return r;
-}
-// same without release ordering: for a thread that only forwards a completion it has observed (the release form
-// waits for the SM's in-flight bulk-copy writes and serialises a pipelined ring: measured)
-__device__ __forceinline__ void mbar_arrive_remote_relaxed(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// bulk copy global -> the same shared-memory offset of every CTA in cta_mask; complete_tx on the mbarrier at the same
-// offset in each of them
-__device__ __forceinline__ void bulk_g2s_multicast(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
-}
-
 // ------------------------------------------------------------------ TMEM
 // one full warp executes these (.sync.aligned)
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_slot, uint32_t ncols) {
@@ -169,59 +138,6 @@ __device__ __forceinline__ void mma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// same, arriving on the mbarrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void mma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)),
-                 "h"(cta_mask)
-                 : "memory");
-}
-
-// ------------------------------------------------------------------ CTA pairs (cta_group::2)
-// Two CTAs of a 2-CTA cluster (one TPC) run ONE M = 256 MMA: each CTA supplies its own 128 A rows and HALF of the B rows
-// (N / 2) from the same shared-memory offsets, and receives its 128 accumulator rows in its own TMEM.  Only the
-// leader (cluster rank 0) issues; descriptors are the leader's.
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_slot, uint32_t ncols) {      // one warp in EACH CTA
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols)
-                 : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() { asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::); }
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols));
-}
-__device__ __forceinline__ void mma_bf16_ss_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}\n" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// arrive on the mbarrier at this offset in every CTA of cta_mask when the pair's MMAs issued so far have completed
-__device__ __forceinline__ void mma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)),
-                 "h"(cta_mask)
-                 : "memory");
-}
-// wait on a local mbarrier that threads of the peer CTA arrive on (cluster-scope acquire)
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t"
-            "}\n"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-    }
-}
-
 // ------------------------------------------------------------------ TMEM -> registers
 // warp w may touch TMEM lanes [32*(w%4), 32*(w%4)+32); thread i gets lane base+i, 32 consecutive columns
 __device__ __forceinline__ void tmem_ld_x32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -233,15 +149,6 @@ __device__ __forceinline__ void tmem_ld_x32(uint32_t taddr, uint32_t (&v)[32]) {
           "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
           "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
           "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_x16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
         : "r"(taddr)
         : "memory");
 }
@@ -297,12 +204,6 @@ __device__ __forceinline__ void tmem_st_x16(uint32_t taddr, const uint32_t (&v)[
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// ------------------------------------------------------------------ canonical-layout addressing
-// byte offset of element (r, k) of an R-row bf16 tile (see the header comment)
-__device__ __forceinline__ uint32_t canon_off(int r, int k, int kchunk_stride) {
-    return (uint32_t)((k >> 3) * kchunk_stride + (r >> 3) * 128 + (r & 7) * 16 + (k & 7) * 2);
-}
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);

@@ -43,7 +43,7 @@ __device__ unsigned long long g_tcg_times[16];
 
 template <int NS>
 __global__ void __launch_bounds__(TCG_THREADS, 1) tc_linear_kernel(const __grid_constant__ TcLinBatch B) {
-    using C = ws::Cfg<128 / NS, NS, 1>;
+    using C = ws::Cfg<128 / NS, NS>;
     const TcLinProblem& P = B.p[blockIdx.z];
     const int M = P.M, K = P.K, N = P.N;
     const int m0 = blockIdx.x * C::R;
@@ -329,7 +329,7 @@ __global__ void __launch_bounds__(TCG_THREADS, 1) tc_linear_kernel(const __grid_
 
 template <int NS>
 static size_t tc_linear_smem(int K, int NB, int stages) {
-    using C = ws::Cfg<128 / NS, NS, 1>;
+    using C = ws::Cfg<128 / NS, NS>;
     const int ksteps = (K + 15) / 16;
     return (((size_t)2 * ksteps * C::KCS + 127) & ~(size_t)127) + (size_t)stages * NS * 2 * (NB / 8) * 128 + (2 * TCG_MAX_STAGES + 5) * 8 + 16;
 }

@@ -30,22 +30,18 @@ template <int NS> constexpr int wsm_floats() { return NS * (WH_SZ + WU_SZ) + 256
 //         the lo x lo product is below the fp32 rounding of the sum) into ONE accumulator -- a weight slab streamed
 //         from L2 serves 128 tile rows instead of 64 (the slab stream is what bounds the k-step rate, DESIGN.md 4.3),
 //         3 instead of 4 tensor-core MACs per algorithmic MAC, half the TMEM read traffic per tile row.
-template <int R_, int NS_, int CL_, int NWX_ = 0, bool KS_ = false>
+template <int R_, int NS_, int NWX_ = 0, bool KS_ = false>
 struct Cfg {
     static constexpr int R = R_, NS = NS_;
     static constexpr bool KS = KS_ && NS_ == 2;
     static constexpr bool STACK = NS_ == 2 && !KS_;
-    static constexpr int CL = CL_;                   // CTAs per cluster: neighbouring tiles share ONE weight stream (multicast)
     static constexpr int NWV = R / 8;                // vector-owning SIMT warps: 8 tile rows each (mma.sync fragments)
     static constexpr int NW = NWV + NWX_;            // all SIMT warps; the NWX extra ones only help with the epilogues,
                                                      // gathers and reductions (more warps in flight per SM quadrant)
     static constexpr int NT_SIMT = 32 * NW;
     static constexpr int NT = NT_SIMT + 64;
     static constexpr int MMA_M = STACK ? 2 * R : R;  // STACK: the hi and lo rows of a tile form ONE 128-row A operand
-#ifndef KPD_KCS_PAD
-#define KPD_KCS_PAD 16
-#endif
-    static constexpr int KCS = (MMA_M / 8) * 128 + KPD_KCS_PAD;   // bytes between k-chunks of A (+16: bank rotation for column walks)
+    static constexpr int KCS = (MMA_M / 8) * 128 + 16;   // bytes between k-chunks of A (+16: bank rotation for column walks)
     static constexpr int STAGES = NS == 1 ? 8 : 4;
     static constexpr int SLAB = NS * 8192;           // one ring stage: one k-step of a 256-row weight (hi [, lo])
     static constexpr int WG_BYTES = NS * 8192;       // gates weight: 16 k-steps x 512 B (hi [, lo])

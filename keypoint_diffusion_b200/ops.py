@@ -5,7 +5,6 @@ torch is used for device memory and streams only; every computation below is a c
 libkpdiff_b200.so.  All tensors must live on one CUDA device (no CPU fallback).
 """
 import ctypes as C
-import os
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
 
@@ -347,9 +346,7 @@ class GvpModel(_Model):
             self.tc_blob, toffs = pack.pack_gvp_tc(sd, **kw)
             tarr = (C.c_int64 * len(toffs))(*toffs)
             check(lib.kpd_gvp_attach_tc(self.handle, ptr(self.tc_blob), tarr, len(toffs), 1), "kpd_gvp_attach_tc")
-            # KPD_EDGE_PAIR=1: pair-packed message weights for a library built with -DKPD_EDGE_PAIR (experimental
-            # cta_group::2 edge kernel; measured slower than the single-CTA kernel, DESIGN.md 4.3)
-            self.tc_blob2, toffs = pack.pack_gvp_tc(sd, split=True, pair=os.environ.get("KPD_EDGE_PAIR", "0") == "1", **kw)
+            self.tc_blob2, toffs = pack.pack_gvp_tc(sd, split=True, **kw)
             tarr = (C.c_int64 * len(toffs))(*toffs)
             check(lib.kpd_gvp_attach_tc(self.handle, ptr(self.tc_blob2), tarr, len(toffs), 2), "kpd_gvp_attach_tc")
         if precision != "fp32":

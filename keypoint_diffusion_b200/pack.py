@@ -258,26 +258,8 @@ def pack_tc_weight(w: torch.Tensor, split: bool = False) -> torch.Tensor:
     return torch.cat(parts)
 
 
-def pack_tc_weight_pair(w: torch.Tensor) -> torch.Tensor:
-    """nn.Linear weight [N <= 256, K] for the CTA-pair (cta_group::2) bf16x3 edge kernel: per k-step the 8 KB each CTA
-    of the pair streams are contiguous -- [k-step][half of the output rows][hi, lo][2 k-chunks][NB/16 row groups][8][8]
-    bf16 -- so a k-step is ONE bulk copy per CTA (rows [0, NB/2) to the leader, [NB/2, NB) to its peer)."""
-    w = w.detach().float().cpu()
-    N, K = w.shape
-    assert N <= 256
-    ks = (K + 15) // 16
-    NB = (N + 31) // 32 * 32
-    wp = torch.zeros(NB, ks * 16)
-    wp[:N, :K] = w
-    hi = wp.to(torch.bfloat16)
-    lo = (wp - hi.float()).to(torch.bfloat16)
-    planes = torch.stack([hi, lo])                                              # [plane, NB, ks*16]
-    x = planes.view(2, 2, NB // 16, 8, ks, 2, 8)                                # [plane, half, group, row, ks, kc, 8]
-    return x.permute(4, 1, 0, 5, 2, 3, 6).contiguous().reshape(-1)              # [ks, half, plane, kc, group, row, 8]
-
-
 def pack_gvp_tc(sd: Dict[str, torch.Tensor], *, n_convs, update_kp, n_message_gvps, n_update_gvps, n_noise_gvps,
-                device, split: bool = False, pair: bool = False) -> Tuple[torch.Tensor, List[int]]:
+                device, split: bool = False) -> Tuple[torch.Tensor, List[int]]:
     """bf16 tensor-core weights of every GVP, in the library's creation order (csrc/gvp.cu kpd_gvp_attach_tc):
     per conv the message GVPs per edge type, then the update GVPs per node type; then the noise head.
     Three entries per GVP: to_feats_out (rows padded to 16), scalar_to_vector_gates (rows padded to 16) and the
@@ -306,10 +288,7 @@ def pack_gvp_tc(sd: Dict[str, torch.Tensor], *, n_convs, update_kp, n_message_gv
 
     for name in names:
         wf = sd[name + ".to_feats_out.0.weight"]
-        # pair=True (experimental CTA-pair edge kernel, library built with -DKPD_EDGE_PAIR): each CTA of a pair streams
-        # its half of the message GVPs' weight rows
-        paired = pair and split and ".edge_message_fns." in name and wf.shape[0] % 32 == 0
-        add(pack_tc_weight_pair(wf) if paired else pack_tc_weight(wf, split))
+        add(pack_tc_weight(wf, split))
         # gates weight: tcgen05 slabs in the bf16 mode; mma.sync B fragments in the bf16x3 mode (the gates GEMM then
         # runs on the warp-level tensor cores straight from the epilogue registers)
         wg = sd[name + ".scalar_to_vector_gates.weight"]

@@ -44,7 +44,7 @@ def build_model(kind, sd, kw, atom_nf, rec_nf, dev):
                         n_convs=kw.get("n_convs", 4), n_hidden_scalars=kw.get("n_hidden_scalars", 128),
                         update_kp=kw.get("update_kp", False), n_message_gvps=kw.get("n_message_gvps", 3),
                         n_update_gvps=kw.get("n_update_gvps", 2), n_noise_gvps=kw.get("n_noise_gvps", 3),
-                        message_norm=kw.get("message_norm", 1), device=dev)
+                        message_norm=kw.get("message_norm", 1), rbf_dim=kw.get("rbf_dim", 16), device=dev)
 
 
 def device_inputs(inputs, dev):
@@ -144,8 +144,9 @@ def test_denoiser_matches_golden(name):
         assert eh < TOL and ex < TOL, (name, t_str, eh, ex)
 
 
-def _full_size_case(arch, cfgs, n_lig=None, n_pockets=3):
-    """Shipped hyper-parameters (20-keypoint models), seeded weights, 6 complexes of mixed size."""
+def _full_size_case(arch, cfgs, n_lig=None, n_pockets=3, rbf_dim=16):
+    """Shipped hyper-parameters (20-keypoint models), seeded weights, 6 complexes of mixed size.  rbf_dim: width of the
+    GVP model's edge-distance RBF embedding (16 as shipped)."""
     from oracle import params as P
     from keypoint_diffusion_b200 import synthetic
     cfg = cfgs[f"{arch}_20kp"]
@@ -163,7 +164,7 @@ def _full_size_case(arch, cfgs, n_lig=None, n_pockets=3):
         d = cfg["dynamics_gvp"]
         rec_nf = cfg["rec_encoder_gvp"]["out_scalar_size"]
         shapes = P.gvp_dynamics_shapes(10, rec_nf, d["vector_size"], d["n_convs"], d["n_hidden_scalars"], d["update_kp"],
-                                       d["n_message_gvps"], d["n_update_gvps"], d["n_noise_gvps"])
+                                       d["n_message_gvps"], d["n_update_gvps"], d["n_noise_gvps"], rbf_dim=rbf_dim)
         sd = P.init_state_dict(shapes, seed=4)
         for k in sd:
             if k.endswith(".Wh") or k.endswith(".Wu"):
@@ -171,7 +172,7 @@ def _full_size_case(arch, cfgs, n_lig=None, n_pockets=3):
         kw = dict(vector_size=d["vector_size"], n_convs=d["n_convs"], n_hidden_scalars=d["n_hidden_scalars"],
                   message_norm=d["message_norm"], update_kp=d["update_kp"], ll_k=d["ll_k"], kl_k=d["kl_k"],
                   n_message_gvps=d["n_message_gvps"], n_update_gvps=d["n_update_gvps"],
-                  n_noise_gvps=d["n_noise_gvps"], graph_cutoffs=cfg["graph"]["graph_cutoffs"])
+                  n_noise_gvps=d["n_noise_gvps"], graph_cutoffs=cfg["graph"]["graph_cutoffs"], rbf_dim=rbf_dim)
         vs = d["vector_size"]
     pockets = [synthetic.keypoint_pocket(i, 20, rec_nf, vs, cfg["graph"]["graph_cutoffs"]["kk"]) for i in range(n_pockets)]
     x_l, h_l = synthetic.ligand_noise_state(n_lig, 10, seed=5)

@@ -131,27 +131,33 @@ def test_gvp_bf16x3_mode_small(name):
 
 
 def test_gvp_bf16x3_mode_full_size():
+    """Shipped-size GVP model (S = 256, V = 16) in the bf16x3 mode against the oracle, for both edge kernels the mode
+    selects from.  A message GVP's first input row is S + rbf_dim + V + 1 columns wide: at rbf_dim = 16 that is
+    289 -> 38 k-chunks, and the KS edge tile needs 232,176 B, inside the 232,448 B (227 KB) a block may have, so the
+    KS kernel runs.  At rbf_dim = 32, 305 columns -> 40 k-chunks, the KS tile would need 240,368 B > 232,448 B: this
+    case runs the stacked (STACK) bf16x3 edge kernel."""
     import yaml
     from helpers import GOLDEN, flat_batch, oracle_cfg, oracle_forward
     from test_gpu_parity import _full_size_case, build_model, device_inputs, run_forward
     from keypoint_diffusion_b200 import ops
     dev = torch.device("cuda:0")
     cfgs = yaml.safe_load(open(GOLDEN / "shipped_configs.yml"))
-    sd, kw, rec_nf, inputs = _full_size_case("gvp", cfgs)
-    cfg = oracle_cfg("gvp", kw, 10, rec_nf)
-    model = build_model("gvp", sd, kw, 10, rec_nf, dev)
-    model.set_precision("bf16x3")
-    batch, kk, t_in = device_inputs(inputs, dev)
-    gp = ops.GraphParams.from_module(kw["ll_k"], kw["kl_k"], kw["graph_cutoffs"])
-    graphs = ops.LigandGraphs(batch, gp, True).build(t_in["lig_x"], t_in["kp_x"])
-    for tval in (0.001, 0.5, 1.0):
-        fb = flat_batch(inputs)
-        ref_h, ref_x = oracle_forward("gvp", sd, cfg, fb, torch.full((fb.B,), tval))
-        eps_h, eps_x = run_forward("gvp", model, batch, graphs, kk, t_in, tval, dev)
-        torch.cuda.synchronize()
-        eh, ex = rel_err(eps_h.cpu(), ref_h), rel_err(eps_x.cpu(), ref_x)
-        print(f"gvp full size bf16x3 t={tval}: rel_err eps_h={eh:.2e} eps_x={ex:.2e}")
-        assert eh < TOL_X3 and ex < TOL_X3
+    for rbf_dim in (16, 32):
+        sd, kw, rec_nf, inputs = _full_size_case("gvp", cfgs, rbf_dim=rbf_dim)
+        cfg = oracle_cfg("gvp", kw, 10, rec_nf)
+        model = build_model("gvp", sd, kw, 10, rec_nf, dev)
+        model.set_precision("bf16x3")
+        batch, kk, t_in = device_inputs(inputs, dev)
+        gp = ops.GraphParams.from_module(kw["ll_k"], kw["kl_k"], kw["graph_cutoffs"])
+        graphs = ops.LigandGraphs(batch, gp, True).build(t_in["lig_x"], t_in["kp_x"])
+        for tval in (0.001, 0.5, 1.0):
+            fb = flat_batch(inputs)
+            ref_h, ref_x = oracle_forward("gvp", sd, cfg, fb, torch.full((fb.B,), tval))
+            eps_h, eps_x = run_forward("gvp", model, batch, graphs, kk, t_in, tval, dev)
+            torch.cuda.synchronize()
+            eh, ex = rel_err(eps_h.cpu(), ref_h), rel_err(eps_x.cpu(), ref_x)
+            print(f"gvp full size bf16x3 rbf_dim={rbf_dim} t={tval}: rel_err eps_h={eh:.2e} eps_x={ex:.2e}")
+            assert eh < TOL_X3 and ex < TOL_X3, (rbf_dim, tval, eh, ex)
 
 
 @pytest.mark.parametrize("name", ["egnn_small_kp", "egnn_small_nokp"])

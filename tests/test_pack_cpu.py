@@ -96,18 +96,3 @@ def test_pack_egnn_tc_entries():
     full_blocks, tail = divmod(n_rows, 256)
     expect = (full_blocks * 256 + (tail + 15) // 16 * 16) * ks * 16 * 2 * 2          # bf16 bytes, hi + lo
     assert first == (expect + 127) // 128 * 128
-
-
-def test_pack_tc_weight_pair_is_the_split_layout_dealt_to_two_ctas():
-    """CTA-pair packing (cta_group::2 edge kernel): per k-step, CTA r of the pair gets ONE contiguous piece holding rows
-    [r * NB/2, (r+1) * NB/2) of both planes and both k-chunks, in the same canonical 8x8 blocks as the split layout."""
-    g = torch.Generator().manual_seed(1)
-    for (N, K) in [(32, 16), (256, 289), (64, 40)]:
-        w = torch.randn(N, K, generator=g)
-        ks = (K + 15) // 16
-        NB = (N + 31) // 32 * 32
-        single = pack.pack_tc_weight(w, True).view(ks, 2, 2, NB // 8, 8, 8)            # k-step, plane, k-chunk, group, row, k
-        pair = pack.pack_tc_weight_pair(w).view(ks, 2, 2, 2, NB // 16, 8, 8)           # k-step, half, plane, k-chunk, ...
-        assert pair.numel() == single.numel()
-        for r in range(2):
-            assert torch.equal(pair[:, r], single[:, :, :, r * (NB // 16):(r + 1) * (NB // 16)])
