@@ -245,6 +245,36 @@ int kpd_ddpm_step(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_k
                   const float* coef, const int32_t* step_ptr,
                   const float* noise_x, const float* noise_h, uint64_t seed, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * (e') Fragment-conditioned reverse step (inpainting with RePaint-style resampling; an extension
+ * beyond the reference, DESIGN.md section 6.1).  Pass u of step s (t = s+1):
+ *   z_unk = x/alpha_t|s - var_terms*eps + sigma*noise             (what kpd_ddpm_step computes)
+ *   z_kn  = alpha_s*(x_fix - init_kp_com + kp_com) + sigma_s*e    positions of the fixed atoms
+ *           alpha_s*h_fix/lig_feat_norm_constant + sigma_s*e      their features
+ *   dx    = mean over fixed atoms of (z_unk_x - z_kn_x), added to z_kn_x and the complex's keypoints
+ *   x, h  = fixed ? z_kn : z_unk; then the ligand COM is removed from ligand and keypoints.
+ * kp_com is the complex's keypoint mean before the step; init_kp_com [B,3] the keypoint mean of
+ * the frame x_fix is given in.  A complex without a fixed atom gets exactly kpd_ddpm_step.
+ *   coef2: [T,4] rows (alpha_s, sigma_s, alpha_t|s, sigma_t|s) (schedule.inpaint_table);
+ *   fixed_mask: uint8 [n_lig] (nonzero = fixed) or NULL; x_fix [n_lig,3], h_fix [n_lig,atom_nf];
+ *   noise: NULL -> Philox keyed by (seed, s, atom, channel, word) with word 3u (posterior) and
+ *          3u+1 (known part); or injected [2][n_lig*(3+atom_nf)]: posterior then known-part draws,
+ *          each x channels [n_lig,3] first, then features [n_lig,atom_nf].
+ * Updates x_lig, h_lig, x_kp in place.
+ * ------------------------------------------------------------------------------------------ */
+int kpd_ddpm_inpaint_step(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_kp,
+                          const float* eps_x, const float* eps_h, int32_t atom_nf,
+                          const float* coef, const float* coef2, const int32_t* step_ptr, int32_t u,
+                          const uint8_t* fixed_mask, const float* x_fix, const float* h_fix,
+                          const float* init_kp_com, float lig_feat_norm_constant,
+                          const float* noise, uint64_t seed, void* stream);
+/* Re-noise between resampling passes: z_t = alpha_t|s*z_s + sigma_t|s*e for positions and features
+ * (Philox word 3u+2, or injected noise [n_lig*(3+atom_nf)], x first), then the ligand COM is removed
+ * from ligand and keypoints. */
+int kpd_renoise(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_kp, int32_t atom_nf,
+                const float* coef2, const int32_t* step_ptr, int32_t u, const float* noise, uint64_t seed,
+                void* stream);
+
 /* remove_com (ligand_diffuser.py:185-203): which = 0 ligand COM, 1 keypoint COM; shifts both
  * node types.  If com_out != NULL the [B,3] means are also written there. */
 int kpd_remove_com(const kpd_batch* batch, float* x_lig, float* x_kp, int32_t which,
@@ -300,6 +330,20 @@ int32_t kpd_sampler_launches_per_step(const kpd_sampler* s);
 /* Offset added to the ligand-atom index of the noise counter (seed, step, atom, channel): lets a caller sample one batch
  * as several sub-batches (own samplers, own streams) and draw exactly the noise of the undivided batch. */
 int kpd_sampler_set_atom_offset(kpd_sampler* s, int32_t first_atom);
+/* Turns a freshly created sampler (not yet run) into an inpainting sampler: every reverse step runs
+ * `resamplings` passes of graph build + denoiser + kpd_ddpm_inpaint_step, with kpd_renoise between
+ * passes; launches_per_step counts all of them.  coef2: [T,4] device table (schedule.inpaint_table),
+ * must outlive the sampler.  Allocates a few bytes of device memory (synchronous).  Pick
+ * steps_per_graph ~ (plain value) / resamplings so that a captured graph stays as large as a plain one.
+ * With injected noise, kpd_sampler_run takes [1 + T*(3*resamplings - 1), n_lig, 3+atom_nf]: slot 0 =
+ * initial draw, then per executed step and pass u the posterior, known-part and (u < resamplings-1)
+ * re-noise draws. */
+int kpd_sampler_enable_inpainting(kpd_sampler* s, int32_t resamplings, const float* coef2);
+/* The fragment of the next runs of an inpainting sampler: fixed_mask uint8 [n_lig] (NULL = no fixed
+ * atom), x_fix [n_lig,3] in the frame of the x_kp passed to kpd_sampler_run, h_fix [n_lig,atom_nf] in
+ * the returned feature space.  Only pointers are kept; each run uploads them to device memory, so a
+ * captured sampler follows new buffers without capturing again. */
+int kpd_sampler_set_fragment(kpd_sampler* s, const uint8_t* fixed_mask, const float* x_fix, const float* h_fix);
 
 /* Output decode, the step right behind the path (reference test.py:199-203: torch.argmax(lig_feat, dim=1) on the
  * host, then dataset.lig_atom_idx_to_element): atom_type[i] = argmax_c h_lig[i, c], lowest index on ties. */

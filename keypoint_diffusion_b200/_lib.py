@@ -91,6 +91,8 @@ def _load():
         "kpd_gvp_forward": (I, [P, C.POINTER(KpdBatch), P, P, P, P, P, P, I, C.POINTER(KpdCsr),
                                 C.POINTER(KpdCsr), C.POINTER(KpdCsr), C.POINTER(KpdCsr), P, P, P, P]),
         "kpd_ddpm_step": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, P, P, P, P, U64, P]),
+        "kpd_ddpm_inpaint_step": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, P, P, P, I, P, P, P, P, F, P, U64, P]),
+        "kpd_renoise": (I, [C.POINTER(KpdBatch), P, P, P, I, P, P, I, P, U64, P]),
         "kpd_remove_com": (I, [C.POINTER(KpdBatch), P, P, I, P, P]),
         "kpd_shift_by_complex": (I, [P, P, I, P, F, P]),
         "kpd_randn_init": (I, [P, P, I, I, U64, P]),
@@ -101,6 +103,8 @@ def _load():
         "kpd_sampler_run": (I, [P, P, P, P, P, P, P, P, U64, I, P]),
         "kpd_sampler_launches_per_step": (I, [P]),
         "kpd_sampler_set_atom_offset": (I, [P, I]),
+        "kpd_sampler_enable_inpainting": (I, [P, I, P]),
+        "kpd_sampler_set_fragment": (I, [P, P, P, P]),
         "kpd_decode_atom_types": (I, [P, I, I, P, P]),
     }
     for name, (res, args) in sig.items():

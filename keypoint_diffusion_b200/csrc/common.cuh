@@ -242,7 +242,24 @@ int launch_shift(float* x, const int* node_batch, int n, const float* v, float s
 int launch_randn_init(float* x_lig, float* h_lig, int n_lig, int F, uint64_t seed, const RunParams* rp, cudaStream_t st);
 int launch_scale(float* x, int n, float s, cudaStream_t st);
 int launch_step_prologue(int* counter, int* step, float* t_cur, const float* coef, cudaStream_t st);
-long long launch_count();   // kernels launched through check_launch() so far (this process)
+
+// ------------------------------------------------------------------ fragment-conditioned sampling (inpaint.cu)
+struct InpaintParams {    // a sampler keeps it in device memory, so that a captured graph can be re-pointed
+    const uint8_t* mask;  // NULL (no fixed atom) or [n_lig], nonzero = fixed
+    const float* x_fix;   // [n_lig][3] fragment positions, frame of the keypoints the caller passed
+    const float* h_fix;   // [n_lig][F] fragment features, returned (un-normalised) feature space
+    const float* coef2;   // [T][4] rows (alpha_s, sigma_s, alpha_t|s, sigma_t|s)
+};
+// noise: NULL or the draws of this call ([2][n_lig][3+F] posterior then known part; [n_lig][3+F] for renoise), x first;
+// with rp (a sampler's run) and ip (its fragment) the slot and the buffers come from device memory instead
+int launch_ddpm_inpaint_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
+                             const float* eps_h, int F, const float* coef, const int* step_ptr, int u, int r,
+                             const InpaintParams& fr, const InpaintParams* ip, const float* init_kp_com, float norm_c,
+                             const float* noise, uint64_t seed, const RunParams* rp, cudaStream_t st);
+int launch_renoise(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, int F, const int* step_ptr, int u, int r,
+                   const float* coef2, const InpaintParams* ip, const float* noise, uint64_t seed, const RunParams* rp,
+                   cudaStream_t st);
+long long launch_count();  // kernels launched through check_launch() so far (this process)
 
 // optional per-kernel CUDA-event timing (bench.py's roofline leg); no-ops unless enabled and
 // never active while a stream is being captured

@@ -9,23 +9,11 @@
 // after a step is bit-identical to the op-by-op PyTorch evaluation the oracle performs.
 // HBM-bound: 2 x (3+F) floats read + (3+F) written per ligand atom, 6 floats per keypoint.
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace kpd {
 
-// ---- Philox4x32-10 (Salmon et al. 2011), counter = (atom, step+1, group, 0), key = seed
-__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
-    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(M0, ctr.x), lo0 = M0 * ctr.x;
-        const uint32_t hi1 = __umulhi(M1, ctr.z), lo1 = M1 * ctr.z;
-        ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-        key.x += W0;
-        key.y += W1;
-    }
-    return ctr;
-}
-
+// ---- Philox4x32-10 (philox.cuh), counter = (atom, step+1, group, 0), key = seed
 // standard normal for (seed, step, atom, channel); channels are drawn 4 at a time
 __device__ float philox_normal(uint64_t seed, int step, int atom, int ch) {
     const uint4 r = philox4x32_10(make_uint4((uint32_t)atom, (uint32_t)(step + 1), (uint32_t)(ch >> 2), 0u),

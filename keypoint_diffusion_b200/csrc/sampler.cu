@@ -7,7 +7,9 @@
 //     step_prologue -> graph_mark/scan/fill -> denoiser -> ddpm_step
 // with all shapes static (edge arrays sized at capacity, counts on the device), so it is
 // captured once into a CUDA graph of `steps_per_graph` steps and replayed T/steps_per_graph
-// times; the step index lives on the device and is decremented by step_prologue.
+// times; the step index lives on the device and is decremented by step_prologue.  An inpainting sampler
+// (kpd_sampler_enable_inpainting) runs r passes per step instead:
+//     step_prologue -> r x (graph_mark/scan/fill -> denoiser -> ddpm_inpaint_step [-> renoise])
 #include "common.cuh"
 #include <string.h>
 
@@ -36,6 +38,10 @@ struct kpd_sampler {
     cudaGraphExec_t exec;
     int launches_per_step;
     int atom_offset;
+    // fragment-conditioned sampling (kpd_sampler_enable_inpainting): 0 = plain loop, else resamplings per step
+    int resamplings;
+    InpaintParams frag;       // host copy, uploaded to frag_dev by every run
+    InpaintParams* frag_dev;
 };
 
 static int64_t model_ws_bytes(const kpd_sampler_config* cfg, const void* model, const kpd_batch* b, int cap_ll,
@@ -101,21 +107,40 @@ extern "C" int64_t kpd_sampler_workspace_bytes(const kpd_sampler_config* cfg, co
     return bytes;
 }
 
-static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
-    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef, st));
+// graph build + denoiser on the current state
+static int enqueue_denoiser(kpd_sampler* s, cudaStream_t st) {
     KPD_TRY(build_graph_impl(&s->batch, s->x_lig, s->x_kp, &s->gp, &s->ll, &s->kl, s->has_lk ? &s->lk : nullptr,
                              nullptr, nullptr, s->graph_ws, s->edge_accum, st));
-    if (s->cfg.arch == 0) {
-        KPD_TRY(kpd_egnn_forward(static_cast<const kpd_egnn_model*>(s->model), &s->batch, s->h_lig, s->x_lig, s->h_kp,
-                                 s->x_kp, s->kp_enc, s->t_cur, 0, &s->ll, &s->kl, s->has_lk ? &s->lk : nullptr,
-                                 s->has_lk ? &s->kk : nullptr, s->eps_h, s->eps_x, s->model_ws, st));
-    } else {
-        KPD_TRY(kpd_gvp_forward(static_cast<const kpd_gvp_model*>(s->model), &s->batch, s->h_lig, s->x_lig, s->h_kp,
-                                s->x_kp, s->v_kp, s->t_cur, 0, &s->ll, &s->kl, s->has_lk ? &s->lk : nullptr,
-                                s->has_lk ? &s->kk : nullptr, s->eps_h, s->eps_x, s->model_ws, st));
-    }
+    if (s->cfg.arch == 0)
+        return kpd_egnn_forward(static_cast<const kpd_egnn_model*>(s->model), &s->batch, s->h_lig, s->x_lig, s->h_kp,
+                                s->x_kp, s->kp_enc, s->t_cur, 0, &s->ll, &s->kl, s->has_lk ? &s->lk : nullptr,
+                                s->has_lk ? &s->kk : nullptr, s->eps_h, s->eps_x, s->model_ws, st);
+    return kpd_gvp_forward(static_cast<const kpd_gvp_model*>(s->model), &s->batch, s->h_lig, s->x_lig, s->h_kp, s->x_kp,
+                           s->v_kp, s->t_cur, 0, &s->ll, &s->kl, s->has_lk ? &s->lk : nullptr,
+                           s->has_lk ? &s->kk : nullptr, s->eps_h, s->eps_x, s->model_ws, st);
+}
+
+static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
+    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef, st));
+    KPD_TRY(enqueue_denoiser(s, st));
     KPD_TRY(launch_ddpm_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->coef,
                              s->step, nullptr, nullptr, 0, s->rp, st));
+    return 0;
+}
+
+// one reverse step of the inpainting loop: prologue, then r x (graph build, denoiser, inpaint step[, re-noise])
+static int enqueue_inpaint_step(kpd_sampler* s, cudaStream_t st) {
+    const int r = s->resamplings, F = s->cfg.atom_nf;
+    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef, st));
+    for (int u = 0; u < r; ++u) {
+        KPD_TRY(enqueue_denoiser(s, st));
+        KPD_TRY(launch_ddpm_inpaint_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, F, s->coef, s->step,
+                                         u, r, InpaintParams{}, s->frag_dev, s->init_kp_com, s->cfg.lig_feat_norm_constant,
+                                         nullptr, 0, s->rp, st));
+        if (u < r - 1)
+            KPD_TRY(launch_renoise(&s->batch, s->x_lig, s->h_lig, s->x_kp, F, s->step, u, r, nullptr, s->frag_dev,
+                                   nullptr, 0, s->rp, st));
+    }
     return 0;
 }
 
@@ -146,6 +171,7 @@ extern "C" int kpd_sampler_create(const kpd_sampler_config* cfg, const void* mod
 extern "C" void kpd_sampler_destroy(kpd_sampler* s) {
     if (!s) return;
     if (s->exec) cudaGraphExecDestroy(s->exec);
+    if (s->frag_dev) cudaFree(s->frag_dev);
     if (s->graph) cudaGraphDestroy(s->graph);
     if (s->ev_in) cudaEventDestroy(s->ev_in);
     if (s->ev_out) cudaEventDestroy(s->ev_out);
@@ -178,11 +204,34 @@ extern "C" int kpd_sampler_set_atom_offset(kpd_sampler* s, int32_t first_atom) {
     return 0;
 }
 
+extern "C" int kpd_sampler_enable_inpainting(kpd_sampler* s, int32_t resamplings, const float* coef2) {
+    KPD_REQUIRE(s && coef2 && resamplings >= 1, "kpd_sampler_enable_inpainting: bad argument");
+    KPD_REQUIRE(!s->exec && !s->resamplings, "kpd_sampler_enable_inpainting: the sampler has already run or is inpainting");
+    KPD_REQUIRE(sizeof(float) * 3 * (size_t)s->batch.max_lig <= 48 * 1024,
+                "kpd_sampler_enable_inpainting: %d atoms in one complex exceed the supported 4096", s->batch.max_lig);
+    const cudaError_t e = cudaMalloc(&s->frag_dev, sizeof(InpaintParams));
+    KPD_REQUIRE(e == cudaSuccess, "kpd_sampler_enable_inpainting: %s", cudaGetErrorString(e));
+    s->resamplings = resamplings;
+    s->frag = InpaintParams{nullptr, nullptr, nullptr, coef2};
+    return 0;
+}
+
+extern "C" int kpd_sampler_set_fragment(kpd_sampler* s, const uint8_t* fixed_mask, const float* x_fix, const float* h_fix) {
+    KPD_REQUIRE(s && s->resamplings, "kpd_sampler_set_fragment: not an inpainting sampler");
+    KPD_REQUIRE(!fixed_mask || (x_fix && h_fix), "kpd_sampler_set_fragment: a fixed mask needs x_fix and h_fix");
+    s->frag.mask = fixed_mask; s->frag.x_fix = x_fix; s->frag.h_fix = h_fix;
+    return 0;
+}
+
+static int enqueue_any_step(kpd_sampler* s, cudaStream_t st) {
+    return s->resamplings ? enqueue_inpaint_step(s, st) : enqueue_step(s, st);
+}
+
 static int capture(kpd_sampler* s) {
     cudaError_t e = cudaStreamBeginCapture(s->stream, cudaStreamCaptureModeThreadLocal);
     KPD_REQUIRE(e == cudaSuccess, "sampler: begin capture: %s", cudaGetErrorString(e));
     int rc = 0;
-    for (int i = 0; i < s->cfg.steps_per_graph && rc == 0; ++i) rc = enqueue_step(s, s->stream);
+    for (int i = 0; i < s->cfg.steps_per_graph && rc == 0; ++i) rc = enqueue_any_step(s, s->stream);
     e = cudaStreamEndCapture(s->stream, &s->graph);
     if (rc != 0) return rc;
     KPD_REQUIRE(e == cudaSuccess, "sampler: end capture: %s", cudaGetErrorString(e));
@@ -217,6 +266,7 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     CU(cudaMemcpyAsync(s->rp, &rp, sizeof(rp), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(s->counter, counter0, sizeof(counter0), cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(s->edge_accum, 0, 4 * sizeof(long long), st));
+    if (s->resamplings) CU(cudaMemcpyAsync(s->frag_dev, &s->frag, sizeof(InpaintParams), cudaMemcpyHostToDevice, st));
 
     // frame setup (ligand_diffuser.py:348-370)
     KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 1, 0, s->init_kp_com, st));                // init_kp_com (:348)
@@ -240,7 +290,7 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     }
     for (; done < n_steps; ++done) {
         const long long l0 = launch_count();
-        KPD_TRY(enqueue_step(s, st));
+        KPD_TRY(enqueue_any_step(s, st));
         s->launches_per_step = (int)(launch_count() - l0);
     }
     // frame restore (:438-447)

@@ -17,7 +17,8 @@ from . import hetero, ops
 from .dynamics import LigRecDynamics, LigRecDynamicsGVP
 from .n_nodes_dist import LigandSizeDistribution
 from .receptor_encoder import ReceptorEncoder, ReceptorEncoderGVP
-from .schedule import PredefinedNoiseSchedule, alpha, coefficient_table, sigma, sigma_and_alpha_t_given_s
+from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_table, inpaint_table, sigma,
+                       sigma_and_alpha_t_given_s)
 from .utils import get_batch_idxs, split_bounds
 
 DEFAULT_SUB_BATCHES = {"gvp": 4, "egnn": 2}      # measured on B200: profiles/r01_sweep_sub_batches_*.txt
@@ -78,6 +79,7 @@ class KeypointDiffusion(nn.Module):
             self.rec_encoder = FixedReceptorEncoder(rec_encoder_config['vector_size'] if architecture == 'gvp' else None)
         object.__setattr__(self, "_samplers", {})
         object.__setattr__(self, "_coef", {})
+        object.__setattr__(self, "_coef2", {})
         object.__setattr__(self, "last_launches_per_step", 0)
         object.__setattr__(self, "_streams", {})
         object.__setattr__(self, "cold_captures", 0)       # capacity buckets captured so far (a cold call each)
@@ -130,6 +132,14 @@ class KeypointDiffusion(nn.Module):
             self._coef.clear()
             self._coef[key] = coefficient_table(self.gamma.gamma, self.n_timesteps).to(device)
         return self._coef[key]
+
+    def inpaint_coef_table(self, device) -> torch.Tensor:
+        """schedule.inpaint_table on `device`, cached like coef_table."""
+        key = (str(device), self.gamma.gamma._version, self.gamma.gamma.data_ptr())
+        if key not in self._coef2:
+            self._coef2.clear()
+            self._coef2[key] = inpaint_table(self.gamma.gamma, self.n_timesteps).to(device)
+        return self._coef2[key]
 
     # ------------------------------------------------------------------ one reverse step (reference :497-538)
     @torch.no_grad()
@@ -221,13 +231,17 @@ class KeypointDiffusion(nn.Module):
             return max(1, min(int(env), n_complexes))
         return max(1, min(DEFAULT_SUB_BATCHES[self.architecture], n_complexes // 16))
 
-    def _capacity_sampler(self, instance: int, plan: "ops.CapacityPlan", device, steps_per_graph, use_cuda_graph):
+    def _capacity_sampler(self, instance: int, plan: "ops.CapacityPlan", device, steps_per_graph, use_cuda_graph,
+                          resamplings: int = 0):
         """The captured loop of capacity bucket plan.key (created on first use, then shared by every batch that lands in
         the bucket -- whatever its per-complex sizes, pockets or kk graph).  Groups of one call that run concurrently
-        and share a bucket take distinct instances 0, 1, ... of it."""
+        and share a bucket take distinct instances 0, 1, ... of it.  resamplings >= 1: the inpainting loop with that
+        many passes per step (cached apart from the plain loop: its captured sequence differs)."""
         model = self.dynamics.device_model(device)
         key = ("cap", instance, plan.key, self.dynamics._st.model_key, steps_per_graph, use_cuda_graph,
                getattr(model, "precision", "fp32"), self.n_timesteps)
+        if resamplings:
+            key = key + ("inpaint", int(resamplings))
         hit = self._cache_get(key)
         if hit is None:
             kp_width = self.n_kp_feat
@@ -235,7 +249,8 @@ class KeypointDiffusion(nn.Module):
             hit = ops.CapacitySampler(model, plan, self.dynamics.graph_params(), self.coef_table(device), self.n_timesteps,
                                       self.n_lig_features, kp_width, v_width, steps_per_graph=steps_per_graph,
                                       use_cuda_graph=use_cuda_graph,
-                                      lig_feat_norm_constant=float(self.lig_feat_norm_constant))
+                                      lig_feat_norm_constant=float(self.lig_feat_norm_constant), resamplings=resamplings,
+                                      inpaint_coef=self.inpaint_coef_table(device) if resamplings else None)
             self._samplers[key] = hit
             object.__setattr__(self, "cold_captures", self.cold_captures + 1)
         return hit
@@ -244,7 +259,9 @@ class KeypointDiffusion(nn.Module):
     def sample_from_encoded_receptors(self, g, visualize=False, init_lig_pos: torch.Tensor = None, noise=None,
                                       seed: Optional[int] = None, steps_per_graph: int = 50, use_cuda_graph: bool = True,
                                       return_device_tensors: bool = False, sub_batches: Optional[int] = None,
-                                      decode: bool = False, capacity: bool = True):
+                                      decode: bool = False, capacity: bool = True, fixed_mask: torch.Tensor = None,
+                                      fixed_pos: torch.Tensor = None, fixed_feat: torch.Tensor = None,
+                                      resamplings: int = 1):
         """Returns (lig_pos, lig_feat): one CPU tensor per complex, as the reference does (:342-469).  ``g`` may live
         on the CPU (pinned or not): its keypoint tensors are uploaded here, straight into the sampler's buffers -- the
         host->device boundary of the path (reference test.py:152-161).
@@ -253,7 +270,18 @@ class KeypointDiffusion(nn.Module):
         tuple of ligand sizes, another pocket or another kk graph re-uses the CUDA graphs captured for its bucket
         instead of re-capturing, so the reference's real entry points -- random sizes per call, :490-495 -- stay warm.
         ``capacity=False`` selects samplers captured for the exact layout (kept for A/B tests).  ``decode=True`` also
-        returns the atom types (argmax over the feature channels, computed on the device: test.py:199-203)."""
+        returns the atom types (argmax over the feature channels, computed on the device: test.py:199-203).
+
+        Fragment-conditioned sampling (inpainting; an extension beyond the reference, DESIGN.md section 6.1): with
+        ``fixed_mask`` (bool [n_lig], g's ligand order) the atoms it marks are pinned to ``fixed_pos`` ([n_lig,3], in the
+        frame the ligands are returned in) and ``fixed_feat`` ([n_lig,F], returned feature space); rows of unmarked atoms
+        are ignored.  Every reverse step runs ``resamplings`` denoiser passes (RePaint resampling, jump length 1), so a
+        call costs about ``resamplings`` plain calls.  Complexes without a marked atom are sampled exactly as without
+        a mask at resamplings=1.  Only the capacity path supports it: ``capacity=False`` raises ValueError."""
+        n_lig_total = int(g.num_nodes('lig'))
+        inpaint = self._check_fragment_args(n_lig_total, fixed_mask, fixed_pos, fixed_feat, resamplings)
+        if inpaint and not capacity:
+            raise ValueError("fragment-conditioned sampling runs on the capacity path only (capacity=True)")
         if visualize:
             raise NotImplementedError("visualize=True (a per-step CPU copy of the whole graph) is a debug feature "
                                       "outside the throughput path")
@@ -303,7 +331,12 @@ class KeypointDiffusion(nn.Module):
             plan = ops.plan_capacity(lig_n[a:b], kp_n[a:b], int(gs.numel()), gp)
             inst = taken.get(plan.key, 0)
             taken[plan.key] = inst + 1
-            smp = self._capacity_sampler(inst, plan, dev, steps_per_graph, use_cuda_graph)
+            smp = self._capacity_sampler(inst, plan, dev, steps_per_graph, use_cuda_graph,
+                                         resamplings=int(resamplings) if inpaint else 0)
+            frag = None
+            if inpaint:
+                l1 = lig_ptr[b]
+                frag = (fixed_mask[l0:l1], fixed_pos[l0:l1], fixed_feat[l0:l1])
             if n_sub > 1 and (slot, str(dev)) not in self._streams:
                 self._streams[(slot, str(dev))] = torch.cuda.Stream(device=dev)
             st = self._streams[(slot, str(dev))] if n_sub > 1 else cur
@@ -311,7 +344,7 @@ class KeypointDiffusion(nn.Module):
                 st.wait_event(ready)
             with torch.cuda.stream(st):
                 out = smp.run(plan, kp['x_0'][k0:k1], kp['h_0'][k0:k1], kv[k0:k1] if kv is not None else None, gs, gd,
-                              init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode)
+                              init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag)
             if n_sub > 1:
                 for t in out:
                     t.record_stream(cur)
@@ -331,6 +364,58 @@ class KeypointDiffusion(nn.Module):
         pos_cpu, feat_cpu = x_lig.cpu(), h_lig.cpu()                # device -> host boundary (reference :464)
         res = (list(torch.split(pos_cpu, lig_n)), list(torch.split(feat_cpu, lig_n)))
         return res + (list(torch.split(atom_type.cpu(), lig_n)),) if decode else res
+
+    def _check_fragment_args(self, n_lig: int, fixed_mask, fixed_pos, fixed_feat, resamplings) -> bool:
+        """ValueError for an inconsistent fragment request (host-side checks, before any device work); True when the
+        call is fragment-conditioned."""
+        if int(resamplings) < 1:
+            raise ValueError(f"resamplings must be >= 1, got {resamplings}")
+        if fixed_mask is None:
+            if fixed_pos is not None or fixed_feat is not None:
+                raise ValueError("fixed_pos / fixed_feat need fixed_mask")
+            if int(resamplings) > 1:
+                raise ValueError("resamplings > 1 needs fixed atoms (fixed_mask)")
+            return False
+        if fixed_pos is None or fixed_feat is None:
+            raise ValueError("fixed_mask needs fixed_pos and fixed_feat")
+        F = self.n_lig_features
+        if tuple(fixed_mask.shape) != (n_lig,):
+            raise ValueError(f"fixed_mask must have shape [{n_lig}], got {tuple(fixed_mask.shape)}")
+        if fixed_pos.dim() != 2 or fixed_pos.shape[1] != 3 or fixed_pos.shape[0] != n_lig:
+            raise ValueError(f"fixed_pos must have shape [{n_lig}, 3], got {tuple(fixed_pos.shape)}")
+        if fixed_feat.dim() != 2 or fixed_feat.shape[1] != F or fixed_feat.shape[0] != n_lig:
+            raise ValueError(f"fixed_feat must have shape [{n_lig}, {F}], got {tuple(fixed_feat.shape)}")
+        if int(resamplings) > 1 and not bool(fixed_mask.any()):
+            raise ValueError("resamplings > 1 needs at least one fixed atom")
+        return True
+
+    def _check_fragments(self, fragments, n_lig_atoms, resamplings) -> bool:
+        """Host-side validation of _sample's per-receptor fragments; True when at least one atom is fixed."""
+        if int(resamplings) < 1:
+            raise ValueError(f"resamplings must be >= 1, got {resamplings}")
+        any_fixed = False
+        if fragments is not None:
+            if len(fragments) != len(n_lig_atoms):
+                raise ValueError(f"fragments: one entry (or None) per receptor, got {len(fragments)} for "
+                                 f"{len(n_lig_atoms)} receptors")
+            F = self.n_lig_features
+            for r, frag in enumerate(fragments):
+                if frag is None:
+                    continue
+                pos, feat = frag
+                if pos.dim() != 2 or pos.shape[1] != 3:
+                    raise ValueError(f"fragment of receptor {r}: positions must be [m, 3], got {tuple(pos.shape)}")
+                if feat.dim() != 2 or feat.shape[1] != F or feat.shape[0] != pos.shape[0]:
+                    raise ValueError(f"fragment of receptor {r}: features must be [{pos.shape[0]}, {F}], got "
+                                     f"{tuple(feat.shape)}")
+                m = int(pos.shape[0])
+                small = [int(n) for n in n_lig_atoms[r] if int(n) < m]
+                if small:
+                    raise ValueError(f"receptor {r}: requested ligand size {small[0]} is below its {m}-atom fragment")
+                any_fixed = any_fixed or (m > 0 and len(n_lig_atoms[r]) > 0)
+        if int(resamplings) > 1 and not any_fixed:
+            raise ValueError("resamplings > 1 needs at least one fragment atom")
+        return any_fixed
 
     def _sample_exact_layout(self, g, dev, init_pos, noise, seed, steps_per_graph, use_cuda_graph, return_device_tensors,
                              n_sub):
@@ -395,14 +480,20 @@ class KeypointDiffusion(nn.Module):
     def _sample(self, ref_graphs: List, n_lig_atoms: List[List[int]], rec_enc_batch_size: int = 32,
                 diff_batch_size: int = 32, visualize=False, use_ref_lig_com: bool = False, encoded: bool = False,
                 init_lig_pos: Optional[List[torch.Tensor]] = None, noise: Optional[List[torch.Tensor]] = None,
-                complexes: Optional[List[int]] = None, **sampler_kw):
+                complexes: Optional[List[int]] = None, fragments: Optional[List] = None, resamplings: int = 1,
+                **sampler_kw):
         """ref_graphs: one single-complex graph per receptor (reference :270-340).  ``encoded=True`` skips the receptor
         encoder (graphs already hold kp nodes + kk edges).  init_lig_pos: optional [3] tensor per receptor.
         noise: optional injected Gaussian draws, one [T+1, n_lig*(3+F)] tensor per diffusion batch (parity runs).
         complexes: optional subset (indices into the flattened receptor-major list of requested ligands) to sample --
         what sample_sharded deals to this rank; the returned lists then hold only those.
+        fragments: optional, one ``(pos [m,3], feat [m,F])`` or None per receptor: every ligand requested for that
+        receptor starts with those m atoms, pinned (fragment growing; positions in the receptor's frame, features in the
+        returned feature space), with ``resamplings`` denoiser passes per reverse step (see
+        sample_from_encoded_receptors).  A diffusion batch without any fragment atom is sampled by the plain loop.
 
         The diffusion batches are assembled on the device (hetero.expand_complexes): no per-complex graph copies."""
+        has_fragment = self._check_fragments(fragments, n_lig_atoms, resamplings)
         n_receptors = len(ref_graphs)
         enc, rec_mean = self._encode_all(ref_graphs, rec_enc_batch_size, encoded)
         dev = enc.device
@@ -420,12 +511,15 @@ class KeypointDiffusion(nn.Module):
         size_t = torch.tensor(sizes, dtype=torch.long, device=dev)
         lig_pos, lig_feat = [], []
         for b in range(ceil(len(todo) / diff_batch_size)):
-            idx = torch.tensor(todo[b * diff_batch_size:(b + 1) * diff_batch_size], dtype=torch.long, device=dev)
+            chunk = todo[b * diff_batch_size:(b + 1) * diff_batch_size]
+            idx = torch.tensor(chunk, dtype=torch.long, device=dev)
             bg = hetero.expand_complexes(enc, pocket_t[idx], size_t[idx], self.n_lig_features)
             if centers is None:
                 raise ValueError("init_lig_pos is required when the graphs have no 'rec' nodes (SURVEY N7)")
+            frag_kw = (self._fragment_rows(fragments, [pocket_of[i] for i in chunk], [sizes[i] for i in chunk], resamplings)
+                       if has_fragment else {})
             p, f = self.sample_from_encoded_receptors(bg, visualize=visualize, init_lig_pos=centers[pocket_t[idx]],
-                                                      noise=None if noise is None else noise[b], **sampler_kw)
+                                                      noise=None if noise is None else noise[b], **frag_kw, **sampler_kw)
             lig_pos.extend(p)
             lig_feat.extend(f)
         if complexes is not None:
@@ -435,6 +529,27 @@ class KeypointDiffusion(nn.Module):
             start, end = end, end + len(n_lig_atoms[rec_idx])
             samples.append({'positions': lig_pos[start:end], 'features': lig_feat[start:end]})
         return samples
+
+    def _fragment_rows(self, fragments, receptors: List[int], sizes: List[int], resamplings: int) -> Dict:
+        """fixed_mask / fixed_pos / fixed_feat (host tensors, batch ligand order) of one diffusion batch whose complexes
+        belong to `receptors`; {} (the plain loop) when none of them has a fragment atom."""
+        F = self.n_lig_features
+        n = sum(sizes)
+        mask = torch.zeros(n, dtype=torch.bool)
+        pos = torch.zeros(n, 3)
+        feat = torch.zeros(n, F)
+        off = 0
+        for r, size in zip(receptors, sizes):
+            frag = fragments[r]
+            if frag is not None and frag[0].shape[0] > 0:
+                m = int(frag[0].shape[0])
+                mask[off:off + m] = True
+                pos[off:off + m] = frag[0].detach().float().cpu()
+                feat[off:off + m] = frag[1].detach().float().cpu()
+            off += size
+        if not bool(mask.any()):
+            return {}
+        return dict(fixed_mask=mask, fixed_pos=pos, fixed_feat=feat, resamplings=resamplings)
 
     @torch.no_grad()
     def sample_sharded(self, ref_graphs: List, n_lig_atoms: List[List[int]], rec_enc_batch_size: int = 32,
@@ -474,9 +589,11 @@ class KeypointDiffusion(nn.Module):
 
     @torch.no_grad()
     def sample_given_pocket(self, rec_graph, n_lig_atoms: torch.Tensor, rec_enc_batch_size: int = 32,
-                            diff_batch_size: int = 32, visualize=False, **kw):
+                            diff_batch_size: int = 32, visualize=False, fragment=None, **kw):
+        """fragment: optional ``(pos [m,3], feat [m,F])``: every ligand starts with these m atoms (see _sample)."""
         samples = self._sample([rec_graph], n_lig_atoms=[n_lig_atoms.tolist()], rec_enc_batch_size=rec_enc_batch_size,
-                               diff_batch_size=diff_batch_size, visualize=visualize, **kw)
+                               diff_batch_size=diff_batch_size, visualize=visualize,
+                               fragments=None if fragment is None else [fragment], **kw)
         return samples[0]['positions'], samples[0]['features']
 
     @torch.no_grad()

@@ -392,6 +392,26 @@ def ddpm_step(batch: DeviceBatch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, step: 
           "kpd_ddpm_step")
 
 
+def ddpm_inpaint_step(batch: DeviceBatch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, coef2, step: torch.Tensor, u: int,
+                      fixed_mask, x_fix, h_fix, init_kp_com, lig_feat_norm_constant=1.0, noise=None, seed=0):
+    """In-place fragment-conditioned reverse step, pass u (kpd_ddpm_inpaint_step): the posterior step with the atoms of
+    fixed_mask (bool / uint8 [n_lig], or None) replaced by a noised copy of (x_fix, h_fix), aligned to the generated
+    part.  noise: None (Philox) or [2, n_lig*(3+F)] injected draws (posterior, known part; x channels first)."""
+    _require_cuda(x_lig, h_lig, x_kp, eps_x, eps_h, coef, coef2, step, init_kp_com, fixed_mask, x_fix, h_fix, noise)
+    mask = fixed_mask.to(torch.uint8).contiguous() if fixed_mask is not None else None
+    check(lib.kpd_ddpm_inpaint_step(C.byref(batch.c), ptr(x_lig), ptr(h_lig), ptr(x_kp), ptr(eps_x), ptr(eps_h),
+                                    h_lig.shape[1], ptr(coef), ptr(coef2), ptr(step), int(u), ptr(mask),
+                                    ptr(x_fix), ptr(h_fix), ptr(init_kp_com), float(lig_feat_norm_constant), ptr(noise),
+                                    int(seed), _stream()), "kpd_ddpm_inpaint_step")
+
+
+def renoise(batch: DeviceBatch, x_lig, h_lig, x_kp, coef2, step: torch.Tensor, u: int, noise=None, seed=0):
+    """In-place re-noise to level t = s+1 after pass u of step s (kpd_renoise); noise: None or [n_lig*(3+F)]."""
+    _require_cuda(x_lig, h_lig, x_kp, coef2, step, noise)
+    check(lib.kpd_renoise(C.byref(batch.c), ptr(x_lig), ptr(h_lig), ptr(x_kp), h_lig.shape[1], ptr(coef2), ptr(step),
+                          int(u), ptr(noise), int(seed), _stream()), "kpd_renoise")
+
+
 def decode_atom_types(h_lig: torch.Tensor) -> torch.Tensor:
     """int32 [n] = argmax over the feature channels of every atom (lowest index wins ties, like torch.argmax on the
     CPU), on the device through kpd_decode_atom_types -- what the reference computes on the host right after sampling
@@ -414,15 +434,25 @@ def remove_com(batch: DeviceBatch, x_lig, x_kp, which: str):
 
 
 class Sampler:
-    """The captured reverse-diffusion loop for one (model, batch) pair (kpd_sampler)."""
+    """The captured reverse-diffusion loop for one (model, batch) pair (kpd_sampler).
+
+    resamplings >= 1 with inpaint_coef (schedule.inpaint_table on the device) makes it a fragment-conditioned
+    (inpainting) sampler: every reverse step runs `resamplings` denoiser passes with the atoms given to set_fragment
+    pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop."""
 
     def __init__(self, model: _Model, batch: DeviceBatch, gp: GraphParams, kk: Optional[Csr], coef: torch.Tensor,
                  T: int, atom_nf: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
-                 lig_feat_norm_constant: float = 1.0, atom_offset: int = 0, caps: Optional[Tuple[int, int]] = None):
+                 lig_feat_norm_constant: float = 1.0, atom_offset: int = 0, caps: Optional[Tuple[int, int]] = None,
+                 resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None):
         self.model, self.batch, self.gp, self.kk, self.coef = model, batch, gp, kk, coef
         _require_cuda(coef)
         self.T, self.atom_nf = int(T), int(atom_nf)
+        self.resamplings = int(resamplings)
+        if self.resamplings < 0 or (self.resamplings > 0) != (inpaint_coef is not None):
+            raise ValueError("an inpainting sampler needs resamplings >= 1 and inpaint_coef; a plain one neither")
         self.has_lk = bool(model.update_kp_feat if model.arch == 0 else model.update_kp)
+        if self.resamplings:        # about as many graph nodes per captured graph as the plain loop
+            steps_per_graph = max(1, int(steps_per_graph) // self.resamplings)
         steps_per_graph = max(1, min(int(steps_per_graph), self.T))
         self.cfg = KpdSamplerConfig(model.arch, self.T, self.atom_nf, steps_per_graph, int(bool(use_cuda_graph)),
                                     float(lig_feat_norm_constant))
@@ -439,6 +469,32 @@ class Sampler:
                                      cap_kl, ptr(self.ws), n, C.byref(self.handle)), "kpd_sampler_create")
         if atom_offset:     # this sampler holds a slice of a larger batch: keep the noise of the undivided batch
             check(lib.kpd_sampler_set_atom_offset(self.handle, int(atom_offset)), "kpd_sampler_set_atom_offset")
+        self.inpaint_coef = inpaint_coef
+        self._fragment = None
+        if self.resamplings:
+            _require_cuda(inpaint_coef)
+            check(lib.kpd_sampler_enable_inpainting(self.handle, self.resamplings, ptr(inpaint_coef)),
+                  "kpd_sampler_enable_inpainting")
+
+    def set_fragment(self, fixed_mask: Optional[torch.Tensor], x_fix: Optional[torch.Tensor],
+                     h_fix: Optional[torch.Tensor]):
+        """The atoms the next runs pin (inpainting samplers only): fixed_mask uint8 [n_lig] (nonzero = fixed; None = no
+        fixed atom), x_fix [n_lig,3] in the frame of the keypoints passed to run(), h_fix [n_lig,F] in the returned
+        feature space.  The tensors must stay alive and in place while runs use them (only their addresses are kept)."""
+        if fixed_mask is not None:
+            _require_cuda(fixed_mask, x_fix, h_fix)
+            assert fixed_mask.dtype == torch.uint8 and x_fix.dtype == torch.float32 and h_fix.dtype == torch.float32
+            assert fixed_mask.shape == (self.batch.n_lig,) and x_fix.shape == (self.batch.n_lig, 3)
+            assert h_fix.shape == (self.batch.n_lig, self.atom_nf)
+            assert fixed_mask.is_contiguous() and x_fix.is_contiguous() and h_fix.is_contiguous()
+        check(lib.kpd_sampler_set_fragment(self.handle, ptr(fixed_mask), ptr(x_fix), ptr(h_fix)),
+              "kpd_sampler_set_fragment")
+        self._fragment = (fixed_mask, x_fix, h_fix)
+
+    @property
+    def noise_slots(self) -> int:
+        """Slots of injected noise run() takes: T+1 (plain) or 1 + T*(3r-1) (inpainting with r resamplings)."""
+        return self.T + 1 if not self.resamplings else 1 + self.T * (3 * self.resamplings - 1)
 
     def __del__(self):
         if getattr(self, "handle", None) and self.handle.value and lib is not None:
@@ -457,7 +513,7 @@ class Sampler:
         n_steps = self.T if n_steps is None else int(n_steps)
         if noise is not None:
             _require_cuda(noise)
-            assert noise.shape == (self.T + 1, b.n_lig * (3 + self.atom_nf)) and noise.dtype == torch.float32
+            assert noise.shape == (self.noise_slots, b.n_lig * (3 + self.atom_nf)) and noise.dtype == torch.float32
         h_kp, init_lig_pos = _f32(h_kp), _f32(init_lig_pos)
         v_kp = _f32(v_kp) if v_kp is not None else None
         check(lib.kpd_sampler_run(self.handle, ptr(x_kp), ptr(h_kp), ptr(v_kp) if v_kp is not None else None,
@@ -564,11 +620,13 @@ def plan_capacity(lig_n: Sequence[int], kp_n: Sequence[int], n_kk_edges: int, gp
 
 class CapacitySampler:
     """A captured reverse-diffusion loop for one capacity bucket (see plan_capacity): owns its layout arrays, kk CSR and
-    input buffers; run() rewrites their CONTENTS for the batch at hand and replays the same CUDA graphs."""
+    input buffers; run() rewrites their CONTENTS for the batch at hand and replays the same CUDA graphs.  With
+    resamplings >= 1 (and inpaint_coef) it is an inpainting sampler that also owns zero-filled fragment buffers sized at
+    capacity: run(fragment=...) fills the rows of the real atoms; filler complexes and atoms are never fixed."""
 
     def __init__(self, model: _Model, plan: CapacityPlan, gp: GraphParams, coef: torch.Tensor, T: int, atom_nf: int,
                  kp_width: int, v_width: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
-                 lig_feat_norm_constant: float = 1.0):
+                 lig_feat_norm_constant: float = 1.0, resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None):
         B, N, K, max_lig, max_kp, cap_ll, cap_kl, cap_kk = plan.key
         dev = model.device
         self.key, self.model, self.atom_nf, self.T = plan.key, model, int(atom_nf), int(T)
@@ -581,18 +639,32 @@ class CapacitySampler:
         self.init_pos = torch.zeros(B, 3, dtype=torch.float32, device=dev)
         self.sampler = Sampler(model, self.batch, gp, self.kk, coef, T, atom_nf, steps_per_graph=steps_per_graph,
                                use_cuda_graph=use_cuda_graph, lig_feat_norm_constant=lig_feat_norm_constant,
-                               caps=(cap_ll, cap_kl))
+                               caps=(cap_ll, cap_kl), resamplings=resamplings, inpaint_coef=inpaint_coef)
+        if self.sampler.resamplings:
+            self.fixed_mask = torch.zeros(N, dtype=torch.uint8, device=dev)
+            self.x_fix = torch.zeros(N, 3, dtype=torch.float32, device=dev)
+            self.h_fix = torch.zeros(N, self.atom_nf, dtype=torch.float32, device=dev)
+            self.sampler.set_fragment(self.fixed_mask, self.x_fix, self.h_fix)
         self.runs = 0
 
     def run(self, plan: CapacityPlan, x_kp, h_kp, v_kp, kk_src, kk_dst, init_pos, seed: int, atom_offset: int = 0,
-            noise: Optional[torch.Tensor] = None, decode: bool = False):
+            noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None):
         """x_kp/h_kp/v_kp: the REAL keypoint rows (host or device tensors; pinned host tensors are uploaded straight
         into the capacity buffers); kk_src/kk_dst: kk edges in this batch's own keypoint numbering; init_pos [B_real,3].
+        fragment (inpainting samplers): (fixed_mask [N_real] bool, x_fix [N_real,3], h_fix [N_real,F]) or None.
         -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]]) on the device."""
         if plan.key != self.key:
             raise ValueError("CapacitySampler.run: the plan belongs to another capacity bucket")
+        if fragment is not None and not self.sampler.resamplings:
+            raise ValueError("CapacitySampler.run: a fragment needs an inpainting sampler")
         B_r, N_r, K_r = plan.n_real, plan.n_lig_real, plan.n_kp_real
         self.batch.set_layout(plan.lig_n, plan.kp_n)
+        if self.sampler.resamplings:     # rows past the real atoms stay zero: fillers are never fixed
+            self.fixed_mask.zero_()
+            if fragment is not None:
+                self.fixed_mask[:N_r].copy_(fragment[0], non_blocking=True)
+                self.x_fix[:N_r].copy_(fragment[1], non_blocking=True)
+                self.h_fix[:N_r].copy_(fragment[2], non_blocking=True)
         self.x_kp[:K_r].copy_(x_kp, non_blocking=True)
         self.h_kp[:K_r].copy_(h_kp, non_blocking=True)
         if self.v_kp is not None:

@@ -5,6 +5,8 @@ Mirrors PredefinedNoiseSchedule / polynomial_schedule / clip_noise_schedule of t
 round-trips through the checkpoint (SURVEY N9).  The table [T,4] = (alpha_t|s, var_terms,
 sigma, t) is what the CUDA step kernel reads; it restates models/ligand_diffuser.py:232-252 and
 :505-527 on the host, once per model (the values are identical for every complex of a batch).
+inpaint_table [T,4] = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) is the second table that
+fragment-conditioned sampling reads (DESIGN.md section 6.1).
 """
 import numpy as np
 import torch
@@ -87,4 +89,20 @@ def coefficient_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
         s2, s1, a = sigma_and_alpha_t_given_s(gt, gs)
         sig_s, sig_t = sigma(gs), sigma(gt)
         rows.append(torch.stack([a[0], (s2 / a / sig_t)[0], (s1 * sig_s / sig_t)[0], t[0].float()]))
+    return torch.stack(rows).contiguous()
+
+
+def inpaint_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
+    """fp32 [T,4] on the CPU; row s = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) with t = s+1: the known-part noising
+    and the re-noise coefficients of fragment-conditioned sampling.  Evaluated like coefficient_table (scalar fp32 ops,
+    row by row), so its alpha_t|s column equals coefficient_table's column 0 bit for bit."""
+    g = gamma.detach().float().cpu()
+    rows = []
+    for s_int in range(T):
+        s = torch.full((1,), s_int) / T
+        t = (torch.full((1,), s_int) + 1) / T
+        gs = g[torch.round(s * T).long()]
+        gt = g[torch.round(t * T).long()]
+        _, s1, a = sigma_and_alpha_t_given_s(gt, gs)
+        rows.append(torch.stack([alpha(gs)[0], sigma(gs)[0], a[0], s1[0]]))
     return torch.stack(rows).contiguous()
