@@ -1,6 +1,7 @@
-"""Teacher-forced parity cases at the SHIPPED hyper-parameters of every BASELINE.json config.
+"""Teacher-forced parity cases at the SHIPPED hyper-parameters of every shipped trained model.
 
-One builder for all five named configs (trained_models/{egnn_20kp, gvp_20kp, egnn_40kp, egnn_all_atom, gvp_ca}): seeded
+One builder for all eight (trained_models/{egnn_20kp, gvp_20kp, egnn_40kp, gvp_40kp, egnn_all_atom, gvp_all_atom,
+egnn_ca, gvp_ca}; the first five are the BASELINE.json configs): seeded
 weights in the reference state_dict layout (oracle/params.py; the checkpoints are not in the reference tree), the
 synthetic pocket kind SURVEY.md section 8d prescribes for the config, a handful of complexes of mixed ligand size so the
 CPU oracle stays cheap.  The hyper-parameters come from tests/golden/shipped_configs.yml, an extract of the reference's
@@ -22,6 +23,10 @@ SHIPPED = {
     "egnn_all_atom": ("all_atom", 336, [20, 33, 5], 2),
     # C-alpha pocket: 42 nodes >= 3.8 A apart, kk = rr radius 3.5 (empty), message_norm 'mean'
     "gvp_ca": ("ca", 42, [20, 1, 44, 9, 27], 2),
+    "gvp_40kp": ("keypoint", 40, [20, 8, 35, 60, 2, 27], 3),
+    # the only GVP model with hundreds of keypoints per complex: fixed encoder, kk := rr, message_norm 'mean'
+    "gvp_all_atom": ("all_atom", 336, [20, 33, 1, 5], 2),
+    "egnn_ca": ("ca", 42, [20, 1, 44, 9, 27], 2),
 }
 
 
@@ -69,8 +74,9 @@ def make_pockets(kind, n_nodes, rec_nf, vector_size, cut, n_pockets):
     if kind == "keypoint":
         return [synthetic.keypoint_pocket(i, n_nodes, rec_nf, vector_size, cut["kk"]) for i in range(n_pockets)]
     if kind == "all_atom":
-        return [synthetic.all_atom_pocket(i, n_nodes, rec_nf, vector_size, cut["rr"]) for i in range(n_pockets)]
-    pockets = [synthetic.ca_pocket(i, n_nodes, rec_nf, vector_size, cut["rr"]) for i in range(n_pockets)]
+        pockets = [synthetic.all_atom_pocket(i, n_nodes, rec_nf, vector_size, cut["rr"]) for i in range(n_pockets)]
+    else:
+        pockets = [synthetic.ca_pocket(i, n_nodes, rec_nf, vector_size, cut["rr"]) for i in range(n_pockets)]
     for i, pk in enumerate(pockets):       # the fixed encoder gives v_0 = 0; non-zero vectors exercise the kp vector path too
         if vector_size:
             pk.kp_v = 0.1 * torch.randn(pk.n_kp, vector_size, 3, generator=torch.Generator().manual_seed(50 + i))
@@ -98,7 +104,7 @@ def assemble_inputs(pockets, n_lig, atom_nf, seed, with_v):
 
 
 def shipped_case(name, n_lig=None):
-    """-> (arch, state_dict, ctor kwargs, rec_nf, flat inputs) for BASELINE config `name`."""
+    """-> (arch, state_dict, ctor kwargs, rec_nf, flat inputs) for shipped config `name`."""
     kind, n_nodes, sizes, n_pockets = SHIPPED[name]
     cfg = shipped_configs()[name]
     arch, kw, rec_nf = dynamics_kwargs(cfg)

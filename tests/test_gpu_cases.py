@@ -35,6 +35,7 @@ def _inputs(pockets, n_lig, atom_nf, seed, with_v):
 
 
 MODES = ["fp32", "bf16x3"]      # SIMT kernels / tcgen05 kernels with split bf16 operands: same 1e-4 bar
+TOL_BY_MODE = {"fp32": TOL, "bf16x3": TOL, "bf16": 3e-2}     # plain bf16 operands: 3e-2 of the output scale
 
 
 def _run_both(arch, sd, kw, atom_nf, rec_nf, inputs, tvals=(0.3,), per_complex_t=False, z_effective=False, mode="fp32"):
@@ -96,7 +97,7 @@ def test_egnn_all_atom_rows_span_many_tiles(mode):
     assert eh < TOL and ex < TOL
 
 
-@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("mode", MODES + ["bf16"])
 @pytest.mark.parametrize("norm", ["mean", 0, 10.0])
 def test_gvp_ca_like_empty_kk_and_norm_modes(norm, mode):
     """C-alpha style pocket: 42 nodes >= 3.8 A apart, kk = radius 3.5 graph => (almost) no kk edges, so
@@ -116,10 +117,10 @@ def test_gvp_ca_like_empty_kk_and_norm_modes(norm, mode):
     assert inputs["kk_src"].numel() < 8
     (eh, ex, _, _), = _run_both("gvp", sd, kw, 10, 10, inputs, mode=mode)
     print(f"gvp ca-like norm={norm} [{mode}]: rel_err {eh:.2e} {ex:.2e}")
-    assert eh < TOL and ex < TOL
+    assert eh < TOL_BY_MODE[mode] and ex < TOL_BY_MODE[mode]
 
 
-@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("mode", MODES + ["bf16"])
 @pytest.mark.parametrize("message_norm", [0.0, 3.0])
 def test_egnn_intended_normalisation_flag(message_norm, mode):
     """z_effective=True divides h_neigh / x_neigh by z (what the reference's comments intend, DESIGN N11)."""
@@ -130,12 +131,14 @@ def test_egnn_intended_normalisation_flag(message_norm, mode):
     sd = P.init_state_dict(P.egnn_dynamics_shapes(10, 24, 3, 48, True, True), seed=13, coord_gain=0.3)
     pockets = [synthetic.keypoint_pocket(i, 20, 24, 0, 8.0) for i in range(3)]
     inputs = _inputs(pockets, [20, 8, 35], 10, seed=6, with_v=False)
+    tol = TOL_BY_MODE[mode]
     res = _run_both("egnn", sd, kw, 10, 24, inputs, z_effective=True, per_complex_t=True, mode=mode)
     for eh, ex, _, _ in res:
-        assert eh < TOL and ex < TOL
+        print(f"egnn z_effective message_norm={message_norm} [{mode}] per-complex t: rel_err {eh:.2e} {ex:.2e}")
+        assert eh < tol and ex < tol
     # and the flag matters: the default (as-executed) result differs
     res0 = _run_both("egnn", sd, kw, 10, 24, inputs, z_effective=False, mode=mode)
-    assert res0[0][0] < TOL
+    assert res0[0][0] < tol
 
 
 def _module_case(arch):

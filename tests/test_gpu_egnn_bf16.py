@@ -137,7 +137,7 @@ def test_egnn_bf16_e3_properties_and_determinism_at_baseline_size():
 
 
 def _loop_sampler(model, fx, dev, use_graph=True):
-    """The injected-noise loop of the loop_egnn golden through the captured sampler."""
+    """The injected-noise loop of a loop_* golden (loop_egnn, loop_gvp) through the captured sampler."""
     from oracle import schedule as S
     from test_gpu_parity import device_inputs
     from keypoint_diffusion_b200 import ops
@@ -153,7 +153,7 @@ def _loop_sampler(model, fx, dev, use_graph=True):
         slots.append(torch.cat([nx.reshape(-1), nh.reshape(-1)]))
     noise = torch.stack(slots).to(dev).contiguous()
     sampler = ops.Sampler(model, batch, gp, kk, coef, T, F, steps_per_graph=4, use_cuda_graph=use_graph)
-    x_lig, h_lig, _ = sampler.run(t_in["kp_x"], t_in["kp_h"], None, fx["init_lig_pos"].to(dev), noise=noise)
+    x_lig, h_lig, _ = sampler.run(t_in["kp_x"], t_in["kp_h"], t_in.get("kp_v"), fx["init_lig_pos"].to(dev), noise=noise)
     torch.cuda.synchronize()
     return x_lig.cpu(), h_lig.cpu()
 

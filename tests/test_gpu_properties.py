@@ -115,7 +115,7 @@ def _forward(arch, model, gp, inputs, device_inputs, dev, tval=0.4):
     return eps_h.clone(), eps_x.clone(), es
 
 
-@pytest.mark.parametrize("mode", ["fp32", "bf16x3"])
+@pytest.mark.parametrize("mode", ["fp32", "bf16x3", "bf16"])
 @pytest.mark.parametrize("arch", ["egnn", "gvp"])
 def test_denoiser_is_e3_equivariant_at_baseline_size(arch, mode):
     dev = _dev()
@@ -136,11 +136,11 @@ def test_denoiser_is_e3_equivariant_at_baseline_size(arch, mode):
     eh = rel_err(h1.cpu(), h0.cpu())
     ex = rel_err(x1.cpu(), (x0.cpu().double() @ R.t()))
     print(f"{arch} [{mode}] equivariance at 100 ligands: invariance of eps_h {eh:.2e}, equivariance of eps_x {ex:.2e}")
-    tol = 2e-5 if mode == "fp32" else 1e-4
+    tol = {"fp32": 2e-5, "bf16x3": 1e-4, "bf16": 3e-2}[mode]     # bf16: operands rounded to an 8-bit mantissa
     assert eh < tol and ex < tol
 
 
-@pytest.mark.parametrize("mode", ["fp32", "bf16x3"])
+@pytest.mark.parametrize("mode", ["fp32", "bf16x3", "bf16"])
 @pytest.mark.parametrize("arch", ["egnn", "gvp"])
 def test_complexes_are_independent_and_runs_are_deterministic(arch, mode):
     dev = _dev()
@@ -164,8 +164,11 @@ def test_complexes_are_independent_and_runs_are_deterministic(arch, mode):
         hb, xb, _ = _forward(arch, model, gp, one, device_inputs, dev)
         eh = rel_err(hb.cpu(), h0[20 * b:20 * (b + 1)].cpu())
         ex = rel_err(xb.cpu(), x0[20 * b:20 * (b + 1)].cpu())
-        # same arithmetic per row; only the tile boundaries of the segmented reduction move
-        assert eh < 2e-5 and ex < 2e-5, (b, eh, ex)
+        # same arithmetic per row; only the tile boundaries of the segmented reduction move.  The EGNN's bf16 edge kernel
+        # rounds the (reassociated) fp32 node features to bf16 operands, so one rounding step can flip: measured <= 2.4e-4
+        print(f"{arch} [{mode}] complex {b} alone vs in the 100-ligand batch: rel_err eps_h {eh:.2e} eps_x {ex:.2e}")
+        tol = 5e-4 if (arch, mode) == ("egnn", "bf16") else 2e-5
+        assert eh < tol and ex < tol, (b, eh, ex)
 
 
 @pytest.mark.parametrize("mode", ["bf16x3", "bf16"])

@@ -1,6 +1,6 @@
-"""GPU parity at the SHIPPED width of every BASELINE.json config, in both parity-grade modes.
+"""GPU parity at the SHIPPED width of every shipped trained model, in both parity-grade modes.
 
-For each of trained_models/{egnn_20kp, gvp_20kp, egnn_40kp, egnn_all_atom, gvp_ca}: the CUDA denoiser (through the C
+For each of tests/shipped_cases.py:SHIPPED (all eight trained_models/*): the CUDA denoiser (through the C
 ABI) against the CPU oracle on the same seeded weights and inputs, teacher-forced at several t, in the fp32 SIMT mode
 and the bf16x3 tensor-core mode; the ll / kl / lk edge sets compared exactly.  Bars (stated here): edge sets exact;
 eps_h, eps_x max|a-b|/max|b| <= 1e-4 (north_star), RMS-relative <= 1e-4, per-channel max-relative <= 5e-4.
