@@ -327,8 +327,8 @@ struct kpd_egnn_model {
     const float* lig_enc[4]; const float* rec_enc[4]; const float* dec[4];
     std::vector<EgnnLayerW> layers;
     size_t edge_smem, edge_smem_ws[2];      // edge_smem_ws[nsplit - 1]
+    void (*edge_ws[2])(EgnnWsLaunch);       // [nsplit - 1]: the tensor-core edge kernel for H; null until kpd_egnn_attach_tc
     int mode;          // 0 = fp32 SIMT, 1 = bf16 tcgen05 (plain operands), 2 = bf16x3 tcgen05 (split operands, fp32-grade)
-    bool tc_ready[2];  // [nsplit - 1]
 };
 
 struct EgnnWs {
@@ -411,7 +411,7 @@ extern "C" int kpd_egnn_create(const kpd_egnn_config* cfg, const float* blob, co
     cudaError_t e = cudaFuncSetAttribute(egnn_edge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->edge_smem);
     if (e != cudaSuccess) { const size_t sm = m->edge_smem; delete m; KPD_REQUIRE(false, "kpd_egnn_create: cannot set %zu B shared memory: %s", sm, cudaGetErrorString(e)); }
     m->mode = 0;
-    m->tc_ready[0] = m->tc_ready[1] = false;
+    m->edge_ws[0] = m->edge_ws[1] = nullptr;
     m->edge_smem_ws[0] = egws::smem_bytes<1>(2 * cdiv(m->H, 16));
     m->edge_smem_ws[1] = egws::smem_bytes<2>(2 * cdiv(m->H, 16));
     *out = m;
@@ -443,16 +443,14 @@ extern "C" int kpd_egnn_attach_tc(kpd_egnn_model* m, const void* tc_blob, const 
             for (int br = 0; br < 2; ++br) T.W2P[e][br] = static_cast<const uint4*>(P());
         for (int nt = 0; nt < m->n_upd; ++nt) { T.Wn1P[nt] = P(); T.Wn2P[nt] = P(); }
     }
-    cudaError_t e;
-    if (nsplit == 1) {
-        e = cudaFuncSetAttribute(egnn_edge_ws_kernel<257, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(egnn_edge_ws_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    } else {
-        e = cudaFuncSetAttribute(egnn_edge_ws_kernel<257, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(egnn_edge_ws_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    }
+    // H = 257 (every shipped model) has a compile-time instantiation; the constants the kernel derives from HS = 257
+    // are exactly what kpd_egnn_forward passes for H = 257
+    void (*kernel)(EgnnWsLaunch);
+    if (nsplit == 1) kernel = m->H == 257 ? egnn_edge_ws_kernel<257, 1> : egnn_edge_ws_kernel<0, 1>;
+    else kernel = m->H == 257 ? egnn_edge_ws_kernel<257, 2> : egnn_edge_ws_kernel<0, 2>;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     KPD_REQUIRE(e == cudaSuccess, "kpd_egnn_attach_tc: cannot set %zu B shared memory: %s", smem, cudaGetErrorString(e));
-    m->tc_ready[nsplit - 1] = true;
+    m->edge_ws[nsplit - 1] = kernel;
     return 0;
 }
 
@@ -470,7 +468,7 @@ extern "C" int kpd_debug_eg_times(unsigned long long* out16) {
 extern "C" int kpd_egnn_set_mode(kpd_egnn_model* m, int32_t mode) {
     KPD_REQUIRE(m, "kpd_egnn_set_mode: null model");
     KPD_REQUIRE(mode >= 0 && mode <= 2, "kpd_egnn_set_mode: mode must be 0 (fp32 SIMT), 1 (bf16) or 2 (bf16x3 tensor cores)");
-    KPD_REQUIRE(mode == 0 || (m->tc_ready[mode - 1] && m->tc_ready[1]),
+    KPD_REQUIRE(mode == 0 || (m->edge_ws[mode - 1] && m->edge_ws[1]),
                 "kpd_egnn_set_mode: mode %d needs kpd_egnn_attach_tc(nsplit = 2)%s first", mode, mode == 1 ? " and (nsplit = 1)" : "");
     m->mode = mode;
     return 0;
@@ -590,16 +588,7 @@ extern "C" int kpd_egnn_forward(const kpd_egnn_model* m, const kpd_batch* b, con
             for (int e = 0; e < m->n_et; ++e)
                 for (int br = 0; br < 2; ++br) WL.t[e].W2P[br] = T.W2P[e][br];
             for (int e = 0; e < 4; ++e) WL.tile_off[e + 1] = WL.tile_off[e] + (e < m->n_et ? cdiv(caps[e] > 0 ? caps[e] : 1, egws::R) : 0);
-            // (the constants the kernel derives from HS = 257 are exactly what this function passes for H = 257)
-            const dim3 grid(WL.tile_off[4]);
-            const size_t smem = m->edge_smem_ws[m->mode - 1];
-            if (m->mode == 1) {
-                if (H == 257) egnn_edge_ws_kernel<257, 1><<<grid, egws::NT, smem, st>>>(WL);
-                else egnn_edge_ws_kernel<0, 1><<<grid, egws::NT, smem, st>>>(WL);
-            } else {
-                if (H == 257) egnn_edge_ws_kernel<257, 2><<<grid, egws::NT, smem, st>>>(WL);
-                else egnn_edge_ws_kernel<0, 2><<<grid, egws::NT, smem, st>>>(WL);
-            }
+            m->edge_ws[m->mode - 1]<<<dim3(WL.tile_off[4]), egws::NT, m->edge_smem_ws[m->mode - 1], st>>>(WL);
             KPD_TRY(check_launch("egnn_edge_ws_kernel"));
         } else {
             egnn_edge_kernel<<<dim3(max_tiles, m->n_et), NT, m->edge_smem, st>>>(L);

@@ -384,14 +384,50 @@ __global__ void __launch_bounds__(NT, 1) gvp_head_kernel(const GvpHeadArgs a) {
 
 using namespace kpd;
 
+// a kernel as kpd_gvp_forward launches it: `threads` per CTA, `rows` edges or nodes per CTA
+template <typename Arg>
+struct GvpKernel {
+    void (*fn)(Arg);
+    int threads;
+    size_t smem;
+    int rows;
+};
+
+// the kernels of one precision mode
+struct GvpKernels {
+    GvpKernel<GvpEdgeLaunch> edge;
+    GvpKernel<GvpNodeLaunch> node[2];   // [full_node_tiles] (kpd_gvp_forward)
+    GvpKernel<GvpHeadArgs> head[2];     // [full_node_tiles]
+};
+
+// the tensor-core kernels: edge tiles of configuration CE, node / head tiles of CN
+template <class CE, class CN>
+static GvpKernels gvp_ws_kernels(int kch) {
+    const size_t smem_n = ws::smem_bytes<CN>(kch);
+    return {{gvp_edge_ws_kernel<CE>, CE::NT, ws::smem_bytes<CE>(kch), CE::R},
+            {{gvp_node_ws_kernel<CN, NODE_ROWS>, CN::NT, smem_n, NODE_ROWS},
+             {gvp_node_ws_kernel<CN, NODE_ROWS_FULL>, CN::NT, smem_n, NODE_ROWS_FULL}},
+            {{gvp_head_ws_kernel<CN, NODE_ROWS>, CN::NT, smem_n, NODE_ROWS},
+             {gvp_head_ws_kernel<CN, NODE_ROWS_FULL>, CN::NT, smem_n, NODE_ROWS_FULL}}};
+}
+
+static cudaError_t gvp_set_smem(const GvpKernels& k) {
+    cudaError_t e = cudaFuncSetAttribute(k.edge.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.edge.smem);
+    for (int f = 0; f < 2 && e == cudaSuccess; ++f) {
+        e = cudaFuncSetAttribute(k.node[f].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.node[f].smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k.head[f].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.head[f].smem);
+    }
+    return e;
+}
+
 // launch, optionally with the highest stream priority as a launch attribute
 template <typename Arg>
-static void launch_with_priority(void (*kernel)(Arg), dim3 grid, int threads, size_t smem, cudaStream_t st, const Arg& arg,
+static void launch_with_priority(const GvpKernel<Arg>& k, dim3 grid, cudaStream_t st, const Arg& arg,
                                  bool high_priority = false) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = smem;
+    cfg.blockDim = dim3(k.threads);
+    cfg.dynamicSmemBytes = k.smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     int na = 0;
@@ -404,7 +440,7 @@ static void launch_with_priority(void (*kernel)(Arg), dim3 grid, int threads, si
     }
     cfg.attrs = attr;
     cfg.numAttrs = na;
-    cudaLaunchKernelEx(&cfg, kernel, arg);
+    cudaLaunchKernelEx(&cfg, k.fn, arg);
 }
 
 struct GvpLayerW {
@@ -421,12 +457,9 @@ struct kpd_gvp_model {
     std::vector<GvpLayerW> layers;
     GvpW head[MAXG];
     const float* WoT; const float* bo;
-    size_t smem, smem_node, smem_ws1, smem_ws2, smem_ws1n, smem_ks;
-    bool edge_ks;       // bf16x3: the edge kernel keeps (hi, lo) planes of 128-row tiles (WsKS) when that tile fits in 227 KB
-                        // of shared memory, and runs the 64-row stacked-operand kernel (WsSplit) otherwise
     int kch;           // k-chunks of the bf16 tile (tensor-core mode)
     int mode;          // 0 = fp32 SIMT, 1 = bf16 tcgen05, 2 = bf16x3 tcgen05 (split operands, fp32-grade)
-    bool tc_ready, tc2_ready;
+    GvpKernels k[3];   // [mode]: filled by kpd_gvp_create (0) and kpd_gvp_attach_tc (nsplit); edge.fn null until then
     std::vector<GvpW*> all_gvps;   // enumeration order of kpd_gvp_attach_tc
     // tensor-core modes: the layers run as a dependency graph over one stream per edge type (see kpd_gvp_forward);
     // created on first use
@@ -542,21 +575,15 @@ extern "C" int kpd_gvp_create(const kpd_gvp_config* cfg, const float* blob, cons
         int wmax = m->S + cfg->rbf_dim + m->V + 1;
         if (wmax < 64 + m->V) wmax = 64 + m->V;
         m->kch = 2 * ((wmax + 15) / 16);
-        m->smem_ws1 = ws::smem_bytes<WsBf16>(m->kch);
-        m->smem_ws2 = ws::smem_bytes<WsSplit>(m->kch);
-        m->smem_ws1n = ws::smem_bytes<WsBf16N>(m->kch);
-        m->smem_ks = ws::smem_bytes<WsKS>(m->kch);
-        m->edge_ks = m->smem_ks <= 227 * 1024;
         m->mode = 0;
-        m->tc_ready = false;
-        m->tc2_ready = false;
     }
-    m->smem = gvp_smem_bytes(m->lds, TE);
-    m->smem_node = gvp_smem_bytes(m->lds, TN);
-    cudaError_t e1 = cudaFuncSetAttribute(gvp_edge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem);
-    cudaError_t e2 = cudaFuncSetAttribute(gvp_node_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_node);
-    cudaError_t e3 = cudaFuncSetAttribute(gvp_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_node);
-    if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess) {
+    // fp32 SIMT: one node / head tile size whatever the batch
+    const size_t smem_node = gvp_smem_bytes(m->lds, TN);
+    GvpKernels& k0 = m->k[0];
+    k0.edge = {gvp_edge_kernel, NT, gvp_smem_bytes(m->lds, TE), TE};
+    k0.node[0] = k0.node[1] = {gvp_node_kernel, NT, smem_node, TN};
+    k0.head[0] = k0.head[1] = {gvp_head_kernel, NT, smem_node, TN};
+    if (gvp_set_smem(k0) != cudaSuccess) {
         delete m;
         KPD_REQUIRE(false, "kpd_gvp_create: cannot set the dynamic shared memory size of the GVP kernels");
     }
@@ -599,8 +626,10 @@ extern "C" int kpd_gvp_attach_tc(kpd_gvp_model* m, const void* tc_blob, const in
     KPD_REQUIRE(n == 3 * (int)m->all_gvps.size(), "kpd_gvp_attach_tc: expected %d offsets, got %d", 3 * (int)m->all_gvps.size(), n);
     KPD_REQUIRE((reinterpret_cast<uintptr_t>(tc_blob) & 127) == 0, "kpd_gvp_attach_tc: blob must be 128-byte aligned");
     KPD_REQUIRE(m->S % 16 == 0, "kpd_gvp_attach_tc: n_hidden_scalars must be a multiple of 16 for the tensor-core mode");
-    KPD_REQUIRE(m->smem_ws1 <= 227 * 1024 && m->smem_ws2 <= 227 * 1024 && m->smem_ws1n <= 227 * 1024,
-                "kpd_gvp_attach_tc: tile needs %zu / %zu / %zu B of shared memory", m->smem_ws1, m->smem_ws2, m->smem_ws1n);
+    const size_t smem_ws1 = ws::smem_bytes<WsBf16>(m->kch), smem_ws2 = ws::smem_bytes<WsSplit>(m->kch),
+                 smem_ws1n = ws::smem_bytes<WsBf16N>(m->kch);
+    KPD_REQUIRE(smem_ws1 <= 227 * 1024 && smem_ws2 <= 227 * 1024 && smem_ws1n <= 227 * 1024,
+                "kpd_gvp_attach_tc: tile needs %zu / %zu / %zu B of shared memory", smem_ws1, smem_ws2, smem_ws1n);
     const char* base = static_cast<const char*>(tc_blob);
     for (size_t i = 0; i < m->all_gvps.size(); ++i) {
         KPD_REQUIRE(byte_offsets[3 * i] % 16 == 0 && byte_offsets[3 * i + 1] % 16 == 0 && byte_offsets[3 * i + 2] % 16 == 0,
@@ -618,26 +647,14 @@ extern "C" int kpd_gvp_attach_tc(kpd_gvp_model* m, const void* tc_blob, const in
             gw->WgP2c = reinterpret_cast<const uint4*>(reinterpret_cast<const char*>(wg) + (size_t)ksg * 1024);
         }
     }
-    if (nsplit == 2) {
-        cudaError_t e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsSplit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        if (e == cudaSuccess && m->edge_ks) e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsKS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ks);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_node_ws_kernel<WsSplit, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_head_ws_kernel<WsSplit, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_node_ws_kernel<WsSplit, NODE_ROWS_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_head_ws_kernel<WsSplit, NODE_ROWS_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws2);
-        KPD_REQUIRE(e == cudaSuccess, "kpd_gvp_attach_tc: cannot set %zu B of dynamic shared memory", m->smem_ws2);
-        m->tc2_ready = true;
-        return gvp_dag_init(m);
-    }
-    {
-        cudaError_t e = cudaFuncSetAttribute(gvp_edge_ws_kernel<WsBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws1);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_node_ws_kernel<WsBf16N, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws1n);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_head_ws_kernel<WsBf16N, NODE_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws1n);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_node_ws_kernel<WsBf16N, NODE_ROWS_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws1n);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(gvp_head_ws_kernel<WsBf16N, NODE_ROWS_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_ws1n);
-        KPD_REQUIRE(e == cudaSuccess, "kpd_gvp_attach_tc: cannot set %zu B of dynamic shared memory", m->smem_ws1);
-    }
-    m->tc_ready = true;
+    // bf16x3: the edge kernel keeps (hi, lo) planes of 128-row tiles (WsKS) when that tile fits in 227 KB of shared
+    // memory, and runs the 64-row stacked-operand kernel (WsSplit) otherwise
+    const GvpKernels k = nsplit == 1 ? gvp_ws_kernels<WsBf16, WsBf16N>(m->kch)
+                       : ws::smem_bytes<WsKS>(m->kch) <= 227 * 1024 ? gvp_ws_kernels<WsKS, WsSplit>(m->kch)
+                                                                   : gvp_ws_kernels<WsSplit, WsSplit>(m->kch);
+    KPD_REQUIRE(gvp_set_smem(k) == cudaSuccess, "kpd_gvp_attach_tc: cannot set %zu / %zu B of dynamic shared memory",
+                k.edge.smem, k.node[0].smem);
+    m->k[nsplit] = k;
     return gvp_dag_init(m);
 }
 
@@ -694,8 +711,7 @@ extern "C" int kpd_debug_ws_times(unsigned long long* out64) {
 extern "C" int kpd_gvp_set_mode(kpd_gvp_model* m, int32_t mode) {
     KPD_REQUIRE(m, "kpd_gvp_set_mode: null model");
     KPD_REQUIRE(mode >= 0 && mode <= 2, "kpd_gvp_set_mode: mode must be 0 (fp32 SIMT), 1 (bf16) or 2 (bf16x3 tensor cores)");
-    KPD_REQUIRE(mode != 1 || m->tc_ready, "kpd_gvp_set_mode: call kpd_gvp_attach_tc(nsplit = 1) first");
-    KPD_REQUIRE(mode != 2 || m->tc2_ready, "kpd_gvp_set_mode: call kpd_gvp_attach_tc(nsplit = 2) first");
+    KPD_REQUIRE(m->k[mode].edge.fn, "kpd_gvp_set_mode: call kpd_gvp_attach_tc(nsplit = %d) first", mode);
     m->mode = mode;
     return 0;
 }
@@ -763,7 +779,7 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
     const int src_nt[4] = {0, 1, 0, 1}, dst_nt[4] = {0, 0, 1, 1};
     const float* X[2] = {x_lig, x_kp};
     const int norm_mode = m->cfg.norm_mode;
-    const int edge_rows = m->mode == 1 ? WsBf16::R : m->mode == 2 ? (m->edge_ks ? WsKS::R : WsSplit::R) : TE;
+    const GvpKernels& K = m->k[m->mode];
 
     // Tensor-core modes run the convs as a DEPENDENCY GRAPH instead of a chain of launches: one edge launch per edge
     // type, one node launch per node type, each waiting only for what it reads --
@@ -774,7 +790,8 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
     // node kernel never overwrites what a still-running edge kernel of the same conv reads.  The point: a conv's
     // 650 edge tiles are 4.4 waves of one CTA per SM and its node tiles a fifth of a wave; as separate launches their
     // tails leave SMs idle, as a graph the tail of one kernel is filled with the CTAs of the next ready one.
-    // The CUDA-event profiler (bench.py's roofline leg) and KPD_GVP_SERIAL=1 use the serial path below.
+    // The fp32 mode, the CUDA-event profiler (bench.py's roofline leg) and KPD_GVP_SERIAL=1 run the convs serially:
+    // one launch for all edge types of a conv and one for all its node types, on the caller's stream.
     const bool dag = m->mode != 0 && !m->serial && !prof_enabled();
     if (dag) KPD_TRY(gvp_dag_init(m));       // normally done by kpd_gvp_attach_tc, outside any stream capture
     // stream of edge type e (ll, kl, lk, kk) and of node type nt
@@ -796,16 +813,10 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
         for (int k = 0; k < L.n_msg; ++k) a.msg[k] = W.msg[e][k];
         a.sm = w.sm[cur][e]; a.vm = w.vm[cur][e]; a.part = w.part[cur][e];
     };
-    auto launch_edge_ws = [&](const GvpEdgeLaunch& L, int tiles, int n_et, cudaStream_t s_) -> int {
-        if (m->mode == 1) launch_with_priority(gvp_edge_ws_kernel<WsBf16>, dim3(tiles, n_et), WsBf16::NT, m->smem_ws1, s_, L);
-        else if (m->edge_ks) launch_with_priority(gvp_edge_ws_kernel<WsKS>, dim3(tiles, n_et), WsKS::NT, m->smem_ks, s_, L);
-        else launch_with_priority(gvp_edge_ws_kernel<WsSplit>, dim3(tiles, n_et), WsSplit::NT, m->smem_ws2, s_, L);
-        return check_launch("gvp_edge_ws_kernel");
-    };
     auto fill_node = [&](GvpNodeLaunch& NL, int slot, int nt, const GvpLayerW& W, int cur, int nxt) {
         GvpNodeArgs& a = NL.nt[slot];
         a.n = N[nt]; a.Sdim = S; a.Vdim = V; a.lds = m->lds; a.pw = m->pw;
-        a.n_upd = m->cfg.n_update_gvps; a.n_et = 2; a.kch = m->kch; a.edge_tile = edge_rows;
+        a.n_upd = m->cfg.n_update_gvps; a.n_et = 2; a.kch = m->kch; a.edge_tile = K.edge.rows;
         a.s = w.s[cur][nt]; a.v = w.v[cur][nt]; a.s_hi = w.s_hi[cur][nt]; a.s_lo = w.s_lo[cur][nt];
         a.s_out = w.s[nxt][nt]; a.v_out = w.v[nxt][nt]; a.s_hi_out = w.s_hi[nxt][nt]; a.s_lo_out = w.s_lo[nxt][nt];
         for (int k = 0; k < 2; ++k) {
@@ -824,24 +835,15 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
     // siblings and SM time, not the critical path, is what counts (gvp_ws.inl: NODE_ROWS; measured: headline, groups of 25:
     // 89.3 -> 92.1 ligands/s; gvp_ca with 16 ligands in one group: 33.1 with 32-row tiles, 29.9 with 64)
     const bool full_node_tiles = b->B >= 32;
-    const int node_rows = full_node_tiles ? NODE_ROWS_FULL : NODE_ROWS;
-    auto launch_node_ws = [&](const GvpNodeLaunch& NL, int max_n, int n_dst, cudaStream_t s_) -> int {
-        const dim3 grid(cdiv(max_n, node_rows), n_dst);
-        if (m->mode == 1) {
-            if (full_node_tiles) launch_with_priority(gvp_node_ws_kernel<WsBf16N, NODE_ROWS_FULL>, grid, WsBf16N::NT, m->smem_ws1n, s_, NL, dag);
-            else launch_with_priority(gvp_node_ws_kernel<WsBf16N, NODE_ROWS>, grid, WsBf16N::NT, m->smem_ws1n, s_, NL, dag);
-        } else {
-            if (full_node_tiles) launch_with_priority(gvp_node_ws_kernel<WsSplit, NODE_ROWS_FULL>, grid, WsSplit::NT, m->smem_ws2, s_, NL, dag);
-            else launch_with_priority(gvp_node_ws_kernel<WsSplit, NODE_ROWS>, grid, WsSplit::NT, m->smem_ws2, s_, NL, dag);
-        }
-        return check_launch("gvp_node_ws_kernel");
-    };
+    const GvpKernel<GvpNodeLaunch>& node_k = K.node[full_node_tiles];
 
     int fin = 0;        // buffer set holding the final ligand features
     for (int l = 0; l < m->cfg.n_convs; ++l) {
         const GvpLayerW& W = m->layers[l];
         // serial paths update in place (set 0); the graph path ping-pongs
         const int cur = dag ? (l & 1) : 0, nxt = dag ? ((l + 1) & 1) : 0;
+        // launch groups: the graph path launches each edge / node type on its own, the serial path all of them at once
+        const int eg = dag ? 1 : W.n_et, ng = dag ? 1 : W.n_dst;
         GvpEdgeLaunch L;
         memset(&L, 0, sizeof(L));
         L.Sdim = S; L.Vdim = V; L.n_msg = m->cfg.n_message_gvps; L.lds = m->lds; L.pw = m->pw;
@@ -849,68 +851,48 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
         L.rbf_step = m->cfg.rbf_dmax / (float)(m->cfg.rbf_dim - 1);   // linspace(0, D_max, D_count)
         L.rbf_sigma = m->cfg.rbf_dmax / (float)m->cfg.rbf_dim;
         L.kch = m->kch;
-        if (dag) {
-            for (int e = 0; e < W.n_et; ++e) {
-                GvpEdgeLaunch Le = L;
-                Le.tl_slot = 8 * l + e;
-                fill_edge(Le, 0, e, W, cur);
-                KPD_CU(cudaStreamWaitEvent(es[e], m->ev_node[src_nt[e]], 0));
-                KPD_TRY(launch_edge_ws(Le, cdiv(caps[e] > 0 ? caps[e] : 1, edge_rows), 1, es[e]));
-                KPD_CU(cudaEventRecord(m->ev_edge[e], es[e]));
-                used[e] = true;
+        for (int e0 = 0; e0 < W.n_et; e0 += eg) {
+            GvpEdgeLaunch Lg = L;
+            Lg.tl_slot = 8 * l + e0;
+            int cap = 1;
+            for (int e = e0; e < e0 + eg; ++e) {
+                fill_edge(Lg, e - e0, e, W, cur);
+                if (caps[e] > cap) cap = caps[e];
+                if (dag) KPD_CU(cudaStreamWaitEvent(es[e], m->ev_node[src_nt[e]], 0));
             }
-            for (int nt = 0; nt < W.n_dst; ++nt) {
-                if (N[nt] <= 0) continue;
-                GvpNodeLaunch NL;
-                memset(&NL, 0, sizeof(NL));
-                fill_node(NL, 0, nt, W, cur, nxt);
-                NL.tl_slot = 8 * l + 4 + nt;
-                for (int k = 0; k < 2; ++k) KPD_CU(cudaStreamWaitEvent(ns[nt], m->ev_edge[2 * nt + k], 0));
-                KPD_TRY(launch_node_ws(NL, N[nt], 1, ns[nt]));
-                KPD_CU(cudaEventRecord(m->ev_node[nt], ns[nt]));
-                nused[nt] = true;
+            prof_begin(PROF_GVP_EDGE, es[e0]);
+            launch_with_priority(K.edge, dim3(cdiv(cap, K.edge.rows), eg), es[e0], Lg);
+            KPD_TRY(check_launch("gvp edge kernel"));
+            prof_end(PROF_GVP_EDGE, es[e0]);
+            if (dag) {
+                KPD_CU(cudaEventRecord(m->ev_edge[e0], es[e0]));
+                used[e0] = true;
             }
-            // a node type this conv does not update (the last conv is lig-only) simply keeps its current set; nothing
-            // reads it afterwards (dynamics_gvp.py:71-72)
-            fin = nxt;
-            continue;
         }
-        int max_tiles = 1, tiles_tc = 1;
-        L.tl_slot = 8 * l;
-        for (int e = 0; e < W.n_et; ++e) {
-            fill_edge(L, e, e, W, cur);
-            const int c1 = caps[e] > 0 ? caps[e] : 1;
-            if (cdiv(c1, TE) > max_tiles) max_tiles = cdiv(c1, TE);
-            if (cdiv(c1, edge_rows) > tiles_tc) tiles_tc = cdiv(c1, edge_rows);
-        }
-        prof_begin(PROF_GVP_EDGE, st);
-        if (m->mode != 0) {
-            KPD_TRY(launch_edge_ws(L, tiles_tc, W.n_et, st));
-        } else {
-            gvp_edge_kernel<<<dim3(max_tiles, W.n_et), NT, m->smem, st>>>(L);
-            KPD_TRY(check_launch("gvp_edge_kernel"));
-        }
-        prof_end(PROF_GVP_EDGE, st);
-        {
+        for (int nt0 = 0; nt0 < W.n_dst; nt0 += ng) {
             GvpNodeLaunch NL;
             memset(&NL, 0, sizeof(NL));
-            NL.tl_slot = 8 * l + 4;
+            NL.tl_slot = 8 * l + 4 + nt0;
             int max_n = 0;
-            for (int nt = 0; nt < W.n_dst; ++nt) {
-                fill_node(NL, nt, nt, W, cur, nxt);
+            for (int nt = nt0; nt < nt0 + ng; ++nt) {
+                fill_node(NL, nt - nt0, nt, W, cur, nxt);
                 if (N[nt] > max_n) max_n = N[nt];
             }
-            if (max_n > 0) {
-                prof_begin(PROF_GVP_NODE, st);
-                if (m->mode != 0) {
-                    KPD_TRY(launch_node_ws(NL, max_n, W.n_dst, st));
-                } else {
-                    gvp_node_kernel<<<dim3(cdiv(max_n, TN), W.n_dst), NT, m->smem_node, st>>>(NL);
-                    KPD_TRY(check_launch("gvp_node_kernel"));
-                }
-                prof_end(PROF_GVP_NODE, st);
+            if (max_n <= 0) continue;
+            if (dag)
+                for (int k = 0; k < 2; ++k) KPD_CU(cudaStreamWaitEvent(ns[nt0], m->ev_edge[2 * nt0 + k], 0));
+            prof_begin(PROF_GVP_NODE, ns[nt0]);
+            launch_with_priority(node_k, dim3(cdiv(max_n, node_k.rows), ng), ns[nt0], NL, dag);
+            KPD_TRY(check_launch("gvp node kernel"));
+            prof_end(PROF_GVP_NODE, ns[nt0]);
+            if (dag) {
+                KPD_CU(cudaEventRecord(m->ev_node[nt0], ns[nt0]));
+                nused[nt0] = true;
             }
         }
+        // graph path: a node type this conv does not update (the last conv is lig-only) simply keeps its current set;
+        // nothing reads it afterwards (dynamics_gvp.py:71-72)
+        fin = nxt;
     }
     if (dag) {
         // join: everything launched on the auxiliary streams is ordered before the head / the end of this call
@@ -929,18 +911,9 @@ extern "C" int kpd_gvp_forward(const kpd_gvp_model* m, const kpd_batch* b, const
         if (a.n > 0) {
             prof_begin(PROF_GVP_HEAD, st);
             a.kch = m->kch;
-            if (m->mode == 1) {
-                if (full_node_tiles) launch_with_priority(gvp_head_ws_kernel<WsBf16N, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, a);
-                else launch_with_priority(gvp_head_ws_kernel<WsBf16N, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsBf16N::NT, m->smem_ws1n, st, a);
-                KPD_TRY(check_launch("gvp_head_ws_kernel"));
-            } else if (m->mode == 2) {
-                if (full_node_tiles) launch_with_priority(gvp_head_ws_kernel<WsSplit, NODE_ROWS_FULL>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, a);
-                else launch_with_priority(gvp_head_ws_kernel<WsSplit, NODE_ROWS>, dim3(cdiv(a.n, node_rows)), WsSplit::NT, m->smem_ws2, st, a);
-                KPD_TRY(check_launch("gvp_head_ws_kernel"));
-            } else {
-                gvp_head_kernel<<<cdiv(a.n, TN), NT, m->smem_node, st>>>(a);
-                KPD_TRY(check_launch("gvp_head_kernel"));
-            }
+            const GvpKernel<GvpHeadArgs>& head_k = K.head[full_node_tiles];
+            launch_with_priority(head_k, dim3(cdiv(a.n, head_k.rows)), st, a);
+            KPD_TRY(check_launch("gvp head kernel"));
             prof_end(PROF_GVP_HEAD, st);
         }
     }

@@ -146,7 +146,7 @@ def test_oracle_parity_across_the_32_complex_node_tile_switch(arch, mode):
 
 # (n_hidden_scalars, rbf_dim, message_norm) -> edge tile of each mode: fp32 SIMT 64 rows; bf16 128; bf16x3 the 128-row
 # KS kernel, except at S = 256, rbf_dim = 32 where its tile does not fit in shared memory and the stacked 64-row
-# kernel runs (gvp.cu: edge_ks).  Shipped width S = 256: at S = 64 the vector output of this case is ~5x worse
+# kernel runs (gvp.cu: kpd_gvp_attach_tc).  Shipped width S = 256: at S = 64 the vector output of this case is ~5x worse
 # conditioned in every mode, and bf16 lands at 3.3e-2.
 MANY_TILE_CASES = {"S256_mean": (256, 16, "mean", {"fp32": 64, "bf16": 128, "bf16x3": 128}),
                    "S256_rbf32_zero": (256, 32, 0, {"fp32": 64, "bf16": 128, "bf16x3": 64})}
