@@ -275,6 +275,20 @@ int kpd_renoise(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_kp,
                 const float* coef2, const int32_t* step_ptr, int32_t u, const float* noise, uint64_t seed,
                 void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * (e'') Start of a run from a given ligand (ligand optimisation by partial noising, SDEdit-style;
+ * an extension beyond the reference, DESIGN.md section 6.2).  One CTA per complex:
+ *   c_b  = mean of x_start over the complex's atoms; x_kp -= c_b
+ *   z_x  = alpha*(x_start - c_b) + sigma*e_x,  z_h = alpha*h_start/lig_feat_norm_constant + sigma*e_h
+ *   then the ligand COM is removed from ligand and keypoints.
+ * alpha / sigma = alpha_t0 / sigma_t0 (schedule.start_coefficients).  noise: NULL -> the Philox draw of
+ * kpd_randn_init (seed, step = -1, atom, channel), or injected [n_lig*(3+atom_nf)], x channels first.
+ * Writes x_lig [n_lig,3], h_lig [n_lig,atom_nf]; updates x_kp in place.
+ * ------------------------------------------------------------------------------------------ */
+int kpd_partial_noise(const kpd_batch* batch, const float* x_start, const float* h_start, float* x_lig,
+                      float* h_lig, float* x_kp, int32_t atom_nf, float alpha, float sigma,
+                      float lig_feat_norm_constant, const float* noise, uint64_t seed, void* stream);
+
 /* remove_com (ligand_diffuser.py:185-203): which = 0 ligand COM, 1 keypoint COM; shifts both
  * node types.  If com_out != NULL the [B,3] means are also written there. */
 int kpd_remove_com(const kpd_batch* batch, float* x_lig, float* x_kp, int32_t which,
@@ -291,7 +305,9 @@ int kpd_randn_init(float* x_lig, float* h_lig, int32_t n_lig, int32_t atom_nf, u
  * The whole loop.  Replaces the body of KeypointDiffusion.sample_from_encoded_receptors
  * (models/ligand_diffuser.py:342-447, visualize=False): frame setup, T reverse steps (graph
  * build + denoiser + posterior step each), frame restore.  The per-step kernel sequence is
- * captured once into a CUDA graph of `steps_per_graph` steps and replayed.
+ * captured once into a CUDA graph of `steps_per_graph` steps and replayed.  With a start ligand
+ * (kpd_sampler_set_start) the frame setup is kpd_partial_noise and the loop runs t0 steps from
+ * step t0 - 1 down, through the same captured graphs.
  * ------------------------------------------------------------------------------------------ */
 typedef struct kpd_sampler kpd_sampler;
 
@@ -316,10 +332,14 @@ int64_t kpd_sampler_workspace_bytes(const kpd_sampler_config* cfg, const void* m
 void kpd_sampler_destroy(kpd_sampler* s);
 
 /* Runs the loop.  x_kp/h_kp/v_kp: encoded keypoints (x_kp is modified in place and restored
- * to the input frame); init_lig_pos [B,3]; x_lig/h_lig: outputs [n_lig,3]/[n_lig,atom_nf].
- * noise: NULL (Philox, `seed`) or device fp32 [(T+1), n_lig, 3+atom_nf] with slot 0 = initial
- * draw and slot 1+k = the k-th executed step (s = T-1-k), x channels first.
- * n_steps: reverse steps to run (T for a full sample; fewer only for testing). */
+ * to the input frame); init_lig_pos [B,3] (not read in a run from a start ligand, but still
+ * required); x_lig/h_lig: outputs [n_lig,3]/[n_lig,atom_nf].
+ * noise: NULL (Philox, `seed`) or device fp32 [(t0+1), n_lig, 3+atom_nf] with slot 0 = initial
+ * draw and slot 1+k = the k-th executed step (s = t0-1-k), x channels first; t0 = T, or the
+ * start step of kpd_sampler_set_start.  An inpainting sampler takes 1 + t0*(3r-1) slots.
+ * n_steps: reverse steps to run, at most t0 (t0 for a full sample; fewer only for testing).
+ * Graph replays cover floor(n_steps / steps_per_graph) * steps_per_graph steps; the rest run
+ * as stream launches. */
 int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, const float* v_kp,
                     const float* init_lig_pos, float* x_lig, float* h_lig, const float* noise,
                     uint64_t seed, int32_t n_steps, void* stream);
@@ -344,6 +364,16 @@ int kpd_sampler_enable_inpainting(kpd_sampler* s, int32_t resamplings, const flo
  * the returned feature space.  Only pointers are kept; each run uploads them to device memory, so a
  * captured sampler follows new buffers without capturing again. */
 int kpd_sampler_set_fragment(kpd_sampler* s, const uint8_t* fixed_mask, const float* x_fix, const float* h_fix);
+/* The start of the next runs (ligand optimisation by partial noising, DESIGN.md section 6.2):
+ * x_start [n_lig,3] in the frame of the x_kp passed to kpd_sampler_run, h_start [n_lig,atom_nf] in
+ * the returned feature space, noised to step start_step (in [0, T]) with alpha / sigma =
+ * alpha_t0 / sigma_t0 (HOST floats, schedule.start_coefficients) by kpd_partial_noise; the runs
+ * then execute reverse steps start_step-1 .. 0.  x_start = NULL restores the plain start from
+ * pure noise at step T.  Works for plain and inpainting samplers.  Only pointers are kept and each
+ * run reads them, so a captured sampler follows new buffers and any start_step without capturing
+ * again. */
+int kpd_sampler_set_start(kpd_sampler* s, int32_t start_step, const float* x_start, const float* h_start,
+                          float alpha, float sigma);
 
 /* Output decode, the step right behind the path (reference test.py:199-203: torch.argmax(lig_feat, dim=1) on the
  * host, then dataset.lig_atom_idx_to_element): atom_type[i] = argmax_c h_lig[i, c], lowest index on ties. */

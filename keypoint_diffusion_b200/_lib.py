@@ -105,6 +105,8 @@ def _load():
         "kpd_sampler_set_atom_offset": (I, [P, I]),
         "kpd_sampler_enable_inpainting": (I, [P, I, P]),
         "kpd_sampler_set_fragment": (I, [P, P, P, P]),
+        "kpd_sampler_set_start": (I, [P, I, P, P, F, F]),
+        "kpd_partial_noise": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, F, F, F, P, U64, P]),
         "kpd_decode_atom_types": (I, [P, I, I, P, P]),
     }
     for name, (res, args) in sig.items():

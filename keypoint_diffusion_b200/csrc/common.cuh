@@ -230,8 +230,9 @@ int launch_sub(const float* a, const float* b, float* out, int n, cudaStream_t s
 struct RunParams {        // lives in device memory so that a captured graph can be re-pointed
     const float* noise;   // NULL or [(T+1)][n_lig][3+F], slot 0 = initial draw
     uint64_t seed;
-    int T;
-    int atom_offset;      // added to the atom index of the Philox counter: a batch sampled as several sub-batches draws
+    int T;                // the step the run starts from (the sampler's T, or t0 of a run from a start ligand): the
+                          // injected-noise slots of executed steps are counted from it
+    int atom_offset;     // added to the atom index of the Philox counter: a batch sampled as several sub-batches draws
                           // the same noise as when it is sampled whole (kpd_sampler_set_atom_offset)
 };
 int launch_ddpm_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
@@ -259,6 +260,12 @@ int launch_ddpm_inpaint_step(const kpd_batch* b, float* x_lig, float* h_lig, flo
 int launch_renoise(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, int F, const int* step_ptr, int u, int r,
                    const float* coef2, const InpaintParams* ip, const float* noise, uint64_t seed, const RunParams* rp,
                    cudaStream_t st);
+// ------------------------------------------------------------------ partial noising of a start ligand (partial_noise.cu)
+// noise: NULL or [n_lig][3+F] (x first) for the stand-alone call; with rp (a sampler's run) seed, noise slot 0 and the
+// atom offset come from device memory instead
+int launch_partial_noise(const kpd_batch* b, const float* x_start, const float* h_start, float* x_lig, float* h_lig,
+                         float* x_kp, int F, float alpha, float sigma, float norm_c, const float* noise, uint64_t seed,
+                         const RunParams* rp, cudaStream_t st);
 long long launch_count();  // kernels launched through check_launch() so far (this process)
 
 // optional per-kernel CUDA-event timing (bench.py's roofline leg); no-ops unless enabled and

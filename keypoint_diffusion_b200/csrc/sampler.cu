@@ -10,6 +10,8 @@
 // times; the step index lives on the device and is decremented by step_prologue.  An inpainting sampler
 // (kpd_sampler_enable_inpainting) runs r passes per step instead:
 //     step_prologue -> r x (graph_mark/scan/fill -> denoiser -> ddpm_inpaint_step [-> renoise])
+// A run from a start ligand (kpd_sampler_set_start) replaces the frame setup by one partial_noise launch and starts the
+// step counter at t0 instead of T; the captured graphs do not depend on the step, so they serve any t0.
 #include "common.cuh"
 #include <string.h>
 
@@ -42,6 +44,10 @@ struct kpd_sampler {
     int resamplings;
     InpaintParams frag;       // host copy, uploaded to frag_dev by every run
     InpaintParams* frag_dev;
+    // partial noising (kpd_sampler_set_start): x_start == NULL = the plain start from pure noise at step T
+    const float *x_start, *h_start;
+    int start_step;
+    float start_alpha, start_sigma;
 };
 
 static int64_t model_ws_bytes(const kpd_sampler_config* cfg, const void* model, const kpd_batch* b, int cap_ll,
@@ -223,6 +229,17 @@ extern "C" int kpd_sampler_set_fragment(kpd_sampler* s, const uint8_t* fixed_mas
     return 0;
 }
 
+extern "C" int kpd_sampler_set_start(kpd_sampler* s, int32_t start_step, const float* x_start, const float* h_start,
+                                     float alpha, float sigma) {
+    KPD_REQUIRE(s, "kpd_sampler_set_start: null sampler");
+    KPD_REQUIRE(!x_start || (h_start && start_step >= 0 && start_step <= s->cfg.T),
+                "kpd_sampler_set_start: a start ligand needs h_start and a start step in [0, T]");
+    s->x_start = x_start; s->h_start = x_start ? h_start : nullptr;
+    s->start_step = x_start ? start_step : 0;
+    s->start_alpha = alpha; s->start_sigma = sigma;
+    return 0;
+}
+
 static int enqueue_any_step(kpd_sampler* s, cudaStream_t st) {
     return s->resamplings ? enqueue_inpaint_step(s, st) : enqueue_step(s, st);
 }
@@ -247,7 +264,9 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
                                uint64_t seed, int32_t n_steps, void* stream) {
     KPD_REQUIRE(s && x_kp && h_kp && init_lig_pos && x_lig && h_lig, "kpd_sampler_run: null argument");
     KPD_REQUIRE(s->cfg.arch == 0 || v_kp, "kpd_sampler_run: the GVP denoiser needs keypoint vectors v_kp");
-    KPD_REQUIRE(n_steps >= 0 && n_steps <= s->cfg.T, "kpd_sampler_run: n_steps out of range");
+    // the first executed reverse step is t0 - 1: t0 = T from pure noise, the start step from a start ligand
+    const int t0 = s->x_start ? s->start_step : s->cfg.T;
+    KPD_REQUIRE(n_steps >= 0 && n_steps <= t0, "kpd_sampler_run: n_steps out of range");
     const kpd_batch& b = s->batch;
     const int F = s->cfg.atom_nf;
     cudaStream_t user = static_cast<cudaStream_t>(stream), st = s->stream;
@@ -260,8 +279,8 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     if (s->v_width) CU(cudaMemcpyAsync(s->v_kp, v_kp, sizeof(float) * (size_t)s->v_width * b.n_kp, cudaMemcpyDeviceToDevice, st));
     CU(cudaMemcpyAsync(s->init_lig_pos, init_lig_pos, sizeof(float) * 3 * b.B, cudaMemcpyDeviceToDevice, st));
     RunParams rp;
-    rp.noise = noise; rp.seed = seed; rp.T = s->cfg.T; rp.atom_offset = s->atom_offset;
-    int counter0[4] = {s->cfg.T, s->cfg.T, 0, 0};
+    rp.noise = noise; rp.seed = seed; rp.T = t0; rp.atom_offset = s->atom_offset;
+    int counter0[4] = {t0, t0, 0, 0};
     // small pageable H2D copies: staged by the runtime before the call returns
     CU(cudaMemcpyAsync(s->rp, &rp, sizeof(rp), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(s->counter, counter0, sizeof(counter0), cudaMemcpyHostToDevice, st));
@@ -270,9 +289,14 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
 
     // frame setup (ligand_diffuser.py:348-370)
     KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 1, 0, s->init_kp_com, st));                // init_kp_com (:348)
-    KPD_TRY(launch_shift(s->x_kp, b.kp_batch, b.n_kp, s->init_lig_pos, -1.0f, st));      // :363
-    KPD_TRY(launch_randn_init(s->x_lig, s->h_lig, b.n_lig, F, seed, s->rp, st));         // :366-367
-    KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 0, 1, nullptr, st));                       // :370
+    if (s->x_start) {       // start ligand noised to t0 in the frame of its own mean (partial_noise.cu)
+        KPD_TRY(launch_partial_noise(&b, s->x_start, s->h_start, s->x_lig, s->h_lig, s->x_kp, F, s->start_alpha,
+                                     s->start_sigma, s->cfg.lig_feat_norm_constant, nullptr, seed, s->rp, st));
+    } else {
+        KPD_TRY(launch_shift(s->x_kp, b.kp_batch, b.n_kp, s->init_lig_pos, -1.0f, st));  // :363
+        KPD_TRY(launch_randn_init(s->x_lig, s->h_lig, b.n_lig, F, seed, s->rp, st));     // :366-367
+        KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 0, 1, nullptr, st));                   // :370
+    }
     if (s->cfg.arch == 0)   // the EGNN keypoint encoder does not depend on t: hoisted out of the loop
         KPD_TRY(kpd_egnn_encode_kp(static_cast<const kpd_egnn_model*>(s->model), s->h_kp, b.n_kp, s->kp_enc, s->model_ws, st));
 

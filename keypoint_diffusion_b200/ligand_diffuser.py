@@ -18,7 +18,7 @@ from .dynamics import LigRecDynamics, LigRecDynamicsGVP
 from .n_nodes_dist import LigandSizeDistribution
 from .receptor_encoder import ReceptorEncoder, ReceptorEncoderGVP
 from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_table, inpaint_table, sigma,
-                       sigma_and_alpha_t_given_s)
+                       sigma_and_alpha_t_given_s, start_coefficients)
 from .utils import get_batch_idxs, split_bounds
 
 DEFAULT_SUB_BATCHES = {"gvp": 4, "egnn": 2}      # measured on B200: profiles/r01_sweep_sub_batches_*.txt
@@ -261,7 +261,8 @@ class KeypointDiffusion(nn.Module):
                                       return_device_tensors: bool = False, sub_batches: Optional[int] = None,
                                       decode: bool = False, capacity: bool = True, fixed_mask: torch.Tensor = None,
                                       fixed_pos: torch.Tensor = None, fixed_feat: torch.Tensor = None,
-                                      resamplings: int = 1):
+                                      resamplings: int = 1, start_pos: torch.Tensor = None,
+                                      start_feat: torch.Tensor = None, start_step: Optional[int] = None):
         """Returns (lig_pos, lig_feat): one CPU tensor per complex, as the reference does (:342-469).  ``g`` may live
         on the CPU (pinned or not): its keypoint tensors are uploaded here, straight into the sampler's buffers -- the
         host->device boundary of the path (reference test.py:152-161).
@@ -277,17 +278,33 @@ class KeypointDiffusion(nn.Module):
         frame the ligands are returned in) and ``fixed_feat`` ([n_lig,F], returned feature space); rows of unmarked atoms
         are ignored.  Every reverse step runs ``resamplings`` denoiser passes (RePaint resampling, jump length 1), so a
         call costs about ``resamplings`` plain calls.  Complexes without a marked atom are sampled exactly as without
-        a mask at resamplings=1.  Only the capacity path supports it: ``capacity=False`` raises ValueError."""
+        a mask at resamplings=1.  Only the capacity path supports it: ``capacity=False`` raises ValueError.
+
+        Ligand optimisation by partial noising (SDEdit-style; an extension beyond the reference, DESIGN.md section 6.2):
+        with ``start_pos`` ([n_lig,3], g's ligand order, in the frame the ligands are returned in), ``start_feat``
+        ([n_lig,F], returned feature space) and ``start_step`` = t0 in [0, T], every ligand starts from its start ligand
+        noised to level t0, and the loop runs the t0 reverse steps t0-1 .. 0 (about t0/T of a plain call): a small t0
+        gives close variants, a large one ligands that only loosely follow the start.  The frame is the start ligands'
+        own: ``init_lig_pos`` is not used and must not be given.  Composes with a fragment (which then stays pinned) and
+        with sub-batches; capacity path only."""
         n_lig_total = int(g.num_nodes('lig'))
         inpaint = self._check_fragment_args(n_lig_total, fixed_mask, fixed_pos, fixed_feat, resamplings)
+        start = self._check_start_args(n_lig_total, start_pos, start_feat, start_step)
         if inpaint and not capacity:
             raise ValueError("fragment-conditioned sampling runs on the capacity path only (capacity=True)")
+        if start and not capacity:
+            raise ValueError("sampling from a start ligand runs on the capacity path only (capacity=True)")
+        if start and init_lig_pos is not None:
+            raise ValueError("init_lig_pos is not used with a start ligand (the start ligands' means set the frame)")
         if visualize:
             raise NotImplementedError("visualize=True (a per-step CPU copy of the whole graph) is a debug feature "
                                       "outside the throughput path")
         dev = torch.device("cuda", torch.cuda.current_device()) if g.device.type != "cuda" else g.device
         batch_size = g.batch_size
-        if init_lig_pos is not None:
+        if start:
+            init_pos = torch.zeros(batch_size, 3)                   # not read by a run from a start ligand
+            a_t0, s_t0 = start_coefficients(self.gamma.gamma, int(start_step))
+        elif init_lig_pos is not None:
             assert init_lig_pos.shape == (batch_size, 3)
             init_pos = init_lig_pos
         else:
@@ -337,6 +354,10 @@ class KeypointDiffusion(nn.Module):
             if inpaint:
                 l1 = lig_ptr[b]
                 frag = (fixed_mask[l0:l1], fixed_pos[l0:l1], fixed_feat[l0:l1])
+            st_rows = None
+            if start:
+                l1 = lig_ptr[b]
+                st_rows = (start_pos[l0:l1], start_feat[l0:l1], int(start_step), a_t0, s_t0)
             if n_sub > 1 and (slot, str(dev)) not in self._streams:
                 self._streams[(slot, str(dev))] = torch.cuda.Stream(device=dev)
             st = self._streams[(slot, str(dev))] if n_sub > 1 else cur
@@ -344,7 +365,8 @@ class KeypointDiffusion(nn.Module):
                 st.wait_event(ready)
             with torch.cuda.stream(st):
                 out = smp.run(plan, kp['x_0'][k0:k1], kp['h_0'][k0:k1], kv[k0:k1] if kv is not None else None, gs, gd,
-                              init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag)
+                              init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag,
+                              start=st_rows)
             if n_sub > 1:
                 for t in out:
                     t.record_stream(cur)
@@ -387,6 +409,65 @@ class KeypointDiffusion(nn.Module):
             raise ValueError(f"fixed_feat must have shape [{n_lig}, {F}], got {tuple(fixed_feat.shape)}")
         if int(resamplings) > 1 and not bool(fixed_mask.any()):
             raise ValueError("resamplings > 1 needs at least one fixed atom")
+        return True
+
+    def _check_start_step(self, start_step):
+        if start_step is None:
+            return
+        if isinstance(start_step, bool) or int(start_step) != start_step or not 0 <= int(start_step) <= self.n_timesteps:
+            raise ValueError(f"start_step must be an integer in [0, {self.n_timesteps}], got {start_step}")
+
+    def _check_start_args(self, n_lig: int, start_pos, start_feat, start_step) -> bool:
+        """ValueError for an inconsistent start-ligand request (host-side checks, before any device work); True when the
+        call runs from a start ligand."""
+        self._check_start_step(start_step)
+        given = start_pos is not None or start_feat is not None
+        if not given:
+            if start_step is not None:
+                raise ValueError("start_step needs a start ligand (start_pos and start_feat)")
+            return False
+        if start_pos is None or start_feat is None:
+            raise ValueError("a start ligand needs both start_pos and start_feat")
+        if start_step is None:
+            raise ValueError("a start ligand needs start_step")
+        F = self.n_lig_features
+        if start_pos.dim() != 2 or tuple(start_pos.shape) != (n_lig, 3):
+            raise ValueError(f"start_pos must have shape [{n_lig}, 3], got {tuple(start_pos.shape)}")
+        if start_feat.dim() != 2 or tuple(start_feat.shape) != (n_lig, F):
+            raise ValueError(f"start_feat must have shape [{n_lig}, {F}], got {tuple(start_feat.shape)}")
+        return True
+
+    def _check_start_ligands(self, start_ligands, start_step, n_lig_atoms, init_lig_pos, use_ref_lig_com,
+                             sampler_kw) -> bool:
+        """Host-side validation of _sample's per-receptor start ligands; True when the call runs from them."""
+        self._check_start_step(start_step)
+        if start_ligands is None:
+            if start_step is not None:
+                raise ValueError("start_step needs start ligands")
+            return False
+        if start_step is None:
+            raise ValueError("start ligands need start_step")
+        if init_lig_pos is not None or use_ref_lig_com:
+            raise ValueError("init_lig_pos / use_ref_lig_com are not used with start ligands (their means set the frame)")
+        if not sampler_kw.get("capacity", True):
+            raise ValueError("sampling from a start ligand runs on the capacity path only (capacity=True)")
+        if len(start_ligands) != len(n_lig_atoms):
+            raise ValueError(f"start_ligands: one entry per receptor, got {len(start_ligands)} for "
+                             f"{len(n_lig_atoms)} receptors")
+        F = self.n_lig_features
+        for r, lig in enumerate(start_ligands):
+            if lig is None:
+                raise ValueError(f"receptor {r} has no start ligand")
+            pos, feat = lig
+            if pos.dim() != 2 or pos.shape[1] != 3:
+                raise ValueError(f"start ligand of receptor {r}: positions must be [m, 3], got {tuple(pos.shape)}")
+            if feat.dim() != 2 or feat.shape[1] != F or feat.shape[0] != pos.shape[0]:
+                raise ValueError(f"start ligand of receptor {r}: features must be [{pos.shape[0]}, {F}], got "
+                                 f"{tuple(feat.shape)}")
+            m = int(pos.shape[0])
+            other = [int(n) for n in n_lig_atoms[r] if int(n) != m]
+            if other:
+                raise ValueError(f"receptor {r}: requested ligand size {other[0]} differs from its {m}-atom start ligand")
         return True
 
     def _check_fragments(self, fragments, n_lig_atoms, resamplings) -> bool:
@@ -481,7 +562,7 @@ class KeypointDiffusion(nn.Module):
                 diff_batch_size: int = 32, visualize=False, use_ref_lig_com: bool = False, encoded: bool = False,
                 init_lig_pos: Optional[List[torch.Tensor]] = None, noise: Optional[List[torch.Tensor]] = None,
                 complexes: Optional[List[int]] = None, fragments: Optional[List] = None, resamplings: int = 1,
-                **sampler_kw):
+                start_ligands: Optional[List] = None, start_step: Optional[int] = None, **sampler_kw):
         """ref_graphs: one single-complex graph per receptor (reference :270-340).  ``encoded=True`` skips the receptor
         encoder (graphs already hold kp nodes + kk edges).  init_lig_pos: optional [3] tensor per receptor.
         noise: optional injected Gaussian draws, one [T+1, n_lig*(3+F)] tensor per diffusion batch (parity runs).
@@ -491,9 +572,15 @@ class KeypointDiffusion(nn.Module):
         receptor starts with those m atoms, pinned (fragment growing; positions in the receptor's frame, features in the
         returned feature space), with ``resamplings`` denoiser passes per reverse step (see
         sample_from_encoded_receptors).  A diffusion batch without any fragment atom is sampled by the plain loop.
+        start_ligands / start_step: optional, one ``(pos [m,3], feat [m,F])`` per receptor and t0 in [0, T]: every
+        ligand requested for that receptor (each of size m) is a variant of its start ligand, noised to level t0 and
+        denoised from there (ligand optimisation, see sample_from_encoded_receptors); with fragments too, the fragment
+        is the start ligand's first atoms and stays pinned.
 
         The diffusion batches are assembled on the device (hetero.expand_complexes): no per-complex graph copies."""
         has_fragment = self._check_fragments(fragments, n_lig_atoms, resamplings)
+        has_start = self._check_start_ligands(start_ligands, start_step, n_lig_atoms, init_lig_pos, use_ref_lig_com,
+                                              sampler_kw)
         n_receptors = len(ref_graphs)
         enc, rec_mean = self._encode_all(ref_graphs, rec_enc_batch_size, encoded)
         dev = enc.device
@@ -514,11 +601,18 @@ class KeypointDiffusion(nn.Module):
             chunk = todo[b * diff_batch_size:(b + 1) * diff_batch_size]
             idx = torch.tensor(chunk, dtype=torch.long, device=dev)
             bg = hetero.expand_complexes(enc, pocket_t[idx], size_t[idx], self.n_lig_features)
-            if centers is None:
+            if centers is None and not has_start:
                 raise ValueError("init_lig_pos is required when the graphs have no 'rec' nodes (SURVEY N7)")
             frag_kw = (self._fragment_rows(fragments, [pocket_of[i] for i in chunk], [sizes[i] for i in chunk], resamplings)
                        if has_fragment else {})
-            p, f = self.sample_from_encoded_receptors(bg, visualize=visualize, init_lig_pos=centers[pocket_t[idx]],
+            if has_start:
+                owners = [pocket_of[i] for i in chunk]
+                frag_kw.update(init_lig_pos=None, start_step=int(start_step),
+                               start_pos=torch.cat([start_ligands[r][0].detach().float().cpu() for r in owners]),
+                               start_feat=torch.cat([start_ligands[r][1].detach().float().cpu() for r in owners]))
+            else:
+                frag_kw.update(init_lig_pos=centers[pocket_t[idx]])
+            p, f = self.sample_from_encoded_receptors(bg, visualize=visualize,
                                                       noise=None if noise is None else noise[b], **frag_kw, **sampler_kw)
             lig_pos.extend(p)
             lig_feat.extend(f)
@@ -589,11 +683,16 @@ class KeypointDiffusion(nn.Module):
 
     @torch.no_grad()
     def sample_given_pocket(self, rec_graph, n_lig_atoms: torch.Tensor, rec_enc_batch_size: int = 32,
-                            diff_batch_size: int = 32, visualize=False, fragment=None, **kw):
-        """fragment: optional ``(pos [m,3], feat [m,F])``: every ligand starts with these m atoms (see _sample)."""
+                            diff_batch_size: int = 32, visualize=False, fragment=None, start_ligand=None,
+                            start_step: Optional[int] = None, **kw):
+        """fragment: optional ``(pos [m,3], feat [m,F])``: every ligand starts with these m atoms (see _sample).
+        start_ligand / start_step: optional ``(pos [m,3], feat [m,F])`` and t0: every ligand (each of size m) is a
+        variant of that ligand, noised to level t0 and denoised from there (see _sample)."""
         samples = self._sample([rec_graph], n_lig_atoms=[n_lig_atoms.tolist()], rec_enc_batch_size=rec_enc_batch_size,
                                diff_batch_size=diff_batch_size, visualize=visualize,
-                               fragments=None if fragment is None else [fragment], **kw)
+                               fragments=None if fragment is None else [fragment],
+                               start_ligands=None if start_ligand is None else [start_ligand], start_step=start_step,
+                               **kw)
         return samples[0]['positions'], samples[0]['features']
 
     @torch.no_grad()

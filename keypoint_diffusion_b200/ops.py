@@ -412,6 +412,20 @@ def renoise(batch: DeviceBatch, x_lig, h_lig, x_kp, coef2, step: torch.Tensor, u
                           int(u), ptr(noise), int(seed), _stream()), "kpd_renoise")
 
 
+def partial_noise(batch: DeviceBatch, x_start, h_start, x_kp, alpha: float, sigma: float, lig_feat_norm_constant=1.0,
+                  noise=None, seed=0):
+    """The start of a run from a given ligand (kpd_partial_noise): x_start [n_lig,3] / h_start [n_lig,F] noised to the
+    level (alpha, sigma) in the frame of each complex's start-ligand mean, then the ligand COM removed; x_kp is moved
+    with the ligand, in place.  noise: None (Philox, the plain loop's initial draw) or [n_lig*(3+F)] (x first).
+    -> (x_lig, h_lig)."""
+    _require_cuda(x_start, h_start, x_kp, noise)
+    x_lig, h_lig = torch.empty_like(x_start), torch.empty_like(h_start)
+    check(lib.kpd_partial_noise(C.byref(batch.c), ptr(x_start), ptr(h_start), ptr(x_lig), ptr(h_lig), ptr(x_kp),
+                                h_start.shape[1], float(alpha), float(sigma), float(lig_feat_norm_constant), ptr(noise),
+                                int(seed), _stream()), "kpd_partial_noise")
+    return x_lig, h_lig
+
+
 def decode_atom_types(h_lig: torch.Tensor) -> torch.Tensor:
     """int32 [n] = argmax over the feature channels of every atom (lowest index wins ties, like torch.argmax on the
     CPU), on the device through kpd_decode_atom_types -- what the reference computes on the host right after sampling
@@ -438,7 +452,8 @@ class Sampler:
 
     resamplings >= 1 with inpaint_coef (schedule.inpaint_table on the device) makes it a fragment-conditioned
     (inpainting) sampler: every reverse step runs `resamplings` denoiser passes with the atoms given to set_fragment
-    pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop."""
+    pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop.
+    Either kind runs from a given ligand after set_start (ligand optimisation by partial noising)."""
 
     def __init__(self, model: _Model, batch: DeviceBatch, gp: GraphParams, kk: Optional[Csr], coef: torch.Tensor,
                  T: int, atom_nf: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
@@ -471,6 +486,7 @@ class Sampler:
             check(lib.kpd_sampler_set_atom_offset(self.handle, int(atom_offset)), "kpd_sampler_set_atom_offset")
         self.inpaint_coef = inpaint_coef
         self._fragment = None
+        self._start = None
         if self.resamplings:
             _require_cuda(inpaint_coef)
             check(lib.kpd_sampler_enable_inpainting(self.handle, self.resamplings, ptr(inpaint_coef)),
@@ -491,10 +507,36 @@ class Sampler:
               "kpd_sampler_set_fragment")
         self._fragment = (fixed_mask, x_fix, h_fix)
 
+    def set_start(self, start_step: Optional[int], x_start: Optional[torch.Tensor] = None,
+                  h_start: Optional[torch.Tensor] = None, alpha: float = 0.0, sigma: float = 0.0):
+        """The ligand the next runs start from (kpd_sampler_set_start): x_start [n_lig,3] in the frame of the keypoints
+        passed to run(), h_start [n_lig,F] in the returned feature space, noised to step start_step in [0, T] with
+        (alpha, sigma) = schedule.start_coefficients(gamma, start_step); the runs then take start_step reverse steps.
+        start_step=None restores the plain start from pure noise.  The tensors must stay alive and in place while runs
+        use them (only their addresses are kept)."""
+        if start_step is None:
+            check(lib.kpd_sampler_set_start(self.handle, 0, None, None, 0.0, 0.0), "kpd_sampler_set_start")
+            self._start = None
+            return
+        _require_cuda(x_start, h_start)
+        assert x_start.dtype == torch.float32 and h_start.dtype == torch.float32
+        assert x_start.shape == (self.batch.n_lig, 3) and h_start.shape == (self.batch.n_lig, self.atom_nf)
+        assert x_start.is_contiguous() and h_start.is_contiguous()
+        check(lib.kpd_sampler_set_start(self.handle, int(start_step), ptr(x_start), ptr(h_start), float(alpha),
+                                        float(sigma)), "kpd_sampler_set_start")
+        self._start = (int(start_step), x_start, h_start)
+
+    @property
+    def start_step(self) -> int:
+        """The step runs start from: T, or the start step of set_start."""
+        return self.T if self._start is None else self._start[0]
+
     @property
     def noise_slots(self) -> int:
-        """Slots of injected noise run() takes: T+1 (plain) or 1 + T*(3r-1) (inpainting with r resamplings)."""
-        return self.T + 1 if not self.resamplings else 1 + self.T * (3 * self.resamplings - 1)
+        """Slots of injected noise run() takes, with t0 = start_step: t0+1 (plain) or 1 + t0*(3r-1) (inpainting with r
+        resamplings)."""
+        t0 = self.start_step
+        return t0 + 1 if not self.resamplings else 1 + t0 * (3 * self.resamplings - 1)
 
     def __del__(self):
         if getattr(self, "handle", None) and self.handle.value and lib is not None:
@@ -510,7 +552,7 @@ class Sampler:
         x_kp = _f32(x_kp).clone()
         x_lig = torch.empty(b.n_lig, 3, dtype=torch.float32, device=b.device)
         h_lig = torch.empty(b.n_lig, self.atom_nf, dtype=torch.float32, device=b.device)
-        n_steps = self.T if n_steps is None else int(n_steps)
+        n_steps = self.start_step if n_steps is None else int(n_steps)
         if noise is not None:
             _require_cuda(noise)
             assert noise.shape == (self.noise_slots, b.n_lig * (3 + self.atom_nf)) and noise.dtype == torch.float32
@@ -622,7 +664,8 @@ class CapacitySampler:
     """A captured reverse-diffusion loop for one capacity bucket (see plan_capacity): owns its layout arrays, kk CSR and
     input buffers; run() rewrites their CONTENTS for the batch at hand and replays the same CUDA graphs.  With
     resamplings >= 1 (and inpaint_coef) it is an inpainting sampler that also owns zero-filled fragment buffers sized at
-    capacity: run(fragment=...) fills the rows of the real atoms; filler complexes and atoms are never fixed."""
+    capacity: run(fragment=...) fills the rows of the real atoms; filler complexes and atoms are never fixed.  Likewise
+    it owns start-ligand buffers at capacity for run(start=...); filler rows stay zero and filler outputs are dropped."""
 
     def __init__(self, model: _Model, plan: CapacityPlan, gp: GraphParams, coef: torch.Tensor, T: int, atom_nf: int,
                  kp_width: int, v_width: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
@@ -645,13 +688,18 @@ class CapacitySampler:
             self.x_fix = torch.zeros(N, 3, dtype=torch.float32, device=dev)
             self.h_fix = torch.zeros(N, self.atom_nf, dtype=torch.float32, device=dev)
             self.sampler.set_fragment(self.fixed_mask, self.x_fix, self.h_fix)
+        self.x_start = torch.zeros(N, 3, dtype=torch.float32, device=dev)
+        self.h_start = torch.zeros(N, self.atom_nf, dtype=torch.float32, device=dev)
         self.runs = 0
 
     def run(self, plan: CapacityPlan, x_kp, h_kp, v_kp, kk_src, kk_dst, init_pos, seed: int, atom_offset: int = 0,
-            noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None):
+            noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None,
+            start: Optional[Tuple] = None):
         """x_kp/h_kp/v_kp: the REAL keypoint rows (host or device tensors; pinned host tensors are uploaded straight
         into the capacity buffers); kk_src/kk_dst: kk edges in this batch's own keypoint numbering; init_pos [B_real,3].
         fragment (inpainting samplers): (fixed_mask [N_real] bool, x_fix [N_real,3], h_fix [N_real,F]) or None.
+        start: (x [N_real,3], h [N_real,F], t0, alpha_t0, sigma_t0) -- run t0 reverse steps from that ligand (see
+        Sampler.set_start) -- or None for the plain start; injected noise then has the slots of a t0-step run.
         -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]]) on the device."""
         if plan.key != self.key:
             raise ValueError("CapacitySampler.run: the plan belongs to another capacity bucket")
@@ -665,6 +713,14 @@ class CapacitySampler:
                 self.fixed_mask[:N_r].copy_(fragment[0], non_blocking=True)
                 self.x_fix[:N_r].copy_(fragment[1], non_blocking=True)
                 self.h_fix[:N_r].copy_(fragment[2], non_blocking=True)
+        if start is not None:            # rows past the real atoms stay zero: filler complexes start from the origin
+            self.x_start.zero_()
+            self.h_start.zero_()
+            self.x_start[:N_r].copy_(start[0], non_blocking=True)
+            self.h_start[:N_r].copy_(start[1], non_blocking=True)
+            self.sampler.set_start(int(start[2]), self.x_start, self.h_start, float(start[3]), float(start[4]))
+        else:
+            self.sampler.set_start(None)
         self.x_kp[:K_r].copy_(x_kp, non_blocking=True)
         self.h_kp[:K_r].copy_(h_kp, non_blocking=True)
         if self.v_kp is not None:

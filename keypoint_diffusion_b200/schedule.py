@@ -6,7 +6,8 @@ round-trips through the checkpoint (SURVEY N9).  The table [T,4] = (alpha_t|s, v
 sigma, t) is what the CUDA step kernel reads; it restates models/ligand_diffuser.py:232-252 and
 :505-527 on the host, once per model (the values are identical for every complex of a batch).
 inpaint_table [T,4] = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) is the second table that
-fragment-conditioned sampling reads (DESIGN.md section 6.1).
+fragment-conditioned sampling reads (DESIGN.md section 6.1); start_coefficients gives (alpha_t0, sigma_t0), the
+forward noising of a start ligand in ligand optimisation (section 6.2).
 """
 import numpy as np
 import torch
@@ -106,3 +107,12 @@ def inpaint_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
         _, s1, a = sigma_and_alpha_t_given_s(gt, gs)
         rows.append(torch.stack([alpha(gs)[0], sigma(gs)[0], a[0], s1[0]]))
     return torch.stack(rows).contiguous()
+
+
+def start_coefficients(gamma: torch.Tensor, t0: int):
+    """(alpha_t0, sigma_t0) as Python floats holding fp32 values: the level a start ligand is noised to before the
+    reverse loop runs from step t0 (ligand optimisation by partial noising).  Evaluated like coefficient_table, with the
+    scalar fp32 ops on a 1-element tensor gamma[t0]."""
+    g = gamma.detach().float().cpu()
+    g0 = g[torch.full((1,), int(t0), dtype=torch.long)]
+    return float(alpha(g0)[0]), float(sigma(g0)[0])
