@@ -228,13 +228,54 @@ int launch_sub(const float* a, const float* b, float* out, int n, cudaStream_t s
 
 // ------------------------------------------------------------------ step ops (ddpm_step.cu)
 struct RunParams {        // lives in device memory so that a captured graph can be re-pointed
-    const float* noise;   // NULL or [(T+1)][n_lig][3+F], slot 0 = initial draw
+    const float* noise;   // NULL or slots of [n_lig][3+F] (x first), numbered by noise_slot()
     uint64_t seed;
     int T;                // the step the run starts from (the sampler's T, or t0 of a run from a start ligand): the
                           // injected-noise slots of executed steps are counted from it
     int atom_offset;     // added to the atom index of the Philox counter: a batch sampled as several sub-batches draws
                           // the same noise as when it is sampled whole (kpd_sampler_set_atom_offset)
 };
+
+// injected-noise slot of draw k of step s in a run from step T: slot 0 is the initial draw (s = -1), then every executed
+// step holds per_step draws (1 in the plain loop; 3r-1 with inpainting: posterior, known part, re-noise but after the last pass)
+__device__ __forceinline__ int noise_slot(int T, int s, int per_step, int k) {
+    return s < 0 ? 0 : 1 + (T - 1 - s) * per_step + k;
+}
+
+// where a step kernel's draws come from: in a sampler run (rp) the run's seed, atom offset and injected slot
+// noise_slot(T, s, per_step, k); in a stand-alone call the caller's noise and seed.  noise == NULL: Philox.
+struct StepDraws {
+    const float* noise;
+    uint64_t seed;
+    int atom_offset;
+};
+__device__ __forceinline__ StepDraws step_draws(const RunParams* rp, const float* noise, uint64_t seed, int s,
+                                                int per_step, int k, size_t slot_len) {
+    if (!rp) return {noise, seed, 0};
+    return {rp->noise ? rp->noise + (size_t)noise_slot(rp->T, s, per_step, k) * slot_len : nullptr, rp->seed,
+            rp->atom_offset};
+}
+
+// One CTA per complex.  mean3: out = the mean of rows [r0, r0+n) of x[][3], threads 0..2 summing in row order
+// (bit-identical to the oracle's sequential mean); the caller syncs before reading out.  sub3: those rows -= v.
+__device__ __forceinline__ void mean3(const float* x, int r0, int n, float* out) {
+    if (threadIdx.x < 3) {
+        float acc = 0.0f;
+        for (int j = 0; j < n; ++j) acc = __fadd_rn(acc, x[3 * (r0 + j) + threadIdx.x]);
+        out[threadIdx.x] = __fdiv_rn(acc, (float)n);
+    }
+}
+__device__ __forceinline__ void sub3(float* x, int r0, int n, const float* v) {
+    for (int i = threadIdx.x; i < n * 3; i += blockDim.x) x[3 * r0 + i] = __fsub_rn(x[3 * r0 + i], v[i % 3]);
+}
+// the ligand COM (into com[3], shared) removed from the complex's ligand and keypoint rows
+__device__ __forceinline__ void remove_ligand_com(float* x_lig, float* x_kp, int l0, int nl, int k0, int nk, float* com) {
+    mean3(x_lig, l0, nl, com);
+    __syncthreads();
+    sub3(x_lig, l0, nl, com);
+    sub3(x_kp, k0, nk, com);
+}
+
 int launch_ddpm_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
                      const float* eps_h, int F, const float* coef, const int* step_ptr, const float* noise_x,
                      const float* noise_h, uint64_t seed, const RunParams* rp, cudaStream_t st);

@@ -13,22 +13,6 @@
 
 namespace kpd {
 
-// ---- Philox4x32-10 (philox.cuh), counter = (atom, step+1, group, 0), key = seed
-// standard normal for (seed, step, atom, channel); channels are drawn 4 at a time
-__device__ float philox_normal(uint64_t seed, int step, int atom, int ch) {
-    const uint4 r = philox4x32_10(make_uint4((uint32_t)atom, (uint32_t)(step + 1), (uint32_t)(ch >> 2), 0u),
-                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-    const int q = ch & 3;
-    const uint32_t ua = q < 2 ? r.x : r.z, ub = q < 2 ? r.y : r.w;
-    // Box-Muller on (0,1] x [0,1)
-    const float u1 = ((float)ua + 1.0f) * 2.3283064365386963e-10f;
-    const float u2 = (float)ub * 2.3283064365386963e-10f;
-    const float rad = sqrtf(-2.0f * logf(u1));
-    float sn, cs;
-    sincosf(6.283185307179586f * u2, &sn, &cs);
-    return (q & 1) ? rad * sn : rad * cs;
-}
-
 __global__ void __launch_bounds__(128)
 ddpm_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_lig, float* __restrict__ x_kp,
                  const float* __restrict__ eps_x, const float* __restrict__ eps_h, int F,
@@ -39,42 +23,24 @@ ddpm_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_l
     const int k0 = b.kp_ptr[c], nk = b.kp_ptr[c + 1] - k0;
     const int s = *step_ptr;
     const float a = coef[4 * s], vt = coef[4 * s + 1], sg = coef[4 * s + 2];
-    int aoff = 0;
-    if (rp) {
-        seed = rp->seed;
-        aoff = rp->atom_offset;
-        if (rp->noise) {
-            const float* slot = rp->noise + (size_t)(1 + (rp->T - 1 - s)) * b.n_lig * (3 + F);
-            noise_x = slot;
-            noise_h = slot + (size_t)b.n_lig * 3;
-        } else {
-            noise_x = noise_h = nullptr;
-        }
-    }
+    const StepDraws d = step_draws(rp, noise_x, seed, s, 1, 0, (size_t)b.n_lig * (3 + F));
+    if (rp) noise_h = d.noise ? d.noise + (size_t)b.n_lig * 3 : nullptr;   // a run's slot holds x, then h
     __shared__ float com[3];
     // mu = z/alpha_t|s - var_terms*eps ; z_s = mu + sigma*noise   (ligand_diffuser.py:522-533)
     for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) {
         const int idx = 3 * l0 + i;
-        const float nz = noise_x ? noise_x[idx] : philox_normal(seed, s, aoff + l0 + i / 3, i % 3);
+        const float nz = d.noise ? d.noise[idx] : philox_normal(d.seed, s, d.atom_offset + l0 + i / 3, i % 3);
         const float mu = __fsub_rn(__fdiv_rn(x_lig[idx], a), __fmul_rn(vt, eps_x[idx]));
         x_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
     }
     for (int i = threadIdx.x; i < nl * F; i += blockDim.x) {
         const int idx = F * l0 + i;
-        const float nz = noise_h ? noise_h[idx] : philox_normal(seed, s, aoff + l0 + i / F, 3 + i % F);
+        const float nz = noise_h ? noise_h[idx] : philox_normal(d.seed, s, d.atom_offset + l0 + i / F, 3 + i % F);
         const float mu = __fsub_rn(__fdiv_rn(h_lig[idx], a), __fmul_rn(vt, eps_h[idx]));
         h_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
     }
     __syncthreads();
-    // remove ligand COM from ligand and keypoints (:536 -> :185-203)
-    if (threadIdx.x < 3) {
-        float acc = 0.0f;
-        for (int j = 0; j < nl; ++j) acc = __fadd_rn(acc, x_lig[3 * (l0 + j) + threadIdx.x]);
-        com[threadIdx.x] = __fdiv_rn(acc, (float)nl);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) x_lig[3 * l0 + i] = __fsub_rn(x_lig[3 * l0 + i], com[i % 3]);
-    for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fsub_rn(x_kp[3 * k0 + i], com[i % 3]);
+    remove_ligand_com(x_lig, x_kp, l0, nl, k0, nk, com);   // :536 -> :185-203
 }
 
 int launch_ddpm_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
@@ -95,18 +61,12 @@ com_kernel(kpd_batch b, float* x_lig, float* x_kp, int which, int shift, float* 
     const int l0 = b.lig_ptr[c], nl = b.lig_ptr[c + 1] - l0;
     const int k0 = b.kp_ptr[c], nk = b.kp_ptr[c + 1] - k0;
     __shared__ float com[3];
-    if (threadIdx.x < 3) {
-        const float* x = which == 0 ? x_lig + 3 * l0 : x_kp + 3 * k0;
-        const int n = which == 0 ? nl : nk;
-        float acc = 0.0f;
-        for (int j = 0; j < n; ++j) acc = __fadd_rn(acc, x[3 * j + threadIdx.x]);
-        com[threadIdx.x] = __fdiv_rn(acc, (float)n);
-        if (com_out) com_out[3 * c + threadIdx.x] = com[threadIdx.x];
-    }
+    mean3(which == 0 ? x_lig : x_kp, which == 0 ? l0 : k0, which == 0 ? nl : nk, com);
+    if (com_out && threadIdx.x < 3) com_out[3 * c + threadIdx.x] = com[threadIdx.x];
     __syncthreads();
     if (!shift) return;
-    for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) x_lig[3 * l0 + i] = __fsub_rn(x_lig[3 * l0 + i], com[i % 3]);
-    for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fsub_rn(x_kp[3 * k0 + i], com[i % 3]);
+    sub3(x_lig, l0, nl, com);
+    sub3(x_kp, k0, nk, com);
 }
 
 int launch_com(const kpd_batch* b, float* x_lig, float* x_kp, int which, int shift, float* com_out, cudaStream_t st) {
@@ -132,13 +92,11 @@ __global__ void randn_init_kernel(float* x_lig, float* h_lig, int n_lig, int F, 
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const int W = 3 + F;
     if (i >= n_lig * W) return;
-    const float* noise = nullptr;
-    int aoff = 0;
-    if (rp) { seed = rp->seed; noise = rp->noise; aoff = rp->atom_offset; }
+    const StepDraws d = step_draws(rp, nullptr, seed, -1, 1, 0, (size_t)n_lig * W);
     const int atom = i / W, ch = i % W;
     float v;
-    if (noise) v = ch < 3 ? noise[3 * atom + ch] : noise[(size_t)3 * n_lig + (size_t)F * atom + (ch - 3)];
-    else v = philox_normal(seed, -1, aoff + atom, ch);
+    if (d.noise) v = ch < 3 ? d.noise[3 * atom + ch] : d.noise[(size_t)3 * n_lig + (size_t)F * atom + (ch - 3)];
+    else v = philox_normal(d.seed, -1, d.atom_offset + atom, ch);
     if (ch < 3) x_lig[3 * atom + ch] = v;
     else h_lig[F * atom + (ch - 3)] = v;
 }

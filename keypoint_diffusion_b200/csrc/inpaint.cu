@@ -17,40 +17,6 @@
 
 namespace kpd {
 
-// standard normal for (seed, step, atom, channel, word): the word is the counter's fourth element.  With word 0 this is
-// ddpm_step.cu's philox_normal, draw for draw; that one stays a separate function so that the plain step's code is not
-// touched by this path.
-__device__ float philox_normal_w(uint64_t seed, int step, int atom, int ch, uint32_t word) {
-    const uint4 r = philox4x32_10(make_uint4((uint32_t)atom, (uint32_t)(step + 1), (uint32_t)(ch >> 2), word),
-                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-    const int q = ch & 3;
-    const uint32_t ua = q < 2 ? r.x : r.z, ub = q < 2 ? r.y : r.w;
-    const float u1 = ((float)ua + 1.0f) * 2.3283064365386963e-10f;
-    const float u2 = (float)ub * 2.3283064365386963e-10f;
-    const float rad = sqrtf(-2.0f * logf(u1));
-    float sn, cs;
-    sincosf(6.283185307179586f * u2, &sn, &cs);
-    return (q & 1) ? rad * sn : rad * cs;
-}
-
-// injected-noise slot of (step s, pass u, kind) in a sampler run: slot 0 is the initial draw, then per executed step
-// the posterior / known / re-noise draws of every pass (no re-noise after the last one): 3r - 1 slots per step
-__device__ __forceinline__ const float* inpaint_slot(const RunParams* rp, int s, int u, int r, int kind, size_t slot_len) {
-    return rp->noise + (size_t)(1 + (rp->T - 1 - s) * (3 * r - 1) + 3 * u + kind) * slot_len;
-}
-
-__device__ __forceinline__ void remove_ligand_com(const kpd_batch& b, float* x_lig, float* x_kp, int l0, int nl, int k0,
-                                                  int nk, float* com) {
-    if (threadIdx.x < 3) {
-        float acc = 0.0f;
-        for (int j = 0; j < nl; ++j) acc = __fadd_rn(acc, x_lig[3 * (l0 + j) + threadIdx.x]);
-        com[threadIdx.x] = __fdiv_rn(acc, (float)nl);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) x_lig[3 * l0 + i] = __fsub_rn(x_lig[3 * l0 + i], com[i % 3]);
-    for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fsub_rn(x_kp[3 * k0 + i], com[i % 3]);
-}
-
 __global__ void __launch_bounds__(128)
 ddpm_inpaint_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_lig, float* __restrict__ x_kp,
                          const float* __restrict__ eps_x, const float* __restrict__ eps_h, int F,
@@ -65,15 +31,10 @@ ddpm_inpaint_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restri
     const float a = coef[4 * s], vt = coef[4 * s + 1], sg = coef[4 * s + 2];
     const float a_s = fr.coef2[4 * s], sg_s = fr.coef2[4 * s + 1];
     const size_t slot_len = (size_t)b.n_lig * (3 + F);
-    const float* nz_post = noise;
-    const float* nz_kn = noise ? noise + slot_len : nullptr;
-    int aoff = 0;
-    if (rp) {
-        seed = rp->seed;
-        aoff = rp->atom_offset;
-        nz_post = rp->noise ? inpaint_slot(rp, s, u, r, 0, slot_len) : nullptr;
-        nz_kn = rp->noise ? inpaint_slot(rp, s, u, r, 1, slot_len) : nullptr;
-    }
+    // the known-part draws (kind 1) follow the posterior ones (kind 0), in a run's slots as in a stand-alone call's noise
+    const StepDraws d = step_draws(rp, noise, seed, s, 3 * r - 1, 3 * u, slot_len);
+    const float* nz_post = d.noise;
+    const float* nz_kn = d.noise ? d.noise + slot_len : nullptr;
     const uint32_t w = 3u * (uint32_t)u;
     const uint8_t* M = fr.mask ? fr.mask + l0 : nullptr;
     extern __shared__ float z_kn[];          // [max_lig][3]: known-part positions of this complex
@@ -84,36 +45,32 @@ ddpm_inpaint_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restri
         int m = 0;
         if (M)
             for (int j = 0; j < nl; ++j) m += M[j] != 0;
-        if (m) {
-            float acc = 0.0f;
-            for (int j = 0; j < nk; ++j) acc = __fadd_rn(acc, x_kp[3 * (k0 + j) + threadIdx.x]);
-            kp_com[threadIdx.x] = __fdiv_rn(acc, (float)nk);
-        }
+        if (m) mean3(x_kp, k0, nk, kp_com);
         if (threadIdx.x == 0) n_fix = m;
     }
     __syncthreads();
     const int m = n_fix;
     // z_unk for every position (the masked mean needs it at the fixed atoms too); z_kn for the fixed ones
     for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) {
-        const int idx = 3 * l0 + i, atom = aoff + l0 + i / 3, ch = i % 3;
-        const float nz = nz_post ? nz_post[idx] : philox_normal_w(seed, s, atom, ch, w);
+        const int idx = 3 * l0 + i, atom = d.atom_offset + l0 + i / 3, ch = i % 3;
+        const float nz = nz_post ? nz_post[idx] : philox_normal(d.seed, s, atom, ch, w);
         const float mu = __fsub_rn(__fdiv_rn(x_lig[idx], a), __fmul_rn(vt, eps_x[idx]));
         x_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
         if (m && M[i / 3]) {
             const float x0 = __fadd_rn(__fsub_rn(fr.x_fix[idx], init_kp_com[3 * c + ch]), kp_com[ch]);
-            const float e = nz_kn ? nz_kn[idx] : philox_normal_w(seed, s, atom, ch, w + 1);
+            const float e = nz_kn ? nz_kn[idx] : philox_normal(d.seed, s, atom, ch, w + 1);
             z_kn[i] = __fadd_rn(__fmul_rn(a_s, x0), __fmul_rn(sg_s, e));
         }
     }
     // features: merged at once (no alignment)
     for (int i = threadIdx.x; i < nl * F; i += blockDim.x) {
-        const int idx = F * l0 + i, atom = aoff + l0 + i / F, ch = 3 + i % F;
+        const int idx = F * l0 + i, atom = d.atom_offset + l0 + i / F, ch = 3 + i % F;
         if (m && M[i / F]) {
             const float h0 = __fdiv_rn(fr.h_fix[idx], norm_c);
-            const float e = nz_kn ? nz_kn[(size_t)b.n_lig * 3 + idx] : philox_normal_w(seed, s, atom, ch, w + 1);
+            const float e = nz_kn ? nz_kn[(size_t)b.n_lig * 3 + idx] : philox_normal(d.seed, s, atom, ch, w + 1);
             h_lig[idx] = __fadd_rn(__fmul_rn(a_s, h0), __fmul_rn(sg_s, e));
         } else {
-            const float nz = nz_post ? nz_post[(size_t)b.n_lig * 3 + idx] : philox_normal_w(seed, s, atom, ch, w);
+            const float nz = nz_post ? nz_post[(size_t)b.n_lig * 3 + idx] : philox_normal(d.seed, s, atom, ch, w);
             const float mu = __fsub_rn(__fdiv_rn(h_lig[idx], a), __fmul_rn(vt, eps_h[idx]));
             h_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
         }
@@ -136,7 +93,7 @@ ddpm_inpaint_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restri
         for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fadd_rn(x_kp[3 * k0 + i], dx[i % 3]);
         __syncthreads();
     }
-    remove_ligand_com(b, x_lig, x_kp, l0, nl, k0, nk, com);
+    remove_ligand_com(x_lig, x_kp, l0, nl, k0, nk, com);
 }
 
 int launch_ddpm_inpaint_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
@@ -164,26 +121,22 @@ renoise_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_lig
     const int s = *step_ptr;
     if (ip) coef2 = ip->coef2;
     const float a = coef2[4 * s + 2], sg = coef2[4 * s + 3];
-    int aoff = 0;
-    if (rp) {
-        seed = rp->seed;
-        aoff = rp->atom_offset;
-        noise = rp->noise ? inpaint_slot(rp, s, u, r, 2, (size_t)b.n_lig * (3 + F)) : nullptr;
-    }
+    const StepDraws d = step_draws(rp, noise, seed, s, 3 * r - 1, 3 * u + 2, (size_t)b.n_lig * (3 + F));
     const uint32_t w = 3u * (uint32_t)u + 2u;
     __shared__ float com[3];
     for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) {
         const int idx = 3 * l0 + i;
-        const float e = noise ? noise[idx] : philox_normal_w(seed, s, aoff + l0 + i / 3, i % 3, w);
+        const float e = d.noise ? d.noise[idx] : philox_normal(d.seed, s, d.atom_offset + l0 + i / 3, i % 3, w);
         x_lig[idx] = __fadd_rn(__fmul_rn(a, x_lig[idx]), __fmul_rn(sg, e));
     }
     for (int i = threadIdx.x; i < nl * F; i += blockDim.x) {
         const int idx = F * l0 + i;
-        const float e = noise ? noise[(size_t)b.n_lig * 3 + idx] : philox_normal_w(seed, s, aoff + l0 + i / F, 3 + i % F, w);
+        const float e = d.noise ? d.noise[(size_t)b.n_lig * 3 + idx]
+                                : philox_normal(d.seed, s, d.atom_offset + l0 + i / F, 3 + i % F, w);
         h_lig[idx] = __fadd_rn(__fmul_rn(a, h_lig[idx]), __fmul_rn(sg, e));
     }
     __syncthreads();
-    remove_ligand_com(b, x_lig, x_kp, l0, nl, k0, nk, com);
+    remove_ligand_com(x_lig, x_kp, l0, nl, k0, nk, com);
 }
 
 int launch_renoise(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, int F, const int* step_ptr, int u, int r,

@@ -15,21 +15,6 @@
 
 namespace kpd {
 
-// ddpm_step.cu's philox_normal, draw for draw (the same counter, key and Box-Muller arithmetic); a copy so that the
-// plain step's translation unit stays untouched
-__device__ float philox_normal_start(uint64_t seed, int step, int atom, int ch) {
-    const uint4 r = philox4x32_10(make_uint4((uint32_t)atom, (uint32_t)(step + 1), (uint32_t)(ch >> 2), 0u),
-                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-    const int q = ch & 3;
-    const uint32_t ua = q < 2 ? r.x : r.z, ub = q < 2 ? r.y : r.w;
-    const float u1 = ((float)ua + 1.0f) * 2.3283064365386963e-10f;
-    const float u2 = (float)ub * 2.3283064365386963e-10f;
-    const float rad = sqrtf(-2.0f * logf(u1));
-    float sn, cs;
-    sincosf(6.283185307179586f * u2, &sn, &cs);
-    return (q & 1) ? rad * sn : rad * cs;
-}
-
 __global__ void __launch_bounds__(128)
 partial_noise_kernel(kpd_batch b, const float* __restrict__ x_start, const float* __restrict__ h_start,
                      float* __restrict__ x_lig, float* __restrict__ h_lig, float* __restrict__ x_kp, int F, float alpha,
@@ -37,38 +22,26 @@ partial_noise_kernel(kpd_batch b, const float* __restrict__ x_start, const float
     const int c = blockIdx.x;
     const int l0 = b.lig_ptr[c], nl = b.lig_ptr[c + 1] - l0;
     const int k0 = b.kp_ptr[c], nk = b.kp_ptr[c + 1] - k0;
-    int aoff = 0;
-    if (rp) { seed = rp->seed; noise = rp->noise; aoff = rp->atom_offset; }
+    const StepDraws d = step_draws(rp, noise, seed, -1, 1, 0, (size_t)b.n_lig * (3 + F));
     __shared__ float cb[3], com[3];
-    if (threadIdx.x < 3) {
-        float acc = 0.0f;
-        for (int j = 0; j < nl; ++j) acc = __fadd_rn(acc, x_start[3 * (l0 + j) + threadIdx.x]);
-        cb[threadIdx.x] = __fdiv_rn(acc, (float)nl);
-    }
+    mean3(x_start, l0, nl, cb);
     __syncthreads();
-    for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fsub_rn(x_kp[3 * k0 + i], cb[i % 3]);
+    sub3(x_kp, k0, nk, cb);
     for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) {
         const int idx = 3 * l0 + i;
-        const float e = noise ? noise[idx] : philox_normal_start(seed, -1, aoff + l0 + i / 3, i % 3);
+        const float e = d.noise ? d.noise[idx] : philox_normal(d.seed, -1, d.atom_offset + l0 + i / 3, i % 3);
         const float x0 = __fsub_rn(x_start[idx], cb[i % 3]);
         x_lig[idx] = __fadd_rn(__fmul_rn(alpha, x0), __fmul_rn(sigma, e));
     }
     for (int i = threadIdx.x; i < nl * F; i += blockDim.x) {
         const int idx = F * l0 + i;
-        const float e = noise ? noise[(size_t)b.n_lig * 3 + idx] : philox_normal_start(seed, -1, aoff + l0 + i / F, 3 + i % F);
+        const float e = d.noise ? d.noise[(size_t)b.n_lig * 3 + idx]
+                                : philox_normal(d.seed, -1, d.atom_offset + l0 + i / F, 3 + i % F);
         const float h0 = __fdiv_rn(h_start[idx], norm_c);
         h_lig[idx] = __fadd_rn(__fmul_rn(alpha, h0), __fmul_rn(sigma, e));
     }
     __syncthreads();
-    // remove the ligand COM from ligand and keypoints (as the plain loop does after its initial draw)
-    if (threadIdx.x < 3) {
-        float acc = 0.0f;
-        for (int j = 0; j < nl; ++j) acc = __fadd_rn(acc, x_lig[3 * (l0 + j) + threadIdx.x]);
-        com[threadIdx.x] = __fdiv_rn(acc, (float)nl);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) x_lig[3 * l0 + i] = __fsub_rn(x_lig[3 * l0 + i], com[i % 3]);
-    for (int i = threadIdx.x; i < nk * 3; i += blockDim.x) x_kp[3 * k0 + i] = __fsub_rn(x_kp[3 * k0 + i], com[i % 3]);
+    remove_ligand_com(x_lig, x_kp, l0, nl, k0, nk, com);   // as the plain loop does after its initial draw
 }
 
 int launch_partial_noise(const kpd_batch* b, const float* x_start, const float* h_start, float* x_lig, float* h_lig,
