@@ -321,7 +321,8 @@ typedef struct {
 } kpd_sampler_config;
 
 /* model: kpd_egnn_model* or kpd_gvp_model*.  kk is the static keypoint graph.  All buffers
- * (state, workspace) are caller-owned; the sampler only keeps pointers. */
+ * (state, workspace) are caller-owned; the sampler only keeps pointers.  coef (schedule.coefficient_table)
+ * is the default schedule of kpd_sampler_set_schedule. */
 int kpd_sampler_create(const kpd_sampler_config* cfg, const void* model, const kpd_batch* batch,
                        const kpd_graph_params* gp, const kpd_csr* kk, int32_t has_lk,
                        const float* coef /*[T,4] device*/, int32_t cap_ll, int32_t cap_kl,
@@ -374,6 +375,16 @@ int kpd_sampler_set_fragment(kpd_sampler* s, const uint8_t* fixed_mask, const fl
  * again. */
 int kpd_sampler_set_start(kpd_sampler* s, int32_t start_step, const float* x_start, const float* h_start,
                           float alpha, float sigma);
+/* The coefficient rows of the next runs (fewer-step sampling, DESIGN.md section 6.3): coef [n_rows,4] device rows
+ * (schedule.coefficient_rows over a step grid; row k is the reverse step tau_{k+1} -> tau_k) and, for an inpainting
+ * sampler (required there), coef2 [n_rows,4] (schedule.inpaint_rows over the same grid); 1 <= n_rows <= T.  A run
+ * then starts at row n_rows - 1, or at the start_step of kpd_sampler_set_start, which counts rows of this schedule
+ * and must be <= n_rows (checked by kpd_sampler_run); injected noise has the slots of a run of that many steps, and
+ * the Philox draws of row k are keyed by k.  coef = NULL restores the tables given at create time (T rows).  Only
+ * pointers are kept: every run copies the active rows into the sampler's own table (cudaMemcpyAsync on its stream),
+ * so a captured sampler serves any schedule without capturing again; the buffers must stay valid while runs use
+ * them. */
+int kpd_sampler_set_schedule(kpd_sampler* s, int32_t n_rows, const float* coef, const float* coef2);
 
 /* Output decode, the step right behind the path (reference test.py:199-203: torch.argmax(lig_feat, dim=1) on the
  * host, then dataset.lig_atom_idx_to_element): atom_type[i] = argmax_c h_lig[i, c], lowest index on ties. */

@@ -12,6 +12,8 @@
 //     step_prologue -> r x (graph_mark/scan/fill -> denoiser -> ddpm_inpaint_step [-> renoise])
 // A run from a start ligand (kpd_sampler_set_start) replaces the frame setup by one partial_noise launch and starts the
 // step counter at t0 instead of T; the captured graphs do not depend on the step, so they serve any t0.
+// Fewer-step sampling (kpd_sampler_set_schedule) swaps the coefficient rows: the step kernels read the sampler's own
+// [T,4] table, which every run fills from the active schedule, so one capture serves every schedule, eta and start.
 #include "common.cuh"
 #include <string.h>
 
@@ -23,10 +25,14 @@ struct kpd_sampler {
     kpd_batch batch;
     kpd_graph_params gp;
     kpd_csr ll, kl, lk, kk;
-    const float* coef;
+    const float* coef;        // create-time tables: the default schedule (T unit steps)
     int has_lk;
+    // the active schedule (kpd_sampler_set_schedule): NULL = the create-time tables, else sched_rows rows of each
+    const float *sched_coef, *sched_coef2;
+    int sched_rows;
     // device state carved from the caller's workspace
     float *x_lig, *h_lig, *x_kp, *h_kp, *v_kp, *eps_h, *eps_x, *kp_enc, *init_kp_com, *init_lig_pos, *t_cur;
+    float* coef_run;          // [T][4]: the rows of the active schedule, copied in by every run; what the steps read
     int *counter, *step;
     long long* edge_accum;
     RunParams* rp;
@@ -42,7 +48,7 @@ struct kpd_sampler {
     int atom_offset;
     // fragment-conditioned sampling (kpd_sampler_enable_inpainting): 0 = plain loop, else resamplings per step
     int resamplings;
-    InpaintParams frag;       // host copy, uploaded to frag_dev by every run
+    InpaintParams frag;       // host copy with the create-time coef2; every run uploads it with the active coef2
     InpaintParams* frag_dev;
     // partial noising (kpd_sampler_set_start): x_start == NULL = the plain start from pure noise at step T
     const float *x_start, *h_start;
@@ -81,6 +87,7 @@ static int carve_sampler(kpd_sampler* s, void* ws, int cap_ll, int cap_kl, int64
     s->init_kp_com = c.take<float>((int64_t)b.B * 3);
     s->init_lig_pos = c.take<float>((int64_t)b.B * 3);
     s->t_cur = c.take<float>(4);
+    s->coef_run = c.take<float>((int64_t)s->cfg.T * 4);
     s->rp = c.take<RunParams>(1);
     s->edge_accum = c.take<long long>(4);
     s->graph_ws = c.take<char>(kpd_graph_workspace_bytes(&b));
@@ -127,9 +134,9 @@ static int enqueue_denoiser(kpd_sampler* s, cudaStream_t st) {
 }
 
 static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
-    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef, st));
+    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef_run, st));
     KPD_TRY(enqueue_denoiser(s, st));
-    KPD_TRY(launch_ddpm_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->coef,
+    KPD_TRY(launch_ddpm_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->coef_run,
                              s->step, nullptr, nullptr, 0, s->rp, st));
     return 0;
 }
@@ -137,12 +144,12 @@ static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
 // one reverse step of the inpainting loop: prologue, then r x (graph build, denoiser, inpaint step[, re-noise])
 static int enqueue_inpaint_step(kpd_sampler* s, cudaStream_t st) {
     const int r = s->resamplings, F = s->cfg.atom_nf;
-    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef, st));
+    KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef_run, st));
     for (int u = 0; u < r; ++u) {
         KPD_TRY(enqueue_denoiser(s, st));
-        KPD_TRY(launch_ddpm_inpaint_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, F, s->coef, s->step,
-                                         u, r, InpaintParams{}, s->frag_dev, s->init_kp_com, s->cfg.lig_feat_norm_constant,
-                                         nullptr, 0, s->rp, st));
+        KPD_TRY(launch_ddpm_inpaint_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, F, s->coef_run,
+                                         s->step, u, r, InpaintParams{}, s->frag_dev, s->init_kp_com,
+                                         s->cfg.lig_feat_norm_constant, nullptr, 0, s->rp, st));
         if (u < r - 1)
             KPD_TRY(launch_renoise(&s->batch, s->x_lig, s->h_lig, s->x_kp, F, s->step, u, r, nullptr, s->frag_dev,
                                    nullptr, 0, s->rp, st));
@@ -240,6 +247,20 @@ extern "C" int kpd_sampler_set_start(kpd_sampler* s, int32_t start_step, const f
     return 0;
 }
 
+extern "C" int kpd_sampler_set_schedule(kpd_sampler* s, int32_t n_rows, const float* coef, const float* coef2) {
+    KPD_REQUIRE(s, "kpd_sampler_set_schedule: null sampler");
+    if (!coef) {
+        s->sched_coef = s->sched_coef2 = nullptr;
+        s->sched_rows = 0;
+        return 0;
+    }
+    KPD_REQUIRE(n_rows >= 1 && n_rows <= s->cfg.T, "kpd_sampler_set_schedule: %d rows outside [1, T = %d]", n_rows,
+                s->cfg.T);
+    KPD_REQUIRE(!s->resamplings || coef2, "kpd_sampler_set_schedule: an inpainting sampler needs coef2");
+    s->sched_coef = coef; s->sched_coef2 = coef2; s->sched_rows = n_rows;
+    return 0;
+}
+
 static int enqueue_any_step(kpd_sampler* s, cudaStream_t st) {
     return s->resamplings ? enqueue_inpaint_step(s, st) : enqueue_step(s, st);
 }
@@ -264,8 +285,13 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
                                uint64_t seed, int32_t n_steps, void* stream) {
     KPD_REQUIRE(s && x_kp && h_kp && init_lig_pos && x_lig && h_lig, "kpd_sampler_run: null argument");
     KPD_REQUIRE(s->cfg.arch == 0 || v_kp, "kpd_sampler_run: the GVP denoiser needs keypoint vectors v_kp");
-    // the first executed reverse step is t0 - 1: t0 = T from pure noise, the start step from a start ligand
-    const int t0 = s->x_start ? s->start_step : s->cfg.T;
+    // the first executed reverse step is row t0 - 1 of the active schedule: t0 = its row count from pure noise, the
+    // start step from a start ligand
+    const int rows = s->sched_coef ? s->sched_rows : s->cfg.T;
+    const float* coef = s->sched_coef ? s->sched_coef : s->coef;
+    const int t0 = s->x_start ? s->start_step : rows;
+    KPD_REQUIRE(t0 <= rows, "kpd_sampler_run: start step %d beyond the %d rows of the schedule", t0, rows);
+    KPD_REQUIRE(!s->resamplings || !s->sched_coef || s->sched_coef2, "kpd_sampler_run: the schedule has no coef2");
     KPD_REQUIRE(n_steps >= 0 && n_steps <= t0, "kpd_sampler_run: n_steps out of range");
     const kpd_batch& b = s->batch;
     const int F = s->cfg.atom_nf;
@@ -278,6 +304,7 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     CU(cudaMemcpyAsync(s->h_kp, h_kp, sizeof(float) * (size_t)s->kp_width * b.n_kp, cudaMemcpyDeviceToDevice, st));
     if (s->v_width) CU(cudaMemcpyAsync(s->v_kp, v_kp, sizeof(float) * (size_t)s->v_width * b.n_kp, cudaMemcpyDeviceToDevice, st));
     CU(cudaMemcpyAsync(s->init_lig_pos, init_lig_pos, sizeof(float) * 3 * b.B, cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemcpyAsync(s->coef_run, coef, sizeof(float) * 4 * (size_t)rows, cudaMemcpyDeviceToDevice, st));
     RunParams rp;
     rp.noise = noise; rp.seed = seed; rp.T = t0; rp.atom_offset = s->atom_offset;
     int counter0[4] = {t0, t0, 0, 0};
@@ -285,7 +312,11 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     CU(cudaMemcpyAsync(s->rp, &rp, sizeof(rp), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(s->counter, counter0, sizeof(counter0), cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(s->edge_accum, 0, 4 * sizeof(long long), st));
-    if (s->resamplings) CU(cudaMemcpyAsync(s->frag_dev, &s->frag, sizeof(InpaintParams), cudaMemcpyHostToDevice, st));
+    if (s->resamplings) {
+        InpaintParams frag = s->frag;
+        if (s->sched_coef) frag.coef2 = s->sched_coef2;
+        CU(cudaMemcpyAsync(s->frag_dev, &frag, sizeof(InpaintParams), cudaMemcpyHostToDevice, st));
+    }
 
     // frame setup (ligand_diffuser.py:348-370)
     KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 1, 0, s->init_kp_com, st));                // init_kp_com (:348)

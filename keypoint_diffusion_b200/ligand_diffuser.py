@@ -5,6 +5,8 @@ models/ligand_diffuser.py:24-538; the 1000-step loop of sample_from_encoded_rece
 replayed CUDA graph inside libkpdiff_b200.so (ops.Sampler).  Training (`forward`, losses) is
 out of scope (SURVEY.md section 8: sampling only) and raises NotImplementedError.
 """
+import math
+import numbers
 import os
 from math import ceil
 from pathlib import Path
@@ -17,8 +19,8 @@ from . import hetero, ops
 from .dynamics import LigRecDynamics, LigRecDynamicsGVP
 from .n_nodes_dist import LigandSizeDistribution
 from .receptor_encoder import ReceptorEncoder, ReceptorEncoderGVP
-from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_table, inpaint_table, sigma,
-                       sigma_and_alpha_t_given_s, start_coefficients)
+from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_rows, coefficient_table, inpaint_rows, inpaint_table,
+                       sigma, sigma_and_alpha_t_given_s, start_coefficients, step_grid)
 from .utils import get_batch_idxs, split_bounds
 
 DEFAULT_SUB_BATCHES = {"gvp": 4, "egnn": 2}      # measured on B200: profiles/r01_sweep_sub_batches_*.txt
@@ -80,6 +82,7 @@ class KeypointDiffusion(nn.Module):
         object.__setattr__(self, "_samplers", {})
         object.__setattr__(self, "_coef", {})
         object.__setattr__(self, "_coef2", {})
+        object.__setattr__(self, "_schedules", {})
         object.__setattr__(self, "last_launches_per_step", 0)
         object.__setattr__(self, "_streams", {})
         object.__setattr__(self, "cold_captures", 0)       # capacity buckets captured so far (a cold call each)
@@ -141,6 +144,24 @@ class KeypointDiffusion(nn.Module):
             self._coef2[key] = inpaint_table(self.gamma.gamma, self.n_timesteps).to(device)
         return self._coef2[key]
 
+    MAX_CACHED_SCHEDULES = 8
+
+    def schedule_tables(self, device, t_start: int, n: int, eta: Optional[float] = None, inpaint: bool = False):
+        """(coef [n,4], coef2 [n,4] or None) on `device`: the rows of the n-step grid over [0, t_start]
+        (schedule.step_grid), ancestral (eta=None) or DDIM(eta) (schedule.coefficient_rows), and with inpaint=True the
+        fragment rows over the same grid (schedule.inpaint_rows).  n scalar rows cost milliseconds on the host; the
+        last few schedules are cached (per device and gamma version), least recently used evicted first."""
+        key = (str(device), self.gamma.gamma._version, self.gamma.gamma.data_ptr(), int(t_start), int(n),
+               None if eta is None else float(eta), bool(inpaint))
+        hit = self._schedules.pop(key, None)
+        if hit is None:
+            grid, T, g = step_grid(t_start, n), self.n_timesteps, self.gamma.gamma
+            hit = (coefficient_rows(g, T, grid, eta).to(device), inpaint_rows(g, T, grid).to(device) if inpaint else None)
+            while len(self._schedules) >= self.MAX_CACHED_SCHEDULES:
+                self._schedules.pop(next(iter(self._schedules)))
+        self._schedules[key] = hit
+        return hit
+
     # ------------------------------------------------------------------ one reverse step (reference :497-538)
     @torch.no_grad()
     def sample_p_zs_given_zt(self, s: torch.Tensor, t: torch.Tensor, g, batch_idxs=None, noise=None,
@@ -150,19 +171,31 @@ class KeypointDiffusion(nn.Module):
         (default) a fresh seed is drawn from torch's global generator on every call, so a caller driving the
         reference-style per-step loop gets new noise per step, per batch and per run, and torch.manual_seed makes it
         reproducible -- like the reference's torch.randn draws (ligand_diffuser.py:520-527).  An explicit seed is
-        deterministic: same (seed, step, atom, channel) -> same draw."""
+        deterministic: same (seed, step, atom, channel) -> same draw.
+
+        Like the reference, any t > s is a step: t_int = round(t T) must exceed s_int = round(s T) (ValueError
+        otherwise).  A strided step (t_int > s_int + 1) uses the row (s_int, t_int) of schedule.coefficient_rows; its
+        Philox draws stay keyed by s_int."""
+        T = self.n_timesteps
+        s_int = int(torch.round(s.flatten()[0] * T).item())
+        t_int = int(torch.round(t.flatten()[0] * T).item())
+        if not s_int < t_int <= T:
+            raise ValueError(f"a reverse step needs s < t <= 1, got s = {s_int}/{T}, t = {t_int}/{T}")
         if seed is None and noise is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         seed = 0 if seed is None else seed
         batch, _ = self._layout(g)
         eps_h, eps_x = self.dynamics(g, t, batch_idxs)
-        s_int = int(torch.round(s.flatten()[0] * self.n_timesteps).item())
         step = torch.tensor([s_int], dtype=torch.int32, device=g.device)
+        coef = self.coef_table(g.device)
+        if t_int != s_int + 1:      # the kernel reads row s_int: the strided row goes there
+            coef = torch.zeros(s_int + 1, 4, device=g.device)
+            coef[s_int] = coefficient_rows(self.gamma.gamma, T, [s_int, t_int])[0].to(g.device)
         x_lig = g.nodes['lig'].data['x_0'].float().contiguous()
         h_lig = g.nodes['lig'].data['h_0'].float().contiguous()
         x_kp = g.nodes['kp'].data['x_0'].float().contiguous()
         nx, nh = (None, None) if noise is None else (noise[0].float().contiguous(), noise[1].float().contiguous())
-        ops.ddpm_step(batch, x_lig, h_lig, x_kp, eps_x, eps_h, self.coef_table(g.device), step, nx, nh, seed)
+        ops.ddpm_step(batch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, step, nx, nh, seed)
         g.nodes['lig'].data['x_0'], g.nodes['lig'].data['h_0'], g.nodes['kp'].data['x_0'] = x_lig, h_lig, x_kp
         return g
 
@@ -262,7 +295,8 @@ class KeypointDiffusion(nn.Module):
                                       decode: bool = False, capacity: bool = True, fixed_mask: torch.Tensor = None,
                                       fixed_pos: torch.Tensor = None, fixed_feat: torch.Tensor = None,
                                       resamplings: int = 1, start_pos: torch.Tensor = None,
-                                      start_feat: torch.Tensor = None, start_step: Optional[int] = None):
+                                      start_feat: torch.Tensor = None, start_step: Optional[int] = None,
+                                      timesteps: Optional[int] = None, eta: Optional[float] = None):
         """Returns (lig_pos, lig_feat): one CPU tensor per complex, as the reference does (:342-469).  ``g`` may live
         on the CPU (pinned or not): its keypoint tensors are uploaded here, straight into the sampler's buffers -- the
         host->device boundary of the path (reference test.py:152-161).
@@ -286,7 +320,14 @@ class KeypointDiffusion(nn.Module):
         noised to level t0, and the loop runs the t0 reverse steps t0-1 .. 0 (about t0/T of a plain call): a small t0
         gives close variants, a large one ligands that only loosely follow the start.  The frame is the start ligands'
         own: ``init_lig_pos`` is not used and must not be given.  Composes with a fragment (which then stays pinned) and
-        with sub-batches; capacity path only."""
+        with sub-batches; capacity path only.
+
+        Fewer-step sampling (DESIGN.md section 6.3): ``timesteps`` = n in [1, t_start] (t_start = T, or t0 of a start
+        ligand) runs n reverse steps on the grid tau_k = (k t_start) // n instead of every step, for about n / t_start
+        of the cost; ``eta`` in [0, 1] makes them DDIM(eta) steps instead of ancestral ones (eta = 0: deterministic
+        steps, though a fragment's known part is still noised at every step).  timesteps = t_start with eta=None is the
+        default run bit for bit; eta alone keeps every step.  Composes with fragments, start ligands and sub-batches,
+        captures nothing new; capacity path only, and not with start_step = 0."""
         n_lig_total = int(g.num_nodes('lig'))
         inpaint = self._check_fragment_args(n_lig_total, fixed_mask, fixed_pos, fixed_feat, resamplings)
         start = self._check_start_args(n_lig_total, start_pos, start_feat, start_step)
@@ -296,6 +337,8 @@ class KeypointDiffusion(nn.Module):
             raise ValueError("sampling from a start ligand runs on the capacity path only (capacity=True)")
         if start and init_lig_pos is not None:
             raise ValueError("init_lig_pos is not used with a start ligand (the start ligands' means set the frame)")
+        t_start = int(start_step) if start else self.n_timesteps
+        n_sched = self._check_schedule_args(timesteps, eta, t_start, capacity)
         if visualize:
             raise NotImplementedError("visualize=True (a per-step CPU copy of the whole graph) is a debug feature "
                                       "outside the throughput path")
@@ -314,6 +357,7 @@ class KeypointDiffusion(nn.Module):
             init_pos = hetero.readout_nodes(g, feat='x_0', op='mean', ntype='rec')
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())      # follows torch.manual_seed like the reference
+        sched = None if n_sched is None else self.schedule_tables(dev, t_start, n_sched, eta, inpaint)
         n_sub = self.default_sub_batches(batch_size) if sub_batches is None else max(1, min(int(sub_batches), batch_size))
         if noise is not None:
             n_sub = 1          # injected noise (parity runs) is laid out for the undivided batch
@@ -357,7 +401,7 @@ class KeypointDiffusion(nn.Module):
             st_rows = None
             if start:
                 l1 = lig_ptr[b]
-                st_rows = (start_pos[l0:l1], start_feat[l0:l1], int(start_step), a_t0, s_t0)
+                st_rows = (start_pos[l0:l1], start_feat[l0:l1], t_start if n_sched is None else n_sched, a_t0, s_t0)
             if n_sub > 1 and (slot, str(dev)) not in self._streams:
                 self._streams[(slot, str(dev))] = torch.cuda.Stream(device=dev)
             st = self._streams[(slot, str(dev))] if n_sub > 1 else cur
@@ -366,7 +410,7 @@ class KeypointDiffusion(nn.Module):
             with torch.cuda.stream(st):
                 out = smp.run(plan, kp['x_0'][k0:k1], kp['h_0'][k0:k1], kv[k0:k1] if kv is not None else None, gs, gd,
                               init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag,
-                              start=st_rows)
+                              start=st_rows, schedule=sched)
             if n_sub > 1:
                 for t in out:
                     t.record_stream(cur)
@@ -386,6 +430,25 @@ class KeypointDiffusion(nn.Module):
         pos_cpu, feat_cpu = x_lig.cpu(), h_lig.cpu()                # device -> host boundary (reference :464)
         res = (list(torch.split(pos_cpu, lig_n)), list(torch.split(feat_cpu, lig_n)))
         return res + (list(torch.split(atom_type.cpu(), lig_n)),) if decode else res
+
+    def _check_schedule_args(self, timesteps, eta, t_start: int, capacity) -> Optional[int]:
+        """ValueError for a bad fewer-step request (host-side checks, before any device work); the step count of the
+        schedule to run, or None for the default tables."""
+        if timesteps is not None:
+            if isinstance(timesteps, bool) or not isinstance(timesteps, numbers.Integral):
+                raise ValueError(f"timesteps must be an int, got {timesteps!r}")
+            if t_start == 0:
+                raise ValueError("timesteps must be None with start_step = 0 (no reverse step runs)")
+            if not 1 <= int(timesteps) <= t_start:
+                raise ValueError(f"timesteps must be in [1, {t_start}], got {timesteps}")
+        if eta is not None and (isinstance(eta, bool) or not isinstance(eta, numbers.Real) or not math.isfinite(eta)
+                                or not 0 <= eta <= 1):
+            raise ValueError(f"eta must be a finite number in [0, 1], got {eta!r}")
+        if (timesteps is not None or eta is not None) and not capacity:
+            raise ValueError("fewer-step sampling runs on the capacity path only (capacity=True)")
+        if (timesteps is None and eta is None) or t_start == 0:
+            return None
+        return t_start if timesteps is None else int(timesteps)
 
     def _check_fragment_args(self, n_lig: int, fixed_mask, fixed_pos, fixed_feat, resamplings) -> bool:
         """ValueError for an inconsistent fragment request (host-side checks, before any device work); True when the
@@ -565,7 +628,8 @@ class KeypointDiffusion(nn.Module):
                 start_ligands: Optional[List] = None, start_step: Optional[int] = None, **sampler_kw):
         """ref_graphs: one single-complex graph per receptor (reference :270-340).  ``encoded=True`` skips the receptor
         encoder (graphs already hold kp nodes + kk edges).  init_lig_pos: optional [3] tensor per receptor.
-        noise: optional injected Gaussian draws, one [T+1, n_lig*(3+F)] tensor per diffusion batch (parity runs).
+        noise: optional injected Gaussian draws, one [n+1, n_lig*(3+F)] tensor per diffusion batch (parity runs), n the
+        reverse steps a call runs: T, t0 of start ligands, or ``timesteps``.
         complexes: optional subset (indices into the flattened receptor-major list of requested ligands) to sample --
         what sample_sharded deals to this rank; the returned lists then hold only those.
         fragments: optional, one ``(pos [m,3], feat [m,F])`` or None per receptor: every ligand requested for that
@@ -576,11 +640,15 @@ class KeypointDiffusion(nn.Module):
         ligand requested for that receptor (each of size m) is a variant of its start ligand, noised to level t0 and
         denoised from there (ligand optimisation, see sample_from_encoded_receptors); with fragments too, the fragment
         is the start ligand's first atoms and stays pinned.
+        timesteps / eta (passed on to sample_from_encoded_receptors, like every other keyword): fewer-step sampling,
+        checked here before any receptor is encoded.
 
         The diffusion batches are assembled on the device (hetero.expand_complexes): no per-complex graph copies."""
         has_fragment = self._check_fragments(fragments, n_lig_atoms, resamplings)
         has_start = self._check_start_ligands(start_ligands, start_step, n_lig_atoms, init_lig_pos, use_ref_lig_com,
                                               sampler_kw)
+        self._check_schedule_args(sampler_kw.get("timesteps"), sampler_kw.get("eta"),
+                                  int(start_step) if has_start else self.n_timesteps, sampler_kw.get("capacity", True))
         n_receptors = len(ref_graphs)
         enc, rec_mean = self._encode_all(ref_graphs, rec_enc_batch_size, encoded)
         dev = enc.device

@@ -453,7 +453,8 @@ class Sampler:
     resamplings >= 1 with inpaint_coef (schedule.inpaint_table on the device) makes it a fragment-conditioned
     (inpainting) sampler: every reverse step runs `resamplings` denoiser passes with the atoms given to set_fragment
     pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop.
-    Either kind runs from a given ligand after set_start (ligand optimisation by partial noising)."""
+    Either kind runs from a given ligand after set_start (ligand optimisation by partial noising), and with fewer,
+    strided or DDIM steps after set_schedule; neither captures again."""
 
     def __init__(self, model: _Model, batch: DeviceBatch, gp: GraphParams, kk: Optional[Csr], coef: torch.Tensor,
                  T: int, atom_nf: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
@@ -487,6 +488,7 @@ class Sampler:
         self.inpaint_coef = inpaint_coef
         self._fragment = None
         self._start = None
+        self._schedule = None
         if self.resamplings:
             _require_cuda(inpaint_coef)
             check(lib.kpd_sampler_enable_inpainting(self.handle, self.resamplings, ptr(inpaint_coef)),
@@ -526,10 +528,37 @@ class Sampler:
                                         float(sigma)), "kpd_sampler_set_start")
         self._start = (int(start_step), x_start, h_start)
 
+    def set_schedule(self, coef: Optional[torch.Tensor] = None, coef2: Optional[torch.Tensor] = None):
+        """The coefficient rows of the next runs (kpd_sampler_set_schedule; fewer-step sampling, DESIGN.md section 6.3):
+        coef fp32 [n,4] on the device, 1 <= n <= T (schedule.coefficient_rows over a step grid) and, for an inpainting
+        sampler, coef2 [n,4] (schedule.inpaint_rows over the same grid).  Runs then take n steps (rows n-1 .. 0), or
+        start_step of set_start, which counts rows of this schedule.  coef=None restores the create-time tables.  The
+        tensors must stay alive and in place while runs use them (only their addresses are kept)."""
+        if coef is None:
+            check(lib.kpd_sampler_set_schedule(self.handle, 0, None, None), "kpd_sampler_set_schedule")
+            self._schedule = None
+            return
+        n = int(coef.shape[0])
+        for c in (coef, coef2) if self.resamplings else (coef,):
+            if c is None:
+                raise ValueError("an inpainting sampler needs coef2 with its schedule")
+            _require_cuda(c)
+            assert c.dtype == torch.float32 and c.is_contiguous() and tuple(c.shape) == (n, 4)
+        if not 1 <= n <= self.T:
+            raise ValueError(f"a schedule has 1 .. {self.T} rows, got {n}")
+        check(lib.kpd_sampler_set_schedule(self.handle, n, ptr(coef), ptr(coef2) if self.resamplings else None),
+              "kpd_sampler_set_schedule")
+        self._schedule = (coef, coef2)
+
+    @property
+    def schedule_rows(self) -> int:
+        """Rows of the active schedule: T, or n of set_schedule."""
+        return self.T if self._schedule is None else int(self._schedule[0].shape[0])
+
     @property
     def start_step(self) -> int:
-        """The step runs start from: T, or the start step of set_start."""
-        return self.T if self._start is None else self._start[0]
+        """The row runs start from: the rows of the active schedule, or the start step of set_start."""
+        return self.schedule_rows if self._start is None else self._start[0]
 
     @property
     def noise_slots(self) -> int:
@@ -694,12 +723,15 @@ class CapacitySampler:
 
     def run(self, plan: CapacityPlan, x_kp, h_kp, v_kp, kk_src, kk_dst, init_pos, seed: int, atom_offset: int = 0,
             noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None,
-            start: Optional[Tuple] = None):
+            start: Optional[Tuple] = None, schedule: Optional[Tuple] = None):
         """x_kp/h_kp/v_kp: the REAL keypoint rows (host or device tensors; pinned host tensors are uploaded straight
         into the capacity buffers); kk_src/kk_dst: kk edges in this batch's own keypoint numbering; init_pos [B_real,3].
         fragment (inpainting samplers): (fixed_mask [N_real] bool, x_fix [N_real,3], h_fix [N_real,F]) or None.
         start: (x [N_real,3], h [N_real,F], t0, alpha_t0, sigma_t0) -- run t0 reverse steps from that ligand (see
         Sampler.set_start) -- or None for the plain start; injected noise then has the slots of a t0-step run.
+        schedule: (coef [n,4], coef2 [n,4] or None) on the device -- run the n rows of that schedule (see
+        Sampler.set_schedule; t0 of start then counts its rows) -- or None for the create-time tables.  A run-time
+        value like the start: no new capture.
         -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]]) on the device."""
         if plan.key != self.key:
             raise ValueError("CapacitySampler.run: the plan belongs to another capacity bucket")
@@ -721,6 +753,7 @@ class CapacitySampler:
             self.sampler.set_start(int(start[2]), self.x_start, self.h_start, float(start[3]), float(start[4]))
         else:
             self.sampler.set_start(None)
+        self.sampler.set_schedule(*(schedule or ()))
         self.x_kp[:K_r].copy_(x_kp, non_blocking=True)
         self.h_kp[:K_r].copy_(h_kp, non_blocking=True)
         if self.v_kp is not None:

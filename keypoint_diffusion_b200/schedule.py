@@ -7,7 +7,9 @@ sigma, t) is what the CUDA step kernel reads; it restates models/ligand_diffuser
 :505-527 on the host, once per model (the values are identical for every complex of a batch).
 inpaint_table [T,4] = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) is the second table that
 fragment-conditioned sampling reads (DESIGN.md section 6.1); start_coefficients gives (alpha_t0, sigma_t0), the
-forward noising of a start ligand in ligand optimisation (section 6.2).
+forward noising of a start ligand in ligand optimisation (section 6.2).  Both tables are the unit-step case of
+coefficient_rows / inpaint_rows over a step grid (step_grid), which also give the strided ancestral and DDIM rows of
+fewer-step sampling (section 6.3).
 """
 import numpy as np
 import torch
@@ -73,40 +75,78 @@ def sigma_and_alpha_t_given_s(gamma_t, gamma_s):
     return sigma2_t_given_s, torch.sqrt(sigma2_t_given_s), alpha_t_given_s
 
 
-def coefficient_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
-    """fp32 [T,4] on the CPU; row s = (alpha_t|s, var_terms, sigma, t=(s+1)/T).
+def step_grid(t_start: int, n: int) -> list:
+    """The n-step grid tau_k = (k t_start) // n, k = 0..n (DESIGN.md section 6.3): tau_0 = 0, tau_n = t_start, strictly
+    increasing; row k of a grid table is the reverse step tau_{k+1} -> tau_k.  n = t_start is the unit grid."""
+    t_start, n = int(t_start), int(n)
+    if not 1 <= n <= t_start:
+        raise ValueError(f"a step grid over [0, {t_start}] needs 1 <= n <= {t_start}, got n = {n}")
+    return [k * t_start // n for k in range(n + 1)]
 
-    Evaluated row by row on 1-element fp32 tensors with the same torch ops the reference applies
-    per step (ligand_diffuser.py:405-408, :505-527).  (A vectorised evaluation over all T rows
-    differs in the last bit because torch's SIMD and scalar transcendental paths round
-    differently; the scalar path is what the oracle pins.)"""
+
+def _row_gammas(g, T, s_int, t_int):
+    """(gamma_s, gamma_t, t) of the step t_int -> s_int as 1-element fp32 tensors, looked up as the reference does
+    (ligand_diffuser.py:405-408, :688-690)."""
+    s = torch.full((1,), s_int) / T
+    t = torch.full((1,), t_int) / T
+    return g[torch.round(s * T).long()], g[torch.round(t * T).long()], t
+
+
+def _ddim_columns(gs, gt, eta: float):
+    """(vt, sg) of a DDIM(eta) row, in fp64 from the fp32 gammas, rounded once to fp32 (DESIGN.md section 6.3):
+    rho = sigma2_t|s / sigma_t^2, vt = (sigma_t / alpha_t|s) rho (1 + eta^2 - eta^2 rho) / (1 + sqrt((1-rho)(1-eta^2 rho))),
+    sg = eta sqrt(rho) sigma_s."""
+    gs, gt = gs.double(), gt.double()
+    s2 = -torch.expm1(F.softplus(gs) - F.softplus(gt))
+    a = torch.exp(0.5 * (F.logsigmoid(-gt) - F.logsigmoid(-gs)))
+    sig2_t = torch.sigmoid(gt)
+    rho = s2 / sig2_t
+    e2 = float(eta) ** 2
+    vt = torch.sqrt(sig2_t) / a * rho * (1 + e2 - e2 * rho) / (1 + torch.sqrt((1 - rho) * (1 - e2 * rho)))
+    sg = float(eta) * torch.sqrt(rho) * torch.sqrt(torch.sigmoid(gs))
+    return vt.float(), sg.float()
+
+
+def coefficient_rows(gamma: torch.Tensor, T: int, grid, eta=None) -> torch.Tensor:
+    """fp32 [n,4] on the CPU over a step grid (step_grid): row k = (alpha_t|s, var_terms, sigma, t = tau_{k+1}/T) of the
+    reverse step tau_{k+1} -> tau_k, the reference's sample_p_zs_given_zt at (s, t) = (tau_k/T, tau_{k+1}/T).
+
+    Evaluated row by row on 1-element fp32 tensors with the same torch ops the reference applies per step
+    (ligand_diffuser.py:405-408, :505-527).  (A vectorised evaluation over all rows differs in the last bit because
+    torch's SIMD and scalar transcendental paths round differently; the scalar path is what the oracle pins.)
+    eta in [0, 1]: DDIM(eta) rows instead -- columns 0 and 3 as above, columns 1 and 2 from _ddim_columns."""
     g = gamma.detach().float().cpu()
     rows = []
-    for s_int in range(T):
-        s = torch.full((1,), s_int) / T
-        t = (torch.full((1,), s_int) + 1) / T
-        gs = g[torch.round(s * T).long()]
-        gt = g[torch.round(t * T).long()]
+    for s_int, t_int in zip(grid[:-1], grid[1:]):
+        gs, gt, t = _row_gammas(g, T, s_int, t_int)
         s2, s1, a = sigma_and_alpha_t_given_s(gt, gs)
         sig_s, sig_t = sigma(gs), sigma(gt)
-        rows.append(torch.stack([a[0], (s2 / a / sig_t)[0], (s1 * sig_s / sig_t)[0], t[0].float()]))
+        vt, sg = (s2 / a / sig_t, s1 * sig_s / sig_t) if eta is None else _ddim_columns(gs, gt, eta)
+        rows.append(torch.stack([a[0], vt[0], sg[0], t[0].float()]))
+    return torch.stack(rows).contiguous()
+
+
+def coefficient_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
+    """fp32 [T,4] on the CPU; row s = (alpha_t|s, var_terms, sigma, t=(s+1)/T): coefficient_rows over the unit grid."""
+    return coefficient_rows(gamma, T, list(range(T + 1)))
+
+
+def inpaint_rows(gamma: torch.Tensor, T: int, grid) -> torch.Tensor:
+    """fp32 [n,4] on the CPU over a step grid; row k = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) with (s, t) = (tau_k,
+    tau_{k+1}): the known-part noising and the re-noise coefficients of fragment-conditioned sampling.  Evaluated like
+    coefficient_rows (scalar fp32 ops, row by row), so its alpha_t|s column equals coefficient_rows' column 0 bit for bit."""
+    g = gamma.detach().float().cpu()
+    rows = []
+    for s_int, t_int in zip(grid[:-1], grid[1:]):
+        gs, gt, _ = _row_gammas(g, T, s_int, t_int)
+        _, s1, a = sigma_and_alpha_t_given_s(gt, gs)
+        rows.append(torch.stack([alpha(gs)[0], sigma(gs)[0], a[0], s1[0]]))
     return torch.stack(rows).contiguous()
 
 
 def inpaint_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
-    """fp32 [T,4] on the CPU; row s = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) with t = s+1: the known-part noising
-    and the re-noise coefficients of fragment-conditioned sampling.  Evaluated like coefficient_table (scalar fp32 ops,
-    row by row), so its alpha_t|s column equals coefficient_table's column 0 bit for bit."""
-    g = gamma.detach().float().cpu()
-    rows = []
-    for s_int in range(T):
-        s = torch.full((1,), s_int) / T
-        t = (torch.full((1,), s_int) + 1) / T
-        gs = g[torch.round(s * T).long()]
-        gt = g[torch.round(t * T).long()]
-        _, s1, a = sigma_and_alpha_t_given_s(gt, gs)
-        rows.append(torch.stack([alpha(gs)[0], sigma(gs)[0], a[0], s1[0]]))
-    return torch.stack(rows).contiguous()
+    """fp32 [T,4] on the CPU: inpaint_rows over the unit grid (row s: t = s+1)."""
+    return inpaint_rows(gamma, T, list(range(T + 1)))
 
 
 def start_coefficients(gamma: torch.Tensor, t0: int):
