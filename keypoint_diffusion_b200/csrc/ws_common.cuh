@@ -93,6 +93,42 @@ __device__ __forceinline__ float act_silu(float x) { return NS == 1 ? silu_fast(
 template <int NS>
 __device__ __forceinline__ float act_sigmoid(float x) { return NS == 1 ? sigmoid_fast(x) : sigmoid_acc(x); }
 
+// Paired fp32 arithmetic (FADD2 / FMUL2 / FFMA2: two IEEE round-to-nearest operations in one instruction, the same bits
+// as two scalar ones -- no .ftz, no contraction).  The operands of one instruction live in an aligned register pair, so
+// the bf16x3 epilogues keep their values as float2.
+__device__ __forceinline__ float2 add2(float2 a, float2 b) { return __fadd2_rn(a, b); }
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
+__device__ __forceinline__ float2 sub2(float2 a, float2 b) {
+    unsigned long long d;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(*reinterpret_cast<unsigned long long*>(&a)), "l"(*reinterpret_cast<unsigned long long*>(&b)));
+    return *reinterpret_cast<float2*>(&d);
+}
+__device__ __forceinline__ float2 bcast2(float x) { return make_float2(x, x); }
+__device__ __forceinline__ float2 u2f2(uint32_t a, uint32_t b) { return make_float2(__uint_as_float(a), __uint_as_float(b)); }
+
+// fp32-grade logistic of two values on three MUFU ops: an ex2 each and ONE reciprocal shared through the product of the
+// denominators, sigmoid(x0) = d1 / (d0 d1).  The ex2 argument is clamped at 62: then d <= 2^62 + 1, d0 d1 <= 2^124 stays
+// finite and its reciprocal >= 2^-124 stays normal under .ftz (an unclamped e = inf would give 0 * inf = NaN).  The clamp
+// only acts for x < -42.9, where sigmoid(x) < 2^-62: the result is off by less than 2^-62 absolute.  The product and the
+// extra multiply add two fp32 roundings to the ~2^-22 of ex2 and rcp.
+__device__ __forceinline__ float2 sigmoid2_acc(float2 x) {
+    const float2 t = mul2(x, bcast2(-1.4426950408889634f));
+    float e0, e1, r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fminf(t.x, 62.f)));
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(fminf(t.y, 62.f)));
+    const float2 d = add2(bcast2(1.f), make_float2(e0, e1));
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d.x * d.y));
+    return mul2(bcast2(r), make_float2(d.y, d.x));
+}
+__device__ __forceinline__ float2 silu2_acc(float2 x) { return mul2(x, sigmoid2_acc(x)); }
+
+// 2 fp32 values -> packed bf16 pair hi and the packed bf16 pair of the residuals lo
+__device__ __forceinline__ void split2(float2 f, uint32_t& hi, uint32_t& lo) {
+    hi = tc::pack_bf16x2(f.x, f.y);
+    const float2 r = sub2(f, u2f2(hi << 16, hi & 0xffff0000u));
+    lo = tc::pack_bf16x2(r.x, r.y);
+}
 
 // 8 fp32 values -> packed bf16 hi (and the bf16 residual lo)
 __device__ __forceinline__ void split8(const float (&f)[8], uint4& hi, uint4& lo) {
