@@ -430,7 +430,7 @@ extern "C" int kpd_egnn_attach_tc(kpd_egnn_model* m, const void* tc_blob, const 
     const int per_layer = 2 + m->n_et * 2 + m->n_upd * 2;
     KPD_REQUIRE(n == m->cfg.n_layers * per_layer, "kpd_egnn_attach_tc: expected %d offsets, got %d", m->cfg.n_layers * per_layer, n);
     KPD_REQUIRE((reinterpret_cast<uintptr_t>(tc_blob) & 127) == 0, "kpd_egnn_attach_tc: blob must be 128-byte aligned");
-    KPD_REQUIRE(m->nmain % 8 == 0 && m->H <= 257, "kpd_egnn_attach_tc: hidden width %d unsupported by the tensor-core tiles", m->H);
+    KPD_REQUIRE(m->nmain >= 8 && m->nmain % 8 == 0 && m->H <= 257, "kpd_egnn_attach_tc: hidden width %d unsupported by the tensor-core tiles", m->H);
     const size_t smem = m->edge_smem_ws[nsplit - 1];
     KPD_REQUIRE(smem <= 227 * 1024, "kpd_egnn_attach_tc: tile needs %zu B of shared memory", smem);
     const char* base = static_cast<const char*>(tc_blob);

@@ -233,6 +233,22 @@ class _Model:
         return ws
 
 
+def egnn_has_tc_tiles(hidden_nf: int) -> bool:
+    """Whether the EGNN tensor-core modes take this width (csrc/egnn.cu kpd_egnn_attach_tc): H = hidden_nf + 1 <= 257
+    and nmain = min(H, 256) rounded down to a multiple of 4 is a non-zero multiple of 8 (the nmain output columns are
+    one MMA of N = nmain padded to 16; the H - nmain <= 3 leftover columns run beside it).  Other widths run the fp32
+    SIMT kernels."""
+    H = hidden_nf + 1
+    nmain = min(H, 256) // 4 * 4
+    return H <= 257 and nmain >= 8 and nmain % 8 == 0
+
+
+def gvp_has_tc_tiles(n_hidden_scalars: int) -> bool:
+    """Whether the GVP tensor-core modes take this scalar width (csrc/gvp.cu kpd_gvp_attach_tc); other widths the
+    library accepts (multiples of 4 up to 256) run the fp32 SIMT kernels."""
+    return n_hidden_scalars % 16 == 0
+
+
 class EgnnModel(_Model):
     """Packed EGNN denoiser weights on the device (kpd_egnn_model)."""
     arch = 0
@@ -257,8 +273,7 @@ class EgnnModel(_Model):
         self.precision = "fp32"
         self.tc_blob = self.tc_blob2 = None
         self._sd_bf16 = None
-        H = hidden_nf + 1
-        if (min(H, 256) // 4 * 4) % 8 == 0 and H <= 257:
+        if egnn_has_tc_tiles(hidden_nf):
             self.tc_blob2 = self._attach_tc(sd, split=True)
             # the plain-bf16 pack is built on the first set_precision('bf16') (from a reference to sd, not a copy): a
             # model that never uses that mode costs no more to create and holds no more packed weights
@@ -340,7 +355,7 @@ class GvpModel(_Model):
         check(lib.kpd_gvp_create(C.byref(cfg), ptr(self.blob), arr, len(offs), C.byref(self.handle)), "kpd_gvp_create")
         self.precision = "fp32"
         self.tc_blob = self.tc_blob2 = None
-        if n_hidden_scalars % 16 == 0:
+        if gvp_has_tc_tiles(n_hidden_scalars):
             kw = dict(n_convs=n_convs, update_kp=update_kp, n_message_gvps=n_message_gvps, n_update_gvps=n_update_gvps,
                       n_noise_gvps=n_noise_gvps, device=self.device)
             self.tc_blob, toffs = pack.pack_gvp_tc(sd, **kw)

@@ -116,7 +116,7 @@ def pack_egnn(sd: Dict[str, torch.Tensor], *, atom_nf, rec_nf, hidden_nf, n_laye
                 W2 = sd[f"{q}{mlp}.{et}.2.weight"].detach().float().cpu()         # [H, H]
                 put(_padcols(W2.t().contiguous(), Hp))                             # W2T
                 put(_padvec(sd[f"{q}{mlp}.{et}.2.bias"].detach().float().cpu(), Hp))
-                lo = torch.zeros(3, Hp)
+                lo = torch.zeros(max(3, nlo), Hp)       # nlo > 3 is refused by kpd_egnn_create, with its reason
                 if nlo:
                     lo[:nlo, :H] = W2[nmain:H, :]
                 put(lo)                                                            # W2lo

@@ -96,3 +96,60 @@ def test_pack_egnn_tc_entries():
     full_blocks, tail = divmod(n_rows, 256)
     expect = (full_blocks * 256 + (tail + 15) // 16 * 16) * ks * 16 * 2 * 2          # bf16 bytes, hi + lo
     assert first == (expect + 127) // 128 * 128
+
+
+def _slab_bytes(n_rows, K, split=True):
+    """Bytes of pack_tc_weight of an [n_rows, K] weight, padded to the 128-byte entry alignment."""
+    ks = (K + 15) // 16
+    rows = sum((min(256, n_rows - n0) + 15) // 16 * 16 for n0 in range(0, n_rows, 256))
+    return (rows * ks * 16 * (2 if split else 1) * 2 + 127) // 128 * 128
+
+
+def test_egnn_tensor_core_rule_and_pack_at_every_width():
+    """hidden_nf 1..259: the tensor-core modes are attached exactly for 8 <= H <= 257 with H % 8 < 4 (nmain = H & ~3 a
+    non-zero multiple of 8); hidden_nf 1 and 2 (nmain = 0) fall back to fp32.  At every such width pack_egnn_tc gives
+    one entry per GEMM, the edge GEMMs nmain output rows padded to 16."""
+    from oracle import params as P
+    from keypoint_diffusion_b200 import ops
+    accepted = []
+    for hid in range(1, 260):
+        H = hid + 1
+        tc = ops.egnn_has_tc_tiles(hid)
+        assert tc == (8 <= H <= 257 and H % 8 < 4), hid
+        if not tc:
+            continue
+        accepted.append(hid)
+        kp = hid % 2 == 0
+        sd = P.init_state_dict(P.egnn_dynamics_shapes(3, 5, 1, hid, kp, False), seed=hid)
+        sd = {k[len("dynamics."):]: v for k, v in sd.items()}
+        blob, offs = pack.pack_egnn_tc(sd, hidden_nf=hid, n_layers=1, update_kp_feat=kp, device="cpu", split=True)
+        n_et, n_upd = (4, 2) if kp else (2, 1)
+        assert len(offs) == 2 + 2 * n_et + 2 * n_upd and all(o % 128 == 0 for o in offs), hid
+        nmain, Hp = min(H, 256) // 4 * 4, (H + 3) // 4 * 4
+        sizes = [b - a for a, b in zip(offs, offs[1:] + [2 * blob.numel()])]
+        assert sizes[2:2 + 2 * n_et] == [_slab_bytes(nmain, H)] * (2 * n_et), hid
+        assert sizes[2 + 2 * n_et:] == [_slab_bytes(H, 2 * Hp), _slab_bytes(H, H)] * n_upd, hid
+    assert accepted[0] == 7 and accepted[-1] == 256 and 255 in accepted and 257 not in accepted
+    assert 36 not in accepted and 1 not in accepted and 2 not in accepted
+
+
+def test_gvp_tensor_core_rule_and_pack_at_every_width():
+    """S = 4..256 step 4, V in {1, 16}, rbf_dim in {2, 32}: the tensor-core modes exactly at S % 16 == 0; there
+    pack_gvp_tc gives three 128-byte-aligned entries per GVP, to_feats_out padded to 16 rows over K = hd + fin."""
+    from oracle import params as P
+    from keypoint_diffusion_b200 import ops
+    for S in range(4, 257, 4):
+        assert ops.gvp_has_tc_tiles(S) == (S % 16 == 0)
+        if S % 16:
+            continue
+        for V in (1, 16):
+            for rbf in (2, 32):
+                sd = P.init_state_dict(P.gvp_dynamics_shapes(10, 12, V, 1, S, False, 1, 1, 1, rbf_dim=rbf), seed=S)
+                sd = {k[len("dynamics."):]: v for k, v in sd.items()}
+                blob, offs = pack.pack_gvp_tc(sd, n_convs=1, update_kp=False, n_message_gvps=1, n_update_gvps=1,
+                                              n_noise_gvps=1, device="cpu", split=True)
+                assert len(offs) == 3 * 4 and all(o % 128 == 0 for o in offs), (S, V, rbf)
+                # GVP order: message ll, message kl, update lig, head; to_feats_out [fout, hd + fin]
+                expect = [(S, V + 1 + S + rbf), (S, V + 1 + S + rbf), (S, V + S), (64, V + S)]
+                for g, (fout, K) in enumerate(expect):
+                    assert offs[3 * g + 1] - offs[3 * g] == _slab_bytes(fout, K), (S, V, rbf, g)
