@@ -385,6 +385,24 @@ int kpd_sampler_set_start(kpd_sampler* s, int32_t start_step, const float* x_sta
  * so a captured sampler serves any schedule without capturing again; the buffers must stay valid while runs use
  * them. */
 int kpd_sampler_set_schedule(kpd_sampler* s, int32_t n_rows, const float* coef, const float* coef2);
+/* Turns a freshly created sampler (not yet run) into a recording one (trajectories, DESIGN.md section 6.4): every
+ * captured step gets one more launch, record_frame_kernel, after its first denoiser pass; launches_per_step counts it.
+ * Allocates a few bytes of device memory (synchronous).  A sampler that never calls this captures what it did before. */
+int kpd_sampler_enable_recording(kpd_sampler* s);
+/* The frames of the next runs of a recording sampler.  A run of n_steps executed steps i = 0 .. n_steps-1 with stride
+ * every >= 1 writes m = ceil(n_steps / every) frames, frame j = the state just before step i = j * every (after its
+ * prologue), and copies the run's outputs into frame m:
+ *   x_frames [m+1, n_lig, 3], h_frames [m+1, n_lig, atom_nf]: positions (x - kp mean) + initial kp mean, features
+ *     h * lig_feat_norm_constant -- the frame and feature space the outputs are returned in;
+ *   x_pred [m, n_lig, 3], h_pred [m, n_lig, atom_nf]: the clean-ligand estimate (z - sigma_t eps) / alpha_t of frame j
+ *     from that step's first denoiser pass, in the same frame (unused, may be NULL, when n_frames == 1);
+ *   pred_coef [n_pred_rows, 2] device: (alpha_t, sigma_t) of the level each row of the active schedule starts from
+ *     (schedule.prediction_rows over its grid).
+ * kpd_sampler_run checks n_frames == ceil(n_steps / every) + 1 and n_pred_rows == the active schedule's rows.
+ * x_frames = NULL records nothing.  Only pointers are kept and each run uploads them, so a captured sampler follows new
+ * buffers and strides without capturing again. */
+int kpd_sampler_set_recording(kpd_sampler* s, int32_t every, int32_t n_frames, float* x_frames, float* h_frames,
+                              float* x_pred, float* h_pred, int32_t n_pred_rows, const float* pred_coef);
 
 /* Output decode, the step right behind the path (reference test.py:199-203: torch.argmax(lig_feat, dim=1) on the
  * host, then dataset.lig_atom_idx_to_element): atom_type[i] = argmax_c h_lig[i, c], lowest index on ties. */

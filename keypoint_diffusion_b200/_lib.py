@@ -107,6 +107,8 @@ def _load():
         "kpd_sampler_set_fragment": (I, [P, P, P, P]),
         "kpd_sampler_set_start": (I, [P, I, P, P, F, F]),
         "kpd_sampler_set_schedule": (I, [P, I, P, P]),
+        "kpd_sampler_enable_recording": (I, [P]),
+        "kpd_sampler_set_recording": (I, [P, I, I, P, P, P, P, I, P]),
         "kpd_partial_noise": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, F, F, F, P, U64, P]),
         "kpd_decode_atom_types": (I, [P, I, I, P, P]),
     }

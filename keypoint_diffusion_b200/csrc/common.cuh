@@ -307,6 +307,18 @@ int launch_renoise(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, 
 int launch_partial_noise(const kpd_batch* b, const float* x_start, const float* h_start, float* x_lig, float* h_lig,
                          float* x_kp, int F, float alpha, float sigma, float norm_c, const float* noise, uint64_t seed,
                          const RunParams* rp, cudaStream_t st);
+// ------------------------------------------------------------------ trajectory recording (trajectory.cu)
+struct RecordParams {     // a recording sampler keeps it in device memory, so that a captured graph can be re-pointed
+    int every;            // frame stride k >= 1: executed step i is recorded when i % k == 0, as frame i / k
+    float* x_frames;      // NULL (record nothing) or [m+1][n_lig][3] state frames, output frame of reference
+    float* h_frames;      // [m+1][n_lig][F]
+    float* x_pred;        // [m][n_lig][3] clean-ligand estimates (x - sigma_t eps_x) / alpha_t, same frame
+    float* h_pred;        // [m][n_lig][F]
+    const float* pred_coef;   // [rows][2] (alpha_t, sigma_t) of the state each row starts from
+};
+int launch_record_frame(const kpd_batch* b, const float* x_lig, const float* h_lig, const float* x_kp,
+                        const float* eps_x, const float* eps_h, int F, const int* step_ptr, const RunParams* rp,
+                        const RecordParams* rec, const float* init_kp_com, float norm_c, cudaStream_t st);
 long long launch_count();  // kernels launched through check_launch() so far (this process)
 
 // optional per-kernel CUDA-event timing (bench.py's roofline leg); no-ops unless enabled and

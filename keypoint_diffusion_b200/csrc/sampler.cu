@@ -14,6 +14,9 @@
 // step counter at t0 instead of T; the captured graphs do not depend on the step, so they serve any t0.
 // Fewer-step sampling (kpd_sampler_set_schedule) swaps the coefficient rows: the step kernels read the sampler's own
 // [T,4] table, which every run fills from the active schedule, so one capture serves every schedule, eta and start.
+// A recording sampler (kpd_sampler_enable_recording) adds record_frame_kernel after the step's first denoiser pass:
+//     step_prologue -> graph_mark/scan/fill -> denoiser -> record_frame -> ddpm_step
+// and the kernel picks its frame slot from the device step counter, so the same graphs serve any stride or buffers.
 #include "common.cuh"
 #include <string.h>
 
@@ -54,6 +57,10 @@ struct kpd_sampler {
     const float *x_start, *h_start;
     int start_step;
     float start_alpha, start_sigma;
+    // trajectory recording (kpd_sampler_enable_recording): rec_dev == NULL = no record_frame launch in the step
+    RecordParams rec;         // host copy; x_frames == NULL records nothing.  Every run uploads it
+    RecordParams* rec_dev;
+    int rec_frames, rec_rows;
 };
 
 static int64_t model_ws_bytes(const kpd_sampler_config* cfg, const void* model, const kpd_batch* b, int cap_ll,
@@ -133,9 +140,17 @@ static int enqueue_denoiser(kpd_sampler* s, cudaStream_t st) {
                            s->has_lk ? &s->kk : nullptr, s->eps_h, s->eps_x, s->model_ws, st);
 }
 
+// the frame of a recording sampler: the state after the prologue and the first denoiser pass's eps
+static int enqueue_record(kpd_sampler* s, cudaStream_t st) {
+    if (!s->rec_dev) return 0;
+    return launch_record_frame(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->step,
+                               s->rp, s->rec_dev, s->init_kp_com, s->cfg.lig_feat_norm_constant, st);
+}
+
 static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
     KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef_run, st));
     KPD_TRY(enqueue_denoiser(s, st));
+    KPD_TRY(enqueue_record(s, st));
     KPD_TRY(launch_ddpm_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->coef_run,
                              s->step, nullptr, nullptr, 0, s->rp, st));
     return 0;
@@ -147,6 +162,7 @@ static int enqueue_inpaint_step(kpd_sampler* s, cudaStream_t st) {
     KPD_TRY(launch_step_prologue(s->counter, s->step, s->t_cur, s->coef_run, st));
     for (int u = 0; u < r; ++u) {
         KPD_TRY(enqueue_denoiser(s, st));
+        if (u == 0) KPD_TRY(enqueue_record(s, st));
         KPD_TRY(launch_ddpm_inpaint_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, F, s->coef_run,
                                          s->step, u, r, InpaintParams{}, s->frag_dev, s->init_kp_com,
                                          s->cfg.lig_feat_norm_constant, nullptr, 0, s->rp, st));
@@ -185,6 +201,7 @@ extern "C" void kpd_sampler_destroy(kpd_sampler* s) {
     if (!s) return;
     if (s->exec) cudaGraphExecDestroy(s->exec);
     if (s->frag_dev) cudaFree(s->frag_dev);
+    if (s->rec_dev) cudaFree(s->rec_dev);
     if (s->graph) cudaGraphDestroy(s->graph);
     if (s->ev_in) cudaEventDestroy(s->ev_in);
     if (s->ev_out) cudaEventDestroy(s->ev_out);
@@ -261,6 +278,33 @@ extern "C" int kpd_sampler_set_schedule(kpd_sampler* s, int32_t n_rows, const fl
     return 0;
 }
 
+extern "C" int kpd_sampler_enable_recording(kpd_sampler* s) {
+    KPD_REQUIRE(s, "kpd_sampler_enable_recording: null sampler");
+    KPD_REQUIRE(!s->exec && !s->rec_dev, "kpd_sampler_enable_recording: the sampler has already run or is recording");
+    const cudaError_t e = cudaMalloc(&s->rec_dev, sizeof(RecordParams));
+    KPD_REQUIRE(e == cudaSuccess, "kpd_sampler_enable_recording: %s", cudaGetErrorString(e));
+    s->rec = RecordParams{1, nullptr, nullptr, nullptr, nullptr, nullptr};
+    return 0;
+}
+
+extern "C" int kpd_sampler_set_recording(kpd_sampler* s, int32_t every, int32_t n_frames, float* x_frames,
+                                         float* h_frames, float* x_pred, float* h_pred, int32_t n_pred_rows,
+                                         const float* pred_coef) {
+    KPD_REQUIRE(s && s->rec_dev, "kpd_sampler_set_recording: not a recording sampler");
+    if (!x_frames) {
+        s->rec = RecordParams{1, nullptr, nullptr, nullptr, nullptr, nullptr};
+        s->rec_frames = s->rec_rows = 0;
+        return 0;
+    }
+    KPD_REQUIRE(every >= 1 && n_frames >= 1 && h_frames && pred_coef && n_pred_rows >= 1,
+                "kpd_sampler_set_recording: bad argument");
+    KPD_REQUIRE(n_frames == 1 || (x_pred && h_pred), "kpd_sampler_set_recording: prediction frames need buffers");
+    s->rec = RecordParams{every, x_frames, h_frames, x_pred, h_pred, pred_coef};
+    s->rec_frames = n_frames;
+    s->rec_rows = n_pred_rows;
+    return 0;
+}
+
 static int enqueue_any_step(kpd_sampler* s, cudaStream_t st) {
     return s->resamplings ? enqueue_inpaint_step(s, st) : enqueue_step(s, st);
 }
@@ -293,6 +337,12 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     KPD_REQUIRE(t0 <= rows, "kpd_sampler_run: start step %d beyond the %d rows of the schedule", t0, rows);
     KPD_REQUIRE(!s->resamplings || !s->sched_coef || s->sched_coef2, "kpd_sampler_run: the schedule has no coef2");
     KPD_REQUIRE(n_steps >= 0 && n_steps <= t0, "kpd_sampler_run: n_steps out of range");
+    // what keeps record_frame_kernel inside its buffers: frame j <= (n_steps-1) / every, prediction row s < rows
+    KPD_REQUIRE(!s->rec.x_frames || s->rec_frames == (n_steps + s->rec.every - 1) / s->rec.every + 1,
+                "kpd_sampler_run: %d frames recorded every %d steps need %d buffers, got %d", n_steps, s->rec.every,
+                (n_steps + s->rec.every - 1) / s->rec.every + 1, s->rec_frames);
+    KPD_REQUIRE(!s->rec.x_frames || s->rec_rows == rows,
+                "kpd_sampler_run: %d prediction rows for a schedule of %d rows", s->rec_rows, rows);
     const kpd_batch& b = s->batch;
     const int F = s->cfg.atom_nf;
     cudaStream_t user = static_cast<cudaStream_t>(stream), st = s->stream;
@@ -317,6 +367,7 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
         if (s->sched_coef) frag.coef2 = s->sched_coef2;
         CU(cudaMemcpyAsync(s->frag_dev, &frag, sizeof(InpaintParams), cudaMemcpyHostToDevice, st));
     }
+    if (s->rec_dev) CU(cudaMemcpyAsync(s->rec_dev, &s->rec, sizeof(RecordParams), cudaMemcpyHostToDevice, st));
 
     // frame setup (ligand_diffuser.py:348-370)
     KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 1, 0, s->init_kp_com, st));                // init_kp_com (:348)
@@ -356,6 +407,12 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
     CU(cudaMemcpyAsync(x_lig, s->x_lig, sizeof(float) * 3 * b.n_lig, cudaMemcpyDeviceToDevice, st));
     CU(cudaMemcpyAsync(h_lig, s->h_lig, sizeof(float) * (size_t)F * b.n_lig, cudaMemcpyDeviceToDevice, st));
     CU(cudaMemcpyAsync(x_kp, s->x_kp, sizeof(float) * 3 * b.n_kp, cudaMemcpyDeviceToDevice, st));
+    if (s->rec.x_frames) {  // the last state frame is the output
+        const size_t last = (size_t)(s->rec_frames - 1) * b.n_lig;
+        CU(cudaMemcpyAsync(s->rec.x_frames + last * 3, s->x_lig, sizeof(float) * 3 * b.n_lig, cudaMemcpyDeviceToDevice, st));
+        CU(cudaMemcpyAsync(s->rec.h_frames + last * F, s->h_lig, sizeof(float) * (size_t)F * b.n_lig,
+                           cudaMemcpyDeviceToDevice, st));
+    }
     CU(cudaEventRecord(s->ev_out, st));
     CU(cudaStreamWaitEvent(user, s->ev_out, 0));
 #undef CU

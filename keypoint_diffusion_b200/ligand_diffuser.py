@@ -19,8 +19,9 @@ from . import hetero, ops
 from .dynamics import LigRecDynamics, LigRecDynamicsGVP
 from .n_nodes_dist import LigandSizeDistribution
 from .receptor_encoder import ReceptorEncoder, ReceptorEncoderGVP
-from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_rows, coefficient_table, inpaint_rows, inpaint_table,
-                       sigma, sigma_and_alpha_t_given_s, start_coefficients, step_grid)
+from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_rows, coefficient_table, frame_levels, inpaint_rows,
+                       inpaint_table, prediction_rows, prediction_table, sigma, sigma_and_alpha_t_given_s,
+                       start_coefficients, step_grid)
 from .utils import get_batch_idxs, split_bounds
 
 DEFAULT_SUB_BATCHES = {"gvp": 4, "egnn": 2}      # measured on B200: profiles/r01_sweep_sub_batches_*.txt
@@ -82,6 +83,7 @@ class KeypointDiffusion(nn.Module):
         object.__setattr__(self, "_samplers", {})
         object.__setattr__(self, "_coef", {})
         object.__setattr__(self, "_coef2", {})
+        object.__setattr__(self, "_pred", {})
         object.__setattr__(self, "_schedules", {})
         object.__setattr__(self, "last_launches_per_step", 0)
         object.__setattr__(self, "_streams", {})
@@ -144,19 +146,29 @@ class KeypointDiffusion(nn.Module):
             self._coef2[key] = inpaint_table(self.gamma.gamma, self.n_timesteps).to(device)
         return self._coef2[key]
 
+    def prediction_coef_table(self, device) -> torch.Tensor:
+        """schedule.prediction_table on `device`, cached like coef_table."""
+        key = (str(device), self.gamma.gamma._version, self.gamma.gamma.data_ptr())
+        if key not in self._pred:
+            self._pred.clear()
+            self._pred[key] = prediction_table(self.gamma.gamma, self.n_timesteps).to(device)
+        return self._pred[key]
+
     MAX_CACHED_SCHEDULES = 8
 
     def schedule_tables(self, device, t_start: int, n: int, eta: Optional[float] = None, inpaint: bool = False):
-        """(coef [n,4], coef2 [n,4] or None) on `device`: the rows of the n-step grid over [0, t_start]
-        (schedule.step_grid), ancestral (eta=None) or DDIM(eta) (schedule.coefficient_rows), and with inpaint=True the
-        fragment rows over the same grid (schedule.inpaint_rows).  n scalar rows cost milliseconds on the host; the
-        last few schedules are cached (per device and gamma version), least recently used evicted first."""
+        """(coef [n,4], coef2 [n,4] or None, pred [n,2]) on `device`: the rows of the n-step grid over [0, t_start]
+        (schedule.step_grid), ancestral (eta=None) or DDIM(eta) (schedule.coefficient_rows), with inpaint=True the
+        fragment rows over the same grid (schedule.inpaint_rows), and the (alpha_t, sigma_t) rows a recorded trajectory
+        reads (schedule.prediction_rows).  n scalar rows cost milliseconds on the host; the last few schedules are
+        cached (per device and gamma version), least recently used evicted first."""
         key = (str(device), self.gamma.gamma._version, self.gamma.gamma.data_ptr(), int(t_start), int(n),
                None if eta is None else float(eta), bool(inpaint))
         hit = self._schedules.pop(key, None)
         if hit is None:
             grid, T, g = step_grid(t_start, n), self.n_timesteps, self.gamma.gamma
-            hit = (coefficient_rows(g, T, grid, eta).to(device), inpaint_rows(g, T, grid).to(device) if inpaint else None)
+            hit = (coefficient_rows(g, T, grid, eta).to(device), inpaint_rows(g, T, grid).to(device) if inpaint else None,
+                   prediction_rows(g, T, grid).to(device))
             while len(self._schedules) >= self.MAX_CACHED_SCHEDULES:
                 self._schedules.pop(next(iter(self._schedules)))
         self._schedules[key] = hit
@@ -265,16 +277,19 @@ class KeypointDiffusion(nn.Module):
         return max(1, min(DEFAULT_SUB_BATCHES[self.architecture], n_complexes // 16))
 
     def _capacity_sampler(self, instance: int, plan: "ops.CapacityPlan", device, steps_per_graph, use_cuda_graph,
-                          resamplings: int = 0):
+                          resamplings: int = 0, record: bool = False):
         """The captured loop of capacity bucket plan.key (created on first use, then shared by every batch that lands in
         the bucket -- whatever its per-complex sizes, pockets or kk graph).  Groups of one call that run concurrently
         and share a bucket take distinct instances 0, 1, ... of it.  resamplings >= 1: the inpainting loop with that
-        many passes per step (cached apart from the plain loop: its captured sequence differs)."""
+        many passes per step; record=True: the recording loop (visualize=True).  Both are cached apart from the plain
+        loop: their captured sequences differ."""
         model = self.dynamics.device_model(device)
         key = ("cap", instance, plan.key, self.dynamics._st.model_key, steps_per_graph, use_cuda_graph,
                getattr(model, "precision", "fp32"), self.n_timesteps)
         if resamplings:
             key = key + ("inpaint", int(resamplings))
+        if record:
+            key = key + ("record",)
         hit = self._cache_get(key)
         if hit is None:
             kp_width = self.n_kp_feat
@@ -283,7 +298,8 @@ class KeypointDiffusion(nn.Module):
                                       self.n_lig_features, kp_width, v_width, steps_per_graph=steps_per_graph,
                                       use_cuda_graph=use_cuda_graph,
                                       lig_feat_norm_constant=float(self.lig_feat_norm_constant), resamplings=resamplings,
-                                      inpaint_coef=self.inpaint_coef_table(device) if resamplings else None)
+                                      inpaint_coef=self.inpaint_coef_table(device) if resamplings else None,
+                                      record=record)
             self._samplers[key] = hit
             object.__setattr__(self, "cold_captures", self.cold_captures + 1)
         return hit
@@ -296,7 +312,8 @@ class KeypointDiffusion(nn.Module):
                                       fixed_pos: torch.Tensor = None, fixed_feat: torch.Tensor = None,
                                       resamplings: int = 1, start_pos: torch.Tensor = None,
                                       start_feat: torch.Tensor = None, start_step: Optional[int] = None,
-                                      timesteps: Optional[int] = None, eta: Optional[float] = None):
+                                      timesteps: Optional[int] = None, eta: Optional[float] = None,
+                                      frame_every: Optional[int] = None):
         """Returns (lig_pos, lig_feat): one CPU tensor per complex, as the reference does (:342-469).  ``g`` may live
         on the CPU (pinned or not): its keypoint tensors are uploaded here, straight into the sampler's buffers -- the
         host->device boundary of the path (reference test.py:152-161).
@@ -327,7 +344,16 @@ class KeypointDiffusion(nn.Module):
         of the cost; ``eta`` in [0, 1] makes them DDIM(eta) steps instead of ancestral ones (eta = 0: deterministic
         steps, though a fragment's known part is still noised at every step).  timesteps = t_start with eta=None is the
         default run bit for bit; eta alone keeps every step.  Composes with fragments, start ligands and sub-batches,
-        captures nothing new; capacity path only, and not with start_step = 0."""
+        captures nothing new; capacity path only, and not with start_step = 0.
+
+        Trajectories (DESIGN.md section 6.4): ``visualize=True`` records the run inside the captured loop, every
+        ``frame_every``-th executed step (None: every step, as the reference records), and returns one more element,
+        last: one dict per complex with m = ceil(n / frame_every) for the n steps run,
+        ``'t'`` long [m+1] (diffusion level of each frame; 0 for the last), ``'positions'`` [m+1, n_atoms, 3] and
+        ``'features'`` [m+1, n_atoms, F] (frame j < m: the state before executed step j*frame_every; frame m: the
+        returned ligand), ``'pred_positions'`` [m, n_atoms, 3] and ``'pred_features'`` [m, n_atoms, F] (the denoiser's
+        clean-ligand estimate (z - sigma_t eps) / alpha_t at frame j).  Every frame is in the frame and feature space the
+        ligands are returned in.  Recording does not change the ligands; capacity path only."""
         n_lig_total = int(g.num_nodes('lig'))
         inpaint = self._check_fragment_args(n_lig_total, fixed_mask, fixed_pos, fixed_feat, resamplings)
         start = self._check_start_args(n_lig_total, start_pos, start_feat, start_step)
@@ -339,9 +365,7 @@ class KeypointDiffusion(nn.Module):
             raise ValueError("init_lig_pos is not used with a start ligand (the start ligands' means set the frame)")
         t_start = int(start_step) if start else self.n_timesteps
         n_sched = self._check_schedule_args(timesteps, eta, t_start, capacity)
-        if visualize:
-            raise NotImplementedError("visualize=True (a per-step CPU copy of the whole graph) is a debug feature "
-                                      "outside the throughput path")
+        every = self._check_visualize_args(visualize, frame_every, capacity)
         dev = torch.device("cuda", torch.cuda.current_device()) if g.device.type != "cuda" else g.device
         batch_size = g.batch_size
         if start:
@@ -358,6 +382,12 @@ class KeypointDiffusion(nn.Module):
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())      # follows torch.manual_seed like the reference
         sched = None if n_sched is None else self.schedule_tables(dev, t_start, n_sched, eta, inpaint)
+        pred = None
+        if visualize:
+            pred = self.prediction_coef_table(dev) if sched is None else sched[2]
+            n_run = t_start if n_sched is None else n_sched
+            levels = frame_levels(list(range(self.n_timesteps + 1)) if n_sched is None else step_grid(t_start, n_sched),
+                                  n_run, every)
         n_sub = self.default_sub_batches(batch_size) if sub_batches is None else max(1, min(int(sub_batches), batch_size))
         if noise is not None:
             n_sub = 1          # injected noise (parity runs) is laid out for the undivided batch
@@ -393,7 +423,7 @@ class KeypointDiffusion(nn.Module):
             inst = taken.get(plan.key, 0)
             taken[plan.key] = inst + 1
             smp = self._capacity_sampler(inst, plan, dev, steps_per_graph, use_cuda_graph,
-                                         resamplings=int(resamplings) if inpaint else 0)
+                                         resamplings=int(resamplings) if inpaint else 0, record=visualize)
             frag = None
             if inpaint:
                 l1 = lig_ptr[b]
@@ -410,10 +440,12 @@ class KeypointDiffusion(nn.Module):
             with torch.cuda.stream(st):
                 out = smp.run(plan, kp['x_0'][k0:k1], kp['h_0'][k0:k1], kv[k0:k1] if kv is not None else None, gs, gd,
                               init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag,
-                              start=st_rows, schedule=sched)
+                              start=st_rows, schedule=None if sched is None else sched[:2],
+                              record_every=every if visualize else None, pred_coef=pred)
             if n_sub > 1:
                 for t in out:
-                    t.record_stream(cur)
+                    for v in (t.values() if isinstance(t, dict) else (t,)):
+                        v.record_stream(cur)
                 used.append(st)
             parts.append(out)
             launches += smp.sampler.launches_per_step
@@ -425,11 +457,21 @@ class KeypointDiffusion(nn.Module):
         object.__setattr__(self, "last_launches_per_step", launches)
         if g.device.type == "cuda":
             g.nodes['lig'].data['x_0'], g.nodes['lig'].data['h_0'], g.nodes['kp'].data['x_0'] = x_lig, h_lig, x_kp
+        frames = []
+        if visualize:       # sub-batches hold consecutive complexes: their frames join along the atom axis
+            fr = {k: torch.cat([p[-1][k] for p in parts], dim=1) for k in parts[0][-1]}
+            fr = {k: v if return_device_tensors else v.cpu() for k, v in fr.items()}
+            t = levels.to(dev) if return_device_tensors else levels
+            split = {k: torch.split(v, lig_n, dim=1) for k, v in fr.items()}
+            frames = [dict(t=t, **{k: split[k][i] for k in split}) for i in range(batch_size)]
         if return_device_tensors:
-            return (x_lig, h_lig, atom_type) if decode else (x_lig, h_lig)
+            res = (x_lig, h_lig, atom_type) if decode else (x_lig, h_lig)
+            return res + (frames,) if visualize else res
         pos_cpu, feat_cpu = x_lig.cpu(), h_lig.cpu()                # device -> host boundary (reference :464)
         res = (list(torch.split(pos_cpu, lig_n)), list(torch.split(feat_cpu, lig_n)))
-        return res + (list(torch.split(atom_type.cpu(), lig_n)),) if decode else res
+        if decode:
+            res = res + (list(torch.split(atom_type.cpu(), lig_n)),)
+        return res + (frames,) if visualize else res
 
     def _check_schedule_args(self, timesteps, eta, t_start: int, capacity) -> Optional[int]:
         """ValueError for a bad fewer-step request (host-side checks, before any device work); the step count of the
@@ -449,6 +491,18 @@ class KeypointDiffusion(nn.Module):
         if (timesteps is None and eta is None) or t_start == 0:
             return None
         return t_start if timesteps is None else int(timesteps)
+
+    @staticmethod
+    def _check_visualize_args(visualize, frame_every, capacity) -> int:
+        """ValueError for a bad trajectory request (host-side checks, before any device work); the frame stride."""
+        if frame_every is not None:
+            if not visualize:
+                raise ValueError("frame_every needs visualize=True")
+            if isinstance(frame_every, bool) or not isinstance(frame_every, numbers.Integral) or frame_every < 1:
+                raise ValueError(f"frame_every must be an integer >= 1, got {frame_every!r}")
+        if visualize and not capacity:
+            raise ValueError("visualize=True runs on the capacity path only (capacity=True)")
+        return 1 if frame_every is None else int(frame_every)
 
     def _check_fragment_args(self, n_lig: int, fixed_mask, fixed_pos, fixed_feat, resamplings) -> bool:
         """ValueError for an inconsistent fragment request (host-side checks, before any device work); True when the
@@ -642,6 +696,8 @@ class KeypointDiffusion(nn.Module):
         is the start ligand's first atoms and stays pinned.
         timesteps / eta (passed on to sample_from_encoded_receptors, like every other keyword): fewer-step sampling,
         checked here before any receptor is encoded.
+        visualize / frame_every: trajectories (see sample_from_encoded_receptors); every receptor's dict then also
+        holds ``'frames'``, one trajectory dict per ligand.  Not with ``complexes`` (sample_sharded).
 
         The diffusion batches are assembled on the device (hetero.expand_complexes): no per-complex graph copies."""
         has_fragment = self._check_fragments(fragments, n_lig_atoms, resamplings)
@@ -649,6 +705,9 @@ class KeypointDiffusion(nn.Module):
                                               sampler_kw)
         self._check_schedule_args(sampler_kw.get("timesteps"), sampler_kw.get("eta"),
                                   int(start_step) if has_start else self.n_timesteps, sampler_kw.get("capacity", True))
+        self._check_visualize_args(visualize, sampler_kw.get("frame_every"), sampler_kw.get("capacity", True))
+        if visualize and complexes is not None:
+            raise ValueError("visualize=True is not supported by sample_sharded")
         n_receptors = len(ref_graphs)
         enc, rec_mean = self._encode_all(ref_graphs, rec_enc_batch_size, encoded)
         dev = enc.device
@@ -664,7 +723,7 @@ class KeypointDiffusion(nn.Module):
             centers = rec_mean
         pocket_t = torch.tensor(pocket_of, dtype=torch.long, device=dev)
         size_t = torch.tensor(sizes, dtype=torch.long, device=dev)
-        lig_pos, lig_feat = [], []
+        lig_pos, lig_feat, frames = [], [], []
         for b in range(ceil(len(todo) / diff_batch_size)):
             chunk = todo[b * diff_batch_size:(b + 1) * diff_batch_size]
             idx = torch.tensor(chunk, dtype=torch.long, device=dev)
@@ -680,8 +739,12 @@ class KeypointDiffusion(nn.Module):
                                start_feat=torch.cat([start_ligands[r][1].detach().float().cpu() for r in owners]))
             else:
                 frag_kw.update(init_lig_pos=centers[pocket_t[idx]])
-            p, f = self.sample_from_encoded_receptors(bg, visualize=visualize,
-                                                      noise=None if noise is None else noise[b], **frag_kw, **sampler_kw)
+            res = self.sample_from_encoded_receptors(bg, visualize=visualize,
+                                                     noise=None if noise is None else noise[b], **frag_kw, **sampler_kw)
+            if visualize:
+                *res, fr = res
+                frames.extend(fr)
+            p, f = res
             lig_pos.extend(p)
             lig_feat.extend(f)
         if complexes is not None:
@@ -690,6 +753,8 @@ class KeypointDiffusion(nn.Module):
         for rec_idx in range(n_receptors):
             start, end = end, end + len(n_lig_atoms[rec_idx])
             samples.append({'positions': lig_pos[start:end], 'features': lig_feat[start:end]})
+            if visualize:
+                samples[-1]['frames'] = frames[start:end]
         return samples
 
     def _fragment_rows(self, fragments, receptors: List[int], sizes: List[int], resamplings: int) -> Dict:
@@ -721,7 +786,10 @@ class KeypointDiffusion(nn.Module):
         captured loops and no per-step communication, and ONE final all_gather (NCCL over NVLink; gloo in the CPU
         tests) brings coordinates + atom features back, so every rank returns the complete, receptor-major result of
         ``_sample``.  The reference's equivalent is a slurm array of independent single-GPU processes
-        (gen_test_commands.py:36-40, test.py:143-184).  Noise follows this rank's torch generator / ``seed``."""
+        (gen_test_commands.py:36-40, test.py:143-184).  Noise follows this rank's torch generator / ``seed``.
+        visualize=True is not supported (ValueError): trajectories are not gathered across ranks."""
+        if kw.get("visualize"):
+            raise ValueError("visualize=True is not supported by sample_sharded")
         import torch.distributed as dist
         from . import dist as kdist
         world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -755,12 +823,16 @@ class KeypointDiffusion(nn.Module):
                             start_step: Optional[int] = None, **kw):
         """fragment: optional ``(pos [m,3], feat [m,F])``: every ligand starts with these m atoms (see _sample).
         start_ligand / start_step: optional ``(pos [m,3], feat [m,F])`` and t0: every ligand (each of size m) is a
-        variant of that ligand, noised to level t0 and denoised from there (see _sample)."""
+        variant of that ligand, noised to level t0 and denoised from there (see _sample).
+        visualize=True: returns (positions, features, frames), one trajectory dict per ligand (see
+        sample_from_encoded_receptors)."""
         samples = self._sample([rec_graph], n_lig_atoms=[n_lig_atoms.tolist()], rec_enc_batch_size=rec_enc_batch_size,
                                diff_batch_size=diff_batch_size, visualize=visualize,
                                fragments=None if fragment is None else [fragment],
                                start_ligands=None if start_ligand is None else [start_ligand], start_step=start_step,
                                **kw)
+        if visualize:
+            return samples[0]['positions'], samples[0]['features'], samples[0]['frames']
         return samples[0]['positions'], samples[0]['features']
 
     @torch.no_grad()

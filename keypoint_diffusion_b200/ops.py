@@ -469,12 +469,13 @@ class Sampler:
     (inpainting) sampler: every reverse step runs `resamplings` denoiser passes with the atoms given to set_fragment
     pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop.
     Either kind runs from a given ligand after set_start (ligand optimisation by partial noising), and with fewer,
-    strided or DDIM steps after set_schedule; neither captures again."""
+    strided or DDIM steps after set_schedule; neither captures again.  record=True makes it a recording sampler: its
+    captured step holds one more launch, and run(record_every=k) returns the trajectory (DESIGN.md section 6.4)."""
 
     def __init__(self, model: _Model, batch: DeviceBatch, gp: GraphParams, kk: Optional[Csr], coef: torch.Tensor,
                  T: int, atom_nf: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
                  lig_feat_norm_constant: float = 1.0, atom_offset: int = 0, caps: Optional[Tuple[int, int]] = None,
-                 resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None):
+                 resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None, record: bool = False):
         self.model, self.batch, self.gp, self.kk, self.coef = model, batch, gp, kk, coef
         _require_cuda(coef)
         self.T, self.atom_nf = int(T), int(atom_nf)
@@ -508,6 +509,9 @@ class Sampler:
             _require_cuda(inpaint_coef)
             check(lib.kpd_sampler_enable_inpainting(self.handle, self.resamplings, ptr(inpaint_coef)),
                   "kpd_sampler_enable_inpainting")
+        self.record = bool(record)
+        if self.record:
+            check(lib.kpd_sampler_enable_recording(self.handle), "kpd_sampler_enable_recording")
 
     def set_fragment(self, fixed_mask: Optional[torch.Tensor], x_fix: Optional[torch.Tensor],
                      h_fix: Optional[torch.Tensor]):
@@ -587,10 +591,17 @@ class Sampler:
             lib.kpd_sampler_destroy(self.handle)
             self.handle = C.c_void_p()
 
-    def run(self, x_kp, h_kp, v_kp, init_lig_pos, noise=None, seed=0, n_steps=None, decode=False):
+    def run(self, x_kp, h_kp, v_kp, init_lig_pos, noise=None, seed=0, n_steps=None, decode=False, record_every=None,
+            pred_coef=None):
         """Returns (x_lig [n_lig,3], h_lig [n_lig,F], x_kp) on the device, in the input frame; with decode=True also
         the atom type of every generated atom (int32 [n_lig] = argmax over the feature channels, the first step of
-        the reference's output handling, test.py:199-203), written by a kernel enqueued behind the loop."""
+        the reference's output handling, test.py:199-203), written by a kernel enqueued behind the loop.
+
+        record_every = k (recording samplers only) also returns, last, the trajectory of the n_steps executed steps as a
+        dict of device tensors with m = ceil(n_steps / k): 'positions' [m+1, n_lig, 3] and 'features' [m+1, n_lig, F]
+        (frame j < m: the state before executed step j*k; frame m: the outputs), 'pred_positions' [m, n_lig, 3] and
+        'pred_features' [m, n_lig, F] (the clean-ligand estimate of frame j), all in the frame and feature space of the
+        outputs.  pred_coef: fp32 [rows, 2] on the device, schedule.prediction_rows over the active schedule's grid."""
         _require_cuda(x_kp, h_kp, init_lig_pos)
         b = self.batch
         x_kp = _f32(x_kp).clone()
@@ -602,12 +613,42 @@ class Sampler:
             assert noise.shape == (self.noise_slots, b.n_lig * (3 + self.atom_nf)) and noise.dtype == torch.float32
         h_kp, init_lig_pos = _f32(h_kp), _f32(init_lig_pos)
         v_kp = _f32(v_kp) if v_kp is not None else None
+        frames = None
+        if self.record:
+            frames = self._set_recording(n_steps, record_every, pred_coef)
+        elif record_every is not None:
+            raise ValueError("record_every needs a recording sampler (record=True)")
         check(lib.kpd_sampler_run(self.handle, ptr(x_kp), ptr(h_kp), ptr(v_kp) if v_kp is not None else None,
                                   ptr(init_lig_pos), ptr(x_lig), ptr(h_lig), ptr(noise), int(seed), n_steps,
                                   _stream()), "kpd_sampler_run")
-        if decode:
-            return x_lig, h_lig, x_kp, decode_atom_types(h_lig)
-        return x_lig, h_lig, x_kp
+        out = (x_lig, h_lig, x_kp) + ((decode_atom_types(h_lig),) if decode else ())
+        return out + (frames,) if frames is not None else out
+
+    def _set_recording(self, n_steps: int, every, pred_coef) -> Optional[Dict[str, torch.Tensor]]:
+        """Frame buffers of one run (kpd_sampler_set_recording), or recording off when every is None."""
+        if every is None:
+            check(lib.kpd_sampler_set_recording(self.handle, 1, 0, None, None, None, None, 0, None),
+                  "kpd_sampler_set_recording")
+            return None
+        if isinstance(every, bool) or int(every) != every or every < 1:
+            raise ValueError(f"record_every must be an integer >= 1, got {every!r}")
+        if pred_coef is None:
+            raise ValueError("recording needs pred_coef (schedule.prediction_rows over the active schedule's grid)")
+        _require_cuda(pred_coef)
+        assert pred_coef.dtype == torch.float32 and pred_coef.is_contiguous() and pred_coef.shape[1:] == (2,)
+        every = int(every)
+        m = -(-n_steps // every)
+        b, F, dev = self.batch, self.atom_nf, self.batch.device
+        fr = {"positions": torch.empty(m + 1, b.n_lig, 3, device=dev),
+              "features": torch.empty(m + 1, b.n_lig, F, device=dev),
+              "pred_positions": torch.empty(m, b.n_lig, 3, device=dev),
+              "pred_features": torch.empty(m, b.n_lig, F, device=dev)}
+        check(lib.kpd_sampler_set_recording(self.handle, every, m + 1, ptr(fr["positions"]), ptr(fr["features"]),
+                                            ptr(fr["pred_positions"]) if m else None,
+                                            ptr(fr["pred_features"]) if m else None, int(pred_coef.shape[0]),
+                                            ptr(pred_coef)), "kpd_sampler_set_recording")
+        self._pred_coef = pred_coef         # read by every recorded step of the run, on the sampler's stream
+        return fr
 
     @property
     def launches_per_step(self):
@@ -709,11 +750,13 @@ class CapacitySampler:
     input buffers; run() rewrites their CONTENTS for the batch at hand and replays the same CUDA graphs.  With
     resamplings >= 1 (and inpaint_coef) it is an inpainting sampler that also owns zero-filled fragment buffers sized at
     capacity: run(fragment=...) fills the rows of the real atoms; filler complexes and atoms are never fixed.  Likewise
-    it owns start-ligand buffers at capacity for run(start=...); filler rows stay zero and filler outputs are dropped."""
+    it owns start-ligand buffers at capacity for run(start=...); filler rows stay zero and filler outputs are dropped.
+    record=True: a recording sampler (see Sampler); run(record_every=...) returns the frames of the real atoms."""
 
     def __init__(self, model: _Model, plan: CapacityPlan, gp: GraphParams, coef: torch.Tensor, T: int, atom_nf: int,
                  kp_width: int, v_width: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
-                 lig_feat_norm_constant: float = 1.0, resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None):
+                 lig_feat_norm_constant: float = 1.0, resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None,
+                 record: bool = False):
         B, N, K, max_lig, max_kp, cap_ll, cap_kl, cap_kk = plan.key
         dev = model.device
         self.key, self.model, self.atom_nf, self.T = plan.key, model, int(atom_nf), int(T)
@@ -726,7 +769,8 @@ class CapacitySampler:
         self.init_pos = torch.zeros(B, 3, dtype=torch.float32, device=dev)
         self.sampler = Sampler(model, self.batch, gp, self.kk, coef, T, atom_nf, steps_per_graph=steps_per_graph,
                                use_cuda_graph=use_cuda_graph, lig_feat_norm_constant=lig_feat_norm_constant,
-                               caps=(cap_ll, cap_kl), resamplings=resamplings, inpaint_coef=inpaint_coef)
+                               caps=(cap_ll, cap_kl), resamplings=resamplings, inpaint_coef=inpaint_coef,
+                               record=record)
         if self.sampler.resamplings:
             self.fixed_mask = torch.zeros(N, dtype=torch.uint8, device=dev)
             self.x_fix = torch.zeros(N, 3, dtype=torch.float32, device=dev)
@@ -738,7 +782,8 @@ class CapacitySampler:
 
     def run(self, plan: CapacityPlan, x_kp, h_kp, v_kp, kk_src, kk_dst, init_pos, seed: int, atom_offset: int = 0,
             noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None,
-            start: Optional[Tuple] = None, schedule: Optional[Tuple] = None):
+            start: Optional[Tuple] = None, schedule: Optional[Tuple] = None, record_every: Optional[int] = None,
+            pred_coef: Optional[torch.Tensor] = None):
         """x_kp/h_kp/v_kp: the REAL keypoint rows (host or device tensors; pinned host tensors are uploaded straight
         into the capacity buffers); kk_src/kk_dst: kk edges in this batch's own keypoint numbering; init_pos [B_real,3].
         fragment (inpainting samplers): (fixed_mask [N_real] bool, x_fix [N_real,3], h_fix [N_real,F]) or None.
@@ -746,8 +791,10 @@ class CapacitySampler:
         Sampler.set_start) -- or None for the plain start; injected noise then has the slots of a t0-step run.
         schedule: (coef [n,4], coef2 [n,4] or None) on the device -- run the n rows of that schedule (see
         Sampler.set_schedule; t0 of start then counts its rows) -- or None for the create-time tables.  A run-time
-        value like the start: no new capture.
-        -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]]) on the device."""
+        value like the start: no new capture.  record_every / pred_coef (recording samplers): see Sampler.run; pred_coef
+        has the rows of the schedule run.
+        -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]][, frames]) on the device,
+        frames holding the real atoms only ([m+1, N_real, .] and [m, N_real, .])."""
         if plan.key != self.key:
             raise ValueError("CapacitySampler.run: the plan belongs to another capacity bucket")
         if fragment is not None and not self.sampler.resamplings:
@@ -783,7 +830,12 @@ class CapacitySampler:
             pad[:, : N_r * 3] = noise[:, : N_r * 3]
             pad[:, N * 3: N * 3 + N_r * F] = noise[:, N_r * 3:]
             noise = pad
-        out = self.sampler.run(self.x_kp, self.h_kp, self.v_kp, self.init_pos, noise=noise, seed=seed, decode=decode)
+        out = self.sampler.run(self.x_kp, self.h_kp, self.v_kp, self.init_pos, noise=noise, seed=seed, decode=decode,
+                               record_every=record_every, pred_coef=pred_coef)
         self.runs += 1
         res = (out[0][:N_r], out[1][:N_r], out[2][:K_r])
-        return res + (out[3][:N_r],) if decode else res
+        if decode:
+            res = res + (out[3][:N_r],)
+        if record_every is not None:
+            res = res + ({k: v[:, :N_r] for k, v in out[-1].items()},)
+        return res

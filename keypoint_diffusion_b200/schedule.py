@@ -9,7 +9,7 @@ inpaint_table [T,4] = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) is the second tab
 fragment-conditioned sampling reads (DESIGN.md section 6.1); start_coefficients gives (alpha_t0, sigma_t0), the
 forward noising of a start ligand in ligand optimisation (section 6.2).  Both tables are the unit-step case of
 coefficient_rows / inpaint_rows over a step grid (step_grid), which also give the strided ancestral and DDIM rows of
-fewer-step sampling (section 6.3).
+fewer-step sampling (section 6.3).  prediction_rows and frame_levels serve recorded trajectories (section 6.4).
 """
 import numpy as np
 import torch
@@ -147,6 +147,32 @@ def inpaint_rows(gamma: torch.Tensor, T: int, grid) -> torch.Tensor:
 def inpaint_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
     """fp32 [T,4] on the CPU: inpaint_rows over the unit grid (row s: t = s+1)."""
     return inpaint_rows(gamma, T, list(range(T + 1)))
+
+
+def prediction_rows(gamma: torch.Tensor, T: int, grid) -> torch.Tensor:
+    """fp32 [n,2] on the CPU over a step grid; row k = (alpha_t, sigma_t) at t = tau_{k+1}, the level of the state row k
+    starts from: what a recorded trajectory's clean-ligand estimate (z - sigma_t eps) / alpha_t divides by (DESIGN.md
+    section 6.4).  Scalar fp32 ops like coefficient_rows, so row k equals start_coefficients(gamma, tau_{k+1}) bit for
+    bit.  The same for every eta."""
+    g = gamma.detach().float().cpu()
+    rows = []
+    for s_int, t_int in zip(grid[:-1], grid[1:]):
+        _, gt, _ = _row_gammas(g, T, s_int, t_int)
+        rows.append(torch.stack([alpha(gt)[0], sigma(gt)[0]]))
+    return torch.stack(rows).contiguous()
+
+
+def prediction_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
+    """fp32 [T,2] on the CPU: prediction_rows over the unit grid (row s: t = s+1)."""
+    return prediction_rows(gamma, T, list(range(T + 1)))
+
+
+def frame_levels(grid, n: int, every: int) -> torch.Tensor:
+    """long [ceil(n / every) + 1]: the diffusion level of every frame a run of n steps records with stride `every`, the
+    run starting from row n-1 of a table over `grid`: frame j < m is the state before executed step j*every, at level
+    tau_{n - j*every}; the last frame, the output, is at level 0."""
+    m = -(-int(n) // int(every))
+    return torch.tensor([grid[int(n) - j * int(every)] for j in range(m)] + [0], dtype=torch.long)
 
 
 def start_coefficients(gamma: torch.Tensor, t0: int):

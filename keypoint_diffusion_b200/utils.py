@@ -1,6 +1,7 @@
 """Batch helpers with the reference's names (reference utils.py:81-170), on the duck-typed
 graph surface of hetero.HeteroBatch (or a real DGL heterograph), and the output decode that follows the
-sampling path (SURVEY 8f rank 4: reference utils.py:11-21, test.py:199-209)."""
+sampling path (SURVEY 8f rank 4: reference utils.py:11-21, test.py:199-209), with a multi-frame XYZ writer for the
+trajectories of visualize=True."""
 from typing import Dict, List, Tuple
 
 import torch
@@ -73,6 +74,18 @@ def decode_ligands(lig_pos: List[torch.Tensor], lig_feat: List[torch.Tensor], li
         idx = torch.argmax(feat, dim=1).tolist()
         out.append((pos, [lig_elements[i] for i in idx]))
     return out
+
+
+def write_xyz_trajectory(frames: Dict[str, torch.Tensor], lig_elements: List[str], filename=None):
+    """A multi-frame XYZ file of one ligand's trajectory (a dict of sample_from_encoded_receptors(visualize=True)): one
+    write_xyz_file block per state frame, its atom types decoded from that frame's features as decode_ligands does.
+    Returns the text when ``filename`` is None, else writes it."""
+    pos, feat = frames['positions'].cpu(), frames['features'].cpu()
+    out = "".join(write_xyz_file(p, elems) for p, elems in decode_ligands(list(pos), list(feat), lig_elements))
+    if filename is None:
+        return out
+    with open(filename, 'w') as f:
+        f.write(out)
 
 
 def split_bounds(n_complexes: int, n_groups: int):
