@@ -246,6 +246,24 @@ int kpd_ddpm_step(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_k
                   const float* noise_x, const float* noise_h, uint64_t seed, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * (e) multistep: one DPM-Solver++(2M) reverse step (an extension beyond the reference, DESIGN.md
+ * section 6.5), what a multistep sampler's captured step runs.  Row s of coef is a DDIM eta = 0 row
+ * (schedule.coefficient_rows(..., eta=0)), row s of ms_coef [rows,4] = (c, alpha_t, sigma_t, 0)
+ * (schedule.multistep_rows over the same grid):
+ *   z'  = z/alpha_t|s - var_terms*eps + sigma*noise          (kpd_ddpm_step, draws included)
+ *   x^  = (z - sigma_t eps) / alpha_t                        positions and features
+ *   z_s = z' + c (x^ - hist)  unless s == first_row;  hist = x^
+ *   then the ligand COM is removed from ligand and keypoints, and from the positions of hist.
+ * first_row: the row a run executes first; that step does not read hist (it may hold anything).
+ * hist_x [n_lig,3] / hist_h [n_lig,atom_nf]: caller-owned history, updated in place.
+ * ------------------------------------------------------------------------------------------ */
+int kpd_ddpm_multistep_step(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_kp,
+                            const float* eps_x, const float* eps_h, int32_t atom_nf,
+                            const float* coef, const float* ms_coef, const int32_t* step_ptr,
+                            int32_t first_row, float* hist_x, float* hist_h,
+                            const float* noise_x, const float* noise_h, uint64_t seed, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * (e') Fragment-conditioned reverse step (inpainting with RePaint-style resampling; an extension
  * beyond the reference, DESIGN.md section 6.1).  Pass u of step s (t = s+1):
  *   z_unk = x/alpha_t|s - var_terms*eps + sigma*noise             (what kpd_ddpm_step computes)
@@ -403,6 +421,18 @@ int kpd_sampler_enable_recording(kpd_sampler* s);
  * buffers and strides without capturing again. */
 int kpd_sampler_set_recording(kpd_sampler* s, int32_t every, int32_t n_frames, float* x_frames, float* h_frames,
                               float* x_pred, float* h_pred, int32_t n_pred_rows, const float* pred_coef);
+
+/* Turns a freshly created sampler (not yet run, not inpainting) into a multistep one (DPM-Solver++(2M), DESIGN.md
+ * section 6.5): its captured step launches the multistep instantiation of the step kernel instead of the plain one, so
+ * launches_per_step does not change.  Allocates a few bytes of device memory (synchronous).  A sampler that never calls
+ * this captures what it did before. */
+int kpd_sampler_enable_multistep(kpd_sampler* s);
+/* The multistep rows and history of the next runs: ms_coef [n_rows,4] device rows (schedule.multistep_rows over the
+ * grid of the active schedule, whose coef rows must be DDIM eta = 0 rows), hist_x [n_lig,3] and hist_h [n_lig,atom_nf]
+ * caller-owned scratch (need no initialisation: the first executed row writes them before any read).
+ * kpd_sampler_run checks n_rows == the active schedule's rows.  Only pointers are kept and each run uploads them, so a
+ * captured sampler follows new rows and buffers without capturing again. */
+int kpd_sampler_set_multistep(kpd_sampler* s, int32_t n_rows, const float* ms_coef, float* hist_x, float* hist_h);
 
 /* Output decode, the step right behind the path (reference test.py:199-203: torch.argmax(lig_feat, dim=1) on the
  * host, then dataset.lig_atom_idx_to_element): atom_type[i] = argmax_c h_lig[i, c], lowest index on ties. */

@@ -91,6 +91,7 @@ def _load():
         "kpd_gvp_forward": (I, [P, C.POINTER(KpdBatch), P, P, P, P, P, P, I, C.POINTER(KpdCsr),
                                 C.POINTER(KpdCsr), C.POINTER(KpdCsr), C.POINTER(KpdCsr), P, P, P, P]),
         "kpd_ddpm_step": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, P, P, P, P, U64, P]),
+        "kpd_ddpm_multistep_step": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, P, P, P, I, P, P, P, P, U64, P]),
         "kpd_ddpm_inpaint_step": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, P, P, P, I, P, P, P, P, F, P, U64, P]),
         "kpd_renoise": (I, [C.POINTER(KpdBatch), P, P, P, I, P, P, I, P, U64, P]),
         "kpd_remove_com": (I, [C.POINTER(KpdBatch), P, P, I, P, P]),
@@ -109,6 +110,8 @@ def _load():
         "kpd_sampler_set_schedule": (I, [P, I, P, P]),
         "kpd_sampler_enable_recording": (I, [P]),
         "kpd_sampler_set_recording": (I, [P, I, I, P, P, P, P, I, P]),
+        "kpd_sampler_enable_multistep": (I, [P]),
+        "kpd_sampler_set_multistep": (I, [P, I, P, P, P]),
         "kpd_partial_noise": (I, [C.POINTER(KpdBatch), P, P, P, P, P, I, F, F, F, P, U64, P]),
         "kpd_decode_atom_types": (I, [P, I, I, P, P]),
     }

@@ -227,6 +227,12 @@ int launch_copy_rows(const float* in, int ldi, float* out, int ldo, int n, int w
 int launch_sub(const float* a, const float* b, float* out, int n, cudaStream_t st);
 
 // ------------------------------------------------------------------ step ops (ddpm_step.cu)
+struct MultistepParams {  // DPM-Solver++(2M) (DESIGN.md section 6.5); a multistep sampler keeps it in device memory,
+                          // so that a captured graph can be re-pointed, like RecordParams
+    const float* ms_coef; // [rows][4] = (c, alpha_t, sigma_t, 0) of the active schedule (schedule.multistep_rows)
+    float* hist_x;        // [n_lig][3] the previous executed row's clean-ligand estimate, frame of the next step
+    float* hist_h;        // [n_lig][F]
+};
 struct RunParams {        // lives in device memory so that a captured graph can be re-pointed
     const float* noise;   // NULL or slots of [n_lig][3+F] (x first), numbered by noise_slot()
     uint64_t seed;
@@ -276,9 +282,13 @@ __device__ __forceinline__ void remove_ligand_com(float* x_lig, float* x_kp, int
     sub3(x_kp, k0, nk, com);
 }
 
+// msp (device, a multistep sampler's) or msv (host copy, a stand-alone call) selects the DPM-Solver++(2M) step; first_row
+// is the row a stand-alone call treats as the run's first (no correction); a sampler's run takes RunParams.T - 1
 int launch_ddpm_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
                      const float* eps_h, int F, const float* coef, const int* step_ptr, const float* noise_x,
-                     const float* noise_h, uint64_t seed, const RunParams* rp, cudaStream_t st);
+                     const float* noise_h, uint64_t seed, const RunParams* rp, cudaStream_t st,
+                     const struct MultistepParams* msp = nullptr, const struct MultistepParams* msv = nullptr,
+                     int first_row = 0);
 int launch_com(const kpd_batch* b, float* x_lig, float* x_kp, int which, int shift, float* com_out, cudaStream_t st);
 int launch_shift(float* x, const int* node_batch, int n, const float* v, float sign, cudaStream_t st);
 int launch_randn_init(float* x_lig, float* h_lig, int n_lig, int F, uint64_t seed, const RunParams* rp, cudaStream_t st);

@@ -13,11 +13,19 @@
 
 namespace kpd {
 
+// MULTISTEP = true: DPM-Solver++(2M) (DESIGN.md section 6.5).  Row s is then a DDIM eta = 0 row, and the step adds
+//   x^ = (z - sigma_t eps) / alpha_t,  z_s += c (x^ - x^_prev)      (c, alpha_t, sigma_t) = row s of ms_coef
+// except on the first row the run executes (RunParams.T - 1, or first_row of a stand-alone call), which neither reads
+// the history nor corrects: 0 * an unwritten history could be NaN.
+// x^ replaces the history, which then moves with the ligand COM (positions only), so it is always in the frame of the
+// next step.  MULTISTEP = false is the plain step and ignores msp / msv / first_row.
+template <bool MULTISTEP>
 __global__ void __launch_bounds__(128)
 ddpm_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_lig, float* __restrict__ x_kp,
                  const float* __restrict__ eps_x, const float* __restrict__ eps_h, int F,
                  const float* __restrict__ coef, const int* __restrict__ step_ptr,
-                 const float* noise_x, const float* noise_h, uint64_t seed, const RunParams* rp) {
+                 const float* noise_x, const float* noise_h, uint64_t seed, const RunParams* rp,
+                 const MultistepParams* msp, MultistepParams msv, int first_row) {
     const int c = blockIdx.x;
     const int l0 = b.lig_ptr[c], nl = b.lig_ptr[c + 1] - l0;
     const int k0 = b.kp_ptr[c], nk = b.kp_ptr[c + 1] - k0;
@@ -26,30 +34,60 @@ ddpm_step_kernel(kpd_batch b, float* __restrict__ x_lig, float* __restrict__ h_l
     const StepDraws d = step_draws(rp, noise_x, seed, s, 1, 0, (size_t)b.n_lig * (3 + F));
     if (rp) noise_h = d.noise ? d.noise + (size_t)b.n_lig * 3 : nullptr;   // a run's slot holds x, then h
     __shared__ float com[3];
+    MultistepParams m{};
+    float mc = 0.0f, ma = 1.0f, ms = 0.0f;
+    bool corr = false;
+    if constexpr (MULTISTEP) {
+        m = msp ? *msp : msv;
+        mc = m.ms_coef[4 * s]; ma = m.ms_coef[4 * s + 1]; ms = m.ms_coef[4 * s + 2];
+        corr = s != (rp ? rp->T - 1 : first_row);
+    }
     // mu = z/alpha_t|s - var_terms*eps ; z_s = mu + sigma*noise   (ligand_diffuser.py:522-533)
     for (int i = threadIdx.x; i < nl * 3; i += blockDim.x) {
         const int idx = 3 * l0 + i;
         const float nz = d.noise ? d.noise[idx] : philox_normal(d.seed, s, d.atom_offset + l0 + i / 3, i % 3);
-        const float mu = __fsub_rn(__fdiv_rn(x_lig[idx], a), __fmul_rn(vt, eps_x[idx]));
-        x_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
+        if constexpr (MULTISTEP) {
+            const float z = x_lig[idx], e = eps_x[idx];
+            const float zs = __fadd_rn(__fsub_rn(__fdiv_rn(z, a), __fmul_rn(vt, e)), __fmul_rn(sg, nz));
+            const float xh = __fdiv_rn(__fsub_rn(z, __fmul_rn(ms, e)), ma);
+            x_lig[idx] = corr ? __fadd_rn(zs, __fmul_rn(mc, __fsub_rn(xh, m.hist_x[idx]))) : zs;
+            m.hist_x[idx] = xh;
+        } else {
+            const float mu = __fsub_rn(__fdiv_rn(x_lig[idx], a), __fmul_rn(vt, eps_x[idx]));
+            x_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
+        }
     }
     for (int i = threadIdx.x; i < nl * F; i += blockDim.x) {
         const int idx = F * l0 + i;
         const float nz = noise_h ? noise_h[idx] : philox_normal(d.seed, s, d.atom_offset + l0 + i / F, 3 + i % F);
-        const float mu = __fsub_rn(__fdiv_rn(h_lig[idx], a), __fmul_rn(vt, eps_h[idx]));
-        h_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
+        if constexpr (MULTISTEP) {
+            const float z = h_lig[idx], e = eps_h[idx];
+            const float zs = __fadd_rn(__fsub_rn(__fdiv_rn(z, a), __fmul_rn(vt, e)), __fmul_rn(sg, nz));
+            const float hh = __fdiv_rn(__fsub_rn(z, __fmul_rn(ms, e)), ma);
+            h_lig[idx] = corr ? __fadd_rn(zs, __fmul_rn(mc, __fsub_rn(hh, m.hist_h[idx]))) : zs;
+            m.hist_h[idx] = hh;
+        } else {
+            const float mu = __fsub_rn(__fdiv_rn(h_lig[idx], a), __fmul_rn(vt, eps_h[idx]));
+            h_lig[idx] = __fadd_rn(mu, __fmul_rn(sg, nz));
+        }
     }
     __syncthreads();
     remove_ligand_com(x_lig, x_kp, l0, nl, k0, nk, com);   // :536 -> :185-203
+    if constexpr (MULTISTEP) sub3(m.hist_x, l0, nl, com);
 }
 
 int launch_ddpm_step(const kpd_batch* b, float* x_lig, float* h_lig, float* x_kp, const float* eps_x,
                      const float* eps_h, int F, const float* coef, const int* step_ptr, const float* noise_x,
-                     const float* noise_h, uint64_t seed, const RunParams* rp, cudaStream_t st) {
+                     const float* noise_h, uint64_t seed, const RunParams* rp, cudaStream_t st,
+                     const MultistepParams* msp, const MultistepParams* msv, int first_row) {
     prof_begin(PROF_STEP, st);
-    ddpm_step_kernel<<<b->B, 128, 0, st>>>(*b, x_lig, h_lig, x_kp, eps_x, eps_h, F, coef, step_ptr, noise_x,
-                                           noise_h, seed, rp);
-    const int rc = check_launch("ddpm_step_kernel");
+    if (msp || msv)
+        ddpm_step_kernel<true><<<b->B, 128, 0, st>>>(*b, x_lig, h_lig, x_kp, eps_x, eps_h, F, coef, step_ptr, noise_x,
+                                                     noise_h, seed, rp, msp, msv ? *msv : MultistepParams{}, first_row);
+    else
+        ddpm_step_kernel<false><<<b->B, 128, 0, st>>>(*b, x_lig, h_lig, x_kp, eps_x, eps_h, F, coef, step_ptr, noise_x,
+                                                      noise_h, seed, rp, nullptr, MultistepParams{}, 0);
+    const int rc = check_launch(msp || msv ? "ddpm_step_kernel<multistep>" : "ddpm_step_kernel");
     prof_end(PROF_STEP, st);
     return rc;
 }
@@ -157,6 +195,21 @@ extern "C" int kpd_ddpm_step(const kpd_batch* batch, float* x_lig, float* h_lig,
     KPD_REQUIRE((noise_x == nullptr) == (noise_h == nullptr), "kpd_ddpm_step: give both noise tensors or neither");
     return launch_ddpm_step(batch, x_lig, h_lig, x_kp, eps_x, eps_h, atom_nf, coef, step_ptr, noise_x, noise_h, seed,
                             nullptr, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int kpd_ddpm_multistep_step(const kpd_batch* batch, float* x_lig, float* h_lig, float* x_kp,
+                                       const float* eps_x, const float* eps_h, int32_t atom_nf, const float* coef,
+                                       const float* ms_coef, const int32_t* step_ptr, int32_t first_row, float* hist_x,
+                                       float* hist_h, const float* noise_x, const float* noise_h, uint64_t seed,
+                                       void* stream) {
+    KPD_REQUIRE(batch && x_lig && h_lig && x_kp && eps_x && eps_h && coef && ms_coef && step_ptr && hist_x && hist_h,
+                "kpd_ddpm_multistep_step: null argument");
+    KPD_REQUIRE((noise_x == nullptr) == (noise_h == nullptr),
+                "kpd_ddpm_multistep_step: give both noise tensors or neither");
+    KPD_REQUIRE(first_row >= 0, "kpd_ddpm_multistep_step: first_row must be >= 0");
+    const MultistepParams msv{ms_coef, hist_x, hist_h};
+    return launch_ddpm_step(batch, x_lig, h_lig, x_kp, eps_x, eps_h, atom_nf, coef, step_ptr, noise_x, noise_h, seed,
+                            nullptr, static_cast<cudaStream_t>(stream), nullptr, &msv, first_row);
 }
 
 extern "C" int kpd_remove_com(const kpd_batch* batch, float* x_lig, float* x_kp, int32_t which, float* com_out,

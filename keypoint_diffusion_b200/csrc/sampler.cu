@@ -17,6 +17,8 @@
 // A recording sampler (kpd_sampler_enable_recording) adds record_frame_kernel after the step's first denoiser pass:
 //     step_prologue -> graph_mark/scan/fill -> denoiser -> record_frame -> ddpm_step
 // and the kernel picks its frame slot from the device step counter, so the same graphs serve any stride or buffers.
+// A multistep sampler (kpd_sampler_enable_multistep) captures the DPM-Solver++(2M) instantiation of the step kernel in
+// place of the plain one (same launch count); its rows and history buffers are re-pointed per run like the recording's.
 #include "common.cuh"
 #include <string.h>
 
@@ -61,6 +63,10 @@ struct kpd_sampler {
     RecordParams rec;         // host copy; x_frames == NULL records nothing.  Every run uploads it
     RecordParams* rec_dev;
     int rec_frames, rec_rows;
+    // DPM-Solver++(2M) (kpd_sampler_enable_multistep): ms_dev == NULL = the plain step kernel
+    MultistepParams ms;       // host copy; every run uploads it
+    MultistepParams* ms_dev;
+    int ms_rows;
 };
 
 static int64_t model_ws_bytes(const kpd_sampler_config* cfg, const void* model, const kpd_batch* b, int cap_ll,
@@ -152,7 +158,7 @@ static int enqueue_step(kpd_sampler* s, cudaStream_t st) {
     KPD_TRY(enqueue_denoiser(s, st));
     KPD_TRY(enqueue_record(s, st));
     KPD_TRY(launch_ddpm_step(&s->batch, s->x_lig, s->h_lig, s->x_kp, s->eps_x, s->eps_h, s->cfg.atom_nf, s->coef_run,
-                             s->step, nullptr, nullptr, 0, s->rp, st));
+                             s->step, nullptr, nullptr, 0, s->rp, st, s->ms_dev));
     return 0;
 }
 
@@ -202,6 +208,7 @@ extern "C" void kpd_sampler_destroy(kpd_sampler* s) {
     if (s->exec) cudaGraphExecDestroy(s->exec);
     if (s->frag_dev) cudaFree(s->frag_dev);
     if (s->rec_dev) cudaFree(s->rec_dev);
+    if (s->ms_dev) cudaFree(s->ms_dev);
     if (s->graph) cudaGraphDestroy(s->graph);
     if (s->ev_in) cudaEventDestroy(s->ev_in);
     if (s->ev_out) cudaEventDestroy(s->ev_out);
@@ -237,6 +244,7 @@ extern "C" int kpd_sampler_set_atom_offset(kpd_sampler* s, int32_t first_atom) {
 extern "C" int kpd_sampler_enable_inpainting(kpd_sampler* s, int32_t resamplings, const float* coef2) {
     KPD_REQUIRE(s && coef2 && resamplings >= 1, "kpd_sampler_enable_inpainting: bad argument");
     KPD_REQUIRE(!s->exec && !s->resamplings, "kpd_sampler_enable_inpainting: the sampler has already run or is inpainting");
+    KPD_REQUIRE(!s->ms_dev, "kpd_sampler_enable_inpainting: a multistep sampler cannot inpaint");
     KPD_REQUIRE(sizeof(float) * 3 * (size_t)s->batch.max_lig <= 48 * 1024,
                 "kpd_sampler_enable_inpainting: %d atoms in one complex exceed the supported 4096", s->batch.max_lig);
     const cudaError_t e = cudaMalloc(&s->frag_dev, sizeof(InpaintParams));
@@ -305,6 +313,25 @@ extern "C" int kpd_sampler_set_recording(kpd_sampler* s, int32_t every, int32_t 
     return 0;
 }
 
+extern "C" int kpd_sampler_enable_multistep(kpd_sampler* s) {
+    KPD_REQUIRE(s, "kpd_sampler_enable_multistep: null sampler");
+    KPD_REQUIRE(!s->exec && !s->ms_dev, "kpd_sampler_enable_multistep: the sampler has already run or is multistep");
+    KPD_REQUIRE(!s->resamplings, "kpd_sampler_enable_multistep: an inpainting sampler cannot run multistep steps");
+    const cudaError_t e = cudaMalloc(&s->ms_dev, sizeof(MultistepParams));
+    KPD_REQUIRE(e == cudaSuccess, "kpd_sampler_enable_multistep: %s", cudaGetErrorString(e));
+    s->ms = MultistepParams{nullptr, nullptr, nullptr};
+    return 0;
+}
+
+extern "C" int kpd_sampler_set_multistep(kpd_sampler* s, int32_t n_rows, const float* ms_coef, float* hist_x,
+                                         float* hist_h) {
+    KPD_REQUIRE(s && s->ms_dev, "kpd_sampler_set_multistep: not a multistep sampler");
+    KPD_REQUIRE(ms_coef && hist_x && hist_h && n_rows >= 1, "kpd_sampler_set_multistep: bad argument");
+    s->ms = MultistepParams{ms_coef, hist_x, hist_h};
+    s->ms_rows = n_rows;
+    return 0;
+}
+
 static int enqueue_any_step(kpd_sampler* s, cudaStream_t st) {
     return s->resamplings ? enqueue_inpaint_step(s, st) : enqueue_step(s, st);
 }
@@ -343,6 +370,10 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
                 (n_steps + s->rec.every - 1) / s->rec.every + 1, s->rec_frames);
     KPD_REQUIRE(!s->rec.x_frames || s->rec_rows == rows,
                 "kpd_sampler_run: %d prediction rows for a schedule of %d rows", s->rec_rows, rows);
+    // what keeps the multistep step kernel inside its rows: row s < rows of the active schedule
+    KPD_REQUIRE(!s->ms_dev || s->ms.ms_coef, "kpd_sampler_run: a multistep sampler needs kpd_sampler_set_multistep");
+    KPD_REQUIRE(!s->ms_dev || s->ms_rows == rows, "kpd_sampler_run: %d multistep rows for a schedule of %d rows",
+                s->ms_rows, rows);
     const kpd_batch& b = s->batch;
     const int F = s->cfg.atom_nf;
     cudaStream_t user = static_cast<cudaStream_t>(stream), st = s->stream;
@@ -368,6 +399,7 @@ extern "C" int kpd_sampler_run(kpd_sampler* s, float* x_kp, const float* h_kp, c
         CU(cudaMemcpyAsync(s->frag_dev, &frag, sizeof(InpaintParams), cudaMemcpyHostToDevice, st));
     }
     if (s->rec_dev) CU(cudaMemcpyAsync(s->rec_dev, &s->rec, sizeof(RecordParams), cudaMemcpyHostToDevice, st));
+    if (s->ms_dev) CU(cudaMemcpyAsync(s->ms_dev, &s->ms, sizeof(MultistepParams), cudaMemcpyHostToDevice, st));
 
     // frame setup (ligand_diffuser.py:348-370)
     KPD_TRY(launch_com(&b, s->x_lig, s->x_kp, 1, 0, s->init_kp_com, st));                // init_kp_com (:348)

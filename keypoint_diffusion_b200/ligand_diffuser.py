@@ -19,9 +19,9 @@ from . import hetero, ops
 from .dynamics import LigRecDynamics, LigRecDynamicsGVP
 from .n_nodes_dist import LigandSizeDistribution
 from .receptor_encoder import ReceptorEncoder, ReceptorEncoderGVP
-from .schedule import (PredefinedNoiseSchedule, alpha, coefficient_rows, coefficient_table, frame_levels, inpaint_rows,
-                       inpaint_table, prediction_rows, prediction_table, sigma, sigma_and_alpha_t_given_s,
-                       start_coefficients, step_grid)
+from .schedule import (SOLVERS, PredefinedNoiseSchedule, alpha, coefficient_rows, coefficient_table, frame_levels,
+                       inpaint_rows, inpaint_table, multistep_rows, prediction_rows, prediction_table, sigma,
+                       sigma_and_alpha_t_given_s, start_coefficients, step_grid)
 from .utils import get_batch_idxs, split_bounds
 
 DEFAULT_SUB_BATCHES = {"gvp": 4, "egnn": 2}      # measured on B200: profiles/r01_sweep_sub_batches_*.txt
@@ -156,19 +156,24 @@ class KeypointDiffusion(nn.Module):
 
     MAX_CACHED_SCHEDULES = 8
 
-    def schedule_tables(self, device, t_start: int, n: int, eta: Optional[float] = None, inpaint: bool = False):
+    def schedule_tables(self, device, t_start: int, n: int, eta: Optional[float] = None, inpaint: bool = False,
+                        solver: Optional[str] = None):
         """(coef [n,4], coef2 [n,4] or None, pred [n,2]) on `device`: the rows of the n-step grid over [0, t_start]
         (schedule.step_grid), ancestral (eta=None) or DDIM(eta) (schedule.coefficient_rows), with inpaint=True the
         fragment rows over the same grid (schedule.inpaint_rows), and the (alpha_t, sigma_t) rows a recorded trajectory
-        reads (schedule.prediction_rows).  n scalar rows cost milliseconds on the host; the last few schedules are
-        cached (per device and gamma version), least recently used evicted first."""
+        reads (schedule.prediction_rows).  solver="dpmpp_2m" (eta must be None): coef holds the DDIM eta = 0 rows, and
+        a fourth element, ms [n,4], the DPM-Solver++(2M) rows (schedule.multistep_rows).  n scalar rows cost
+        milliseconds on the host; the last few schedules are cached (per device and gamma version), least recently
+        used evicted first."""
         key = (str(device), self.gamma.gamma._version, self.gamma.gamma.data_ptr(), int(t_start), int(n),
-               None if eta is None else float(eta), bool(inpaint))
+               None if eta is None else float(eta), bool(inpaint), solver)
         hit = self._schedules.pop(key, None)
         if hit is None:
             grid, T, g = step_grid(t_start, n), self.n_timesteps, self.gamma.gamma
-            hit = (coefficient_rows(g, T, grid, eta).to(device), inpaint_rows(g, T, grid).to(device) if inpaint else None,
-                   prediction_rows(g, T, grid).to(device))
+            hit = (coefficient_rows(g, T, grid, 0.0 if solver else eta).to(device),
+                   inpaint_rows(g, T, grid).to(device) if inpaint else None, prediction_rows(g, T, grid).to(device))
+            if solver:
+                hit = hit + (multistep_rows(g, T, grid).to(device),)
             while len(self._schedules) >= self.MAX_CACHED_SCHEDULES:
                 self._schedules.pop(next(iter(self._schedules)))
         self._schedules[key] = hit
@@ -277,12 +282,12 @@ class KeypointDiffusion(nn.Module):
         return max(1, min(DEFAULT_SUB_BATCHES[self.architecture], n_complexes // 16))
 
     def _capacity_sampler(self, instance: int, plan: "ops.CapacityPlan", device, steps_per_graph, use_cuda_graph,
-                          resamplings: int = 0, record: bool = False):
+                          resamplings: int = 0, record: bool = False, multistep: bool = False):
         """The captured loop of capacity bucket plan.key (created on first use, then shared by every batch that lands in
         the bucket -- whatever its per-complex sizes, pockets or kk graph).  Groups of one call that run concurrently
         and share a bucket take distinct instances 0, 1, ... of it.  resamplings >= 1: the inpainting loop with that
-        many passes per step; record=True: the recording loop (visualize=True).  Both are cached apart from the plain
-        loop: their captured sequences differ."""
+        many passes per step; record=True: the recording loop (visualize=True); multistep=True: the DPM-Solver++(2M)
+        loop (solver="dpmpp_2m").  All are cached apart from the plain loop: their captured sequences differ."""
         model = self.dynamics.device_model(device)
         key = ("cap", instance, plan.key, self.dynamics._st.model_key, steps_per_graph, use_cuda_graph,
                getattr(model, "precision", "fp32"), self.n_timesteps)
@@ -290,6 +295,8 @@ class KeypointDiffusion(nn.Module):
             key = key + ("inpaint", int(resamplings))
         if record:
             key = key + ("record",)
+        if multistep:
+            key = key + ("multistep",)
         hit = self._cache_get(key)
         if hit is None:
             kp_width = self.n_kp_feat
@@ -299,7 +306,7 @@ class KeypointDiffusion(nn.Module):
                                       use_cuda_graph=use_cuda_graph,
                                       lig_feat_norm_constant=float(self.lig_feat_norm_constant), resamplings=resamplings,
                                       inpaint_coef=self.inpaint_coef_table(device) if resamplings else None,
-                                      record=record)
+                                      record=record, multistep=multistep)
             self._samplers[key] = hit
             object.__setattr__(self, "cold_captures", self.cold_captures + 1)
         return hit
@@ -313,7 +320,7 @@ class KeypointDiffusion(nn.Module):
                                       resamplings: int = 1, start_pos: torch.Tensor = None,
                                       start_feat: torch.Tensor = None, start_step: Optional[int] = None,
                                       timesteps: Optional[int] = None, eta: Optional[float] = None,
-                                      frame_every: Optional[int] = None):
+                                      frame_every: Optional[int] = None, solver: Optional[str] = None):
         """Returns (lig_pos, lig_feat): one CPU tensor per complex, as the reference does (:342-469).  ``g`` may live
         on the CPU (pinned or not): its keypoint tensors are uploaded here, straight into the sampler's buffers -- the
         host->device boundary of the path (reference test.py:152-161).
@@ -353,7 +360,14 @@ class KeypointDiffusion(nn.Module):
         ``'features'`` [m+1, n_atoms, F] (frame j < m: the state before executed step j*frame_every; frame m: the
         returned ligand), ``'pred_positions'`` [m, n_atoms, 3] and ``'pred_features'`` [m, n_atoms, F] (the denoiser's
         clean-ligand estimate (z - sigma_t eps) / alpha_t at frame j).  Every frame is in the frame and feature space the
-        ligands are returned in.  Recording does not change the ligands; capacity path only."""
+        ligands are returned in.  Recording does not change the ligands; capacity path only.
+
+        Second-order multistep sampling (DESIGN.md section 6.5): ``solver="dpmpp_2m"`` runs DPM-Solver++(2M) steps on the
+        grid of ``timesteps`` (all t_start rows without it): each step is the DDIM eta = 0 step plus a correction from
+        the previous step's clean-ligand estimate, more accurate than DDIM at the same step count (10-25 steps is where
+        it pays; pass steps_per_graph <= timesteps so that those steps replay a captured graph).  Composes with start
+        ligands, sub-batches and visualize=True (the prediction frames are the estimates the solver uses).  ValueError
+        with eta, a fragment, capacity=False or start_step = 0.  solver=None (default) is the run without it."""
         n_lig_total = int(g.num_nodes('lig'))
         inpaint = self._check_fragment_args(n_lig_total, fixed_mask, fixed_pos, fixed_feat, resamplings)
         start = self._check_start_args(n_lig_total, start_pos, start_feat, start_step)
@@ -364,7 +378,7 @@ class KeypointDiffusion(nn.Module):
         if start and init_lig_pos is not None:
             raise ValueError("init_lig_pos is not used with a start ligand (the start ligands' means set the frame)")
         t_start = int(start_step) if start else self.n_timesteps
-        n_sched = self._check_schedule_args(timesteps, eta, t_start, capacity)
+        n_sched = self._check_schedule_args(timesteps, eta, t_start, capacity, solver, inpaint)
         every = self._check_visualize_args(visualize, frame_every, capacity)
         dev = torch.device("cuda", torch.cuda.current_device()) if g.device.type != "cuda" else g.device
         batch_size = g.batch_size
@@ -381,7 +395,7 @@ class KeypointDiffusion(nn.Module):
             init_pos = hetero.readout_nodes(g, feat='x_0', op='mean', ntype='rec')
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())      # follows torch.manual_seed like the reference
-        sched = None if n_sched is None else self.schedule_tables(dev, t_start, n_sched, eta, inpaint)
+        sched = None if n_sched is None else self.schedule_tables(dev, t_start, n_sched, eta, inpaint, solver)
         pred = None
         if visualize:
             pred = self.prediction_coef_table(dev) if sched is None else sched[2]
@@ -423,7 +437,8 @@ class KeypointDiffusion(nn.Module):
             inst = taken.get(plan.key, 0)
             taken[plan.key] = inst + 1
             smp = self._capacity_sampler(inst, plan, dev, steps_per_graph, use_cuda_graph,
-                                         resamplings=int(resamplings) if inpaint else 0, record=visualize)
+                                         resamplings=int(resamplings) if inpaint else 0, record=visualize,
+                                         multistep=solver is not None)
             frag = None
             if inpaint:
                 l1 = lig_ptr[b]
@@ -441,7 +456,8 @@ class KeypointDiffusion(nn.Module):
                 out = smp.run(plan, kp['x_0'][k0:k1], kp['h_0'][k0:k1], kv[k0:k1] if kv is not None else None, gs, gd,
                               init_pos[a:b], seed=seed, atom_offset=l0, noise=noise, decode=decode, fragment=frag,
                               start=st_rows, schedule=None if sched is None else sched[:2],
-                              record_every=every if visualize else None, pred_coef=pred)
+                              record_every=every if visualize else None, pred_coef=pred,
+                              multistep=None if solver is None else sched[3])
             if n_sub > 1:
                 for t in out:
                     for v in (t.values() if isinstance(t, dict) else (t,)):
@@ -473,9 +489,9 @@ class KeypointDiffusion(nn.Module):
             res = res + (list(torch.split(atom_type.cpu(), lig_n)),)
         return res + (frames,) if visualize else res
 
-    def _check_schedule_args(self, timesteps, eta, t_start: int, capacity) -> Optional[int]:
-        """ValueError for a bad fewer-step request (host-side checks, before any device work); the step count of the
-        schedule to run, or None for the default tables."""
+    def _check_schedule_args(self, timesteps, eta, t_start: int, capacity, solver=None, fragment=False) -> Optional[int]:
+        """ValueError for a bad fewer-step or solver request (host-side checks, before any device work); the step count
+        of the schedule to run, or None for the default tables."""
         if timesteps is not None:
             if isinstance(timesteps, bool) or not isinstance(timesteps, numbers.Integral):
                 raise ValueError(f"timesteps must be an int, got {timesteps!r}")
@@ -488,7 +504,18 @@ class KeypointDiffusion(nn.Module):
             raise ValueError(f"eta must be a finite number in [0, 1], got {eta!r}")
         if (timesteps is not None or eta is not None) and not capacity:
             raise ValueError("fewer-step sampling runs on the capacity path only (capacity=True)")
-        if (timesteps is None and eta is None) or t_start == 0:
+        if solver is not None:
+            if not isinstance(solver, str) or solver not in SOLVERS:
+                raise ValueError(f"solver must be None or one of {SOLVERS}, got {solver!r}")
+            if eta is not None:
+                raise ValueError(f"solver={solver!r} takes no eta (its steps are built on the eta = 0 rows)")
+            if fragment:
+                raise ValueError(f"solver={solver!r} does not combine with a fragment (re-noising breaks its history)")
+            if not capacity:
+                raise ValueError(f"solver={solver!r} runs on the capacity path only (capacity=True)")
+            if t_start == 0:
+                raise ValueError(f"solver={solver!r} needs start_step > 0 (no reverse step runs at start_step = 0)")
+        if (timesteps is None and eta is None and solver is None) or t_start == 0:
             return None
         return t_start if timesteps is None else int(timesteps)
 
@@ -694,8 +721,8 @@ class KeypointDiffusion(nn.Module):
         ligand requested for that receptor (each of size m) is a variant of its start ligand, noised to level t0 and
         denoised from there (ligand optimisation, see sample_from_encoded_receptors); with fragments too, the fragment
         is the start ligand's first atoms and stays pinned.
-        timesteps / eta (passed on to sample_from_encoded_receptors, like every other keyword): fewer-step sampling,
-        checked here before any receptor is encoded.
+        timesteps / eta / solver (passed on to sample_from_encoded_receptors, like every other keyword): fewer-step and
+        multistep sampling, checked here before any receptor is encoded.
         visualize / frame_every: trajectories (see sample_from_encoded_receptors); every receptor's dict then also
         holds ``'frames'``, one trajectory dict per ligand.  Not with ``complexes`` (sample_sharded).
 
@@ -704,7 +731,8 @@ class KeypointDiffusion(nn.Module):
         has_start = self._check_start_ligands(start_ligands, start_step, n_lig_atoms, init_lig_pos, use_ref_lig_com,
                                               sampler_kw)
         self._check_schedule_args(sampler_kw.get("timesteps"), sampler_kw.get("eta"),
-                                  int(start_step) if has_start else self.n_timesteps, sampler_kw.get("capacity", True))
+                                  int(start_step) if has_start else self.n_timesteps, sampler_kw.get("capacity", True),
+                                  sampler_kw.get("solver"), has_fragment)
         self._check_visualize_args(visualize, sampler_kw.get("frame_every"), sampler_kw.get("capacity", True))
         if visualize and complexes is not None:
             raise ValueError("visualize=True is not supported by sample_sharded")

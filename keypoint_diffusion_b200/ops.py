@@ -407,6 +407,18 @@ def ddpm_step(batch: DeviceBatch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, step: 
           "kpd_ddpm_step")
 
 
+def ddpm_multistep_step(batch: DeviceBatch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, ms_coef, step: torch.Tensor,
+                        first_row: int, hist_x, hist_h, noise_x=None, noise_h=None, seed=0):
+    """In-place DPM-Solver++(2M) reverse step (kpd_ddpm_multistep_step, DESIGN.md section 6.5): the DDIM eta = 0 row of
+    coef, plus c (x^ - hist) with row `step` of ms_coef (schedule.multistep_rows) unless step == first_row; hist_x /
+    hist_h then hold x^, its positions moved with the ligand COM."""
+    _require_cuda(x_lig, h_lig, x_kp, eps_x, eps_h, coef, ms_coef, step, hist_x, hist_h, noise_x, noise_h)
+    check(lib.kpd_ddpm_multistep_step(C.byref(batch.c), ptr(x_lig), ptr(h_lig), ptr(x_kp), ptr(eps_x), ptr(eps_h),
+                                      h_lig.shape[1], ptr(coef), ptr(ms_coef), ptr(step), int(first_row), ptr(hist_x),
+                                      ptr(hist_h), ptr(noise_x), ptr(noise_h), int(seed), _stream()),
+          "kpd_ddpm_multistep_step")
+
+
 def ddpm_inpaint_step(batch: DeviceBatch, x_lig, h_lig, x_kp, eps_x, eps_h, coef, coef2, step: torch.Tensor, u: int,
                       fixed_mask, x_fix, h_fix, init_kp_com, lig_feat_norm_constant=1.0, noise=None, seed=0):
     """In-place fragment-conditioned reverse step, pass u (kpd_ddpm_inpaint_step): the posterior step with the atoms of
@@ -470,18 +482,24 @@ class Sampler:
     pinned, and a captured graph holds steps_per_graph // resamplings steps.  0 (default) = the plain loop.
     Either kind runs from a given ligand after set_start (ligand optimisation by partial noising), and with fewer,
     strided or DDIM steps after set_schedule; neither captures again.  record=True makes it a recording sampler: its
-    captured step holds one more launch, and run(record_every=k) returns the trajectory (DESIGN.md section 6.4)."""
+    captured step holds one more launch, and run(record_every=k) returns the trajectory (DESIGN.md section 6.4).
+    multistep=True makes it a DPM-Solver++(2M) sampler (DESIGN.md section 6.5; not with resamplings): its captured step
+    runs the multistep step kernel, which carries the previous step's clean-ligand estimate in a history the sampler
+    allocates for its layout; every run needs DDIM eta = 0 rows (set_schedule) and their set_multistep rows."""
 
     def __init__(self, model: _Model, batch: DeviceBatch, gp: GraphParams, kk: Optional[Csr], coef: torch.Tensor,
                  T: int, atom_nf: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
                  lig_feat_norm_constant: float = 1.0, atom_offset: int = 0, caps: Optional[Tuple[int, int]] = None,
-                 resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None, record: bool = False):
+                 resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None, record: bool = False,
+                 multistep: bool = False):
         self.model, self.batch, self.gp, self.kk, self.coef = model, batch, gp, kk, coef
         _require_cuda(coef)
         self.T, self.atom_nf = int(T), int(atom_nf)
         self.resamplings = int(resamplings)
         if self.resamplings < 0 or (self.resamplings > 0) != (inpaint_coef is not None):
             raise ValueError("an inpainting sampler needs resamplings >= 1 and inpaint_coef; a plain one neither")
+        if multistep and self.resamplings:
+            raise ValueError("a multistep sampler cannot inpaint (resamplings must be 0)")
         self.has_lk = bool(model.update_kp_feat if model.arch == 0 else model.update_kp)
         if self.resamplings:        # about as many graph nodes per captured graph as the plain loop
             steps_per_graph = max(1, int(steps_per_graph) // self.resamplings)
@@ -512,6 +530,26 @@ class Sampler:
         self.record = bool(record)
         if self.record:
             check(lib.kpd_sampler_enable_recording(self.handle), "kpd_sampler_enable_recording")
+        self.multistep = bool(multistep)
+        self._ms_coef = None
+        if self.multistep:
+            check(lib.kpd_sampler_enable_multistep(self.handle), "kpd_sampler_enable_multistep")
+            self.hist_x = torch.empty(batch.n_lig, 3, dtype=torch.float32, device=batch.device)
+            self.hist_h = torch.empty(batch.n_lig, self.atom_nf, dtype=torch.float32, device=batch.device)
+
+    def set_multistep(self, ms_coef: torch.Tensor):
+        """The DPM-Solver++(2M) rows of the next runs (multistep samplers only; kpd_sampler_set_multistep): ms_coef fp32
+        [n,4] on the device, schedule.multistep_rows over the grid of the active schedule, which must hold the DDIM
+        eta = 0 rows of that grid (n == schedule_rows, checked by the run).  The tensor must stay alive and in place
+        while runs use it (only its address is kept)."""
+        if not self.multistep:
+            raise ValueError("set_multistep needs a multistep sampler (multistep=True)")
+        _require_cuda(ms_coef)
+        assert ms_coef.dtype == torch.float32 and ms_coef.is_contiguous() and ms_coef.dim() == 2
+        assert ms_coef.shape[1] == 4
+        check(lib.kpd_sampler_set_multistep(self.handle, int(ms_coef.shape[0]), ptr(ms_coef), ptr(self.hist_x),
+                                            ptr(self.hist_h)), "kpd_sampler_set_multistep")
+        self._ms_coef = ms_coef
 
     def set_fragment(self, fixed_mask: Optional[torch.Tensor], x_fix: Optional[torch.Tensor],
                      h_fix: Optional[torch.Tensor]):
@@ -751,12 +789,14 @@ class CapacitySampler:
     resamplings >= 1 (and inpaint_coef) it is an inpainting sampler that also owns zero-filled fragment buffers sized at
     capacity: run(fragment=...) fills the rows of the real atoms; filler complexes and atoms are never fixed.  Likewise
     it owns start-ligand buffers at capacity for run(start=...); filler rows stay zero and filler outputs are dropped.
-    record=True: a recording sampler (see Sampler); run(record_every=...) returns the frames of the real atoms."""
+    record=True: a recording sampler (see Sampler); run(record_every=...) returns the frames of the real atoms.
+    multistep=True: a DPM-Solver++(2M) sampler (see Sampler) whose history is sized at capacity; run(multistep=...) takes
+    the rows of each run."""
 
     def __init__(self, model: _Model, plan: CapacityPlan, gp: GraphParams, coef: torch.Tensor, T: int, atom_nf: int,
                  kp_width: int, v_width: int, steps_per_graph: int = 50, use_cuda_graph: bool = True,
                  lig_feat_norm_constant: float = 1.0, resamplings: int = 0, inpaint_coef: Optional[torch.Tensor] = None,
-                 record: bool = False):
+                 record: bool = False, multistep: bool = False):
         B, N, K, max_lig, max_kp, cap_ll, cap_kl, cap_kk = plan.key
         dev = model.device
         self.key, self.model, self.atom_nf, self.T = plan.key, model, int(atom_nf), int(T)
@@ -770,7 +810,7 @@ class CapacitySampler:
         self.sampler = Sampler(model, self.batch, gp, self.kk, coef, T, atom_nf, steps_per_graph=steps_per_graph,
                                use_cuda_graph=use_cuda_graph, lig_feat_norm_constant=lig_feat_norm_constant,
                                caps=(cap_ll, cap_kl), resamplings=resamplings, inpaint_coef=inpaint_coef,
-                               record=record)
+                               record=record, multistep=multistep)
         if self.sampler.resamplings:
             self.fixed_mask = torch.zeros(N, dtype=torch.uint8, device=dev)
             self.x_fix = torch.zeros(N, 3, dtype=torch.float32, device=dev)
@@ -783,7 +823,7 @@ class CapacitySampler:
     def run(self, plan: CapacityPlan, x_kp, h_kp, v_kp, kk_src, kk_dst, init_pos, seed: int, atom_offset: int = 0,
             noise: Optional[torch.Tensor] = None, decode: bool = False, fragment: Optional[Tuple] = None,
             start: Optional[Tuple] = None, schedule: Optional[Tuple] = None, record_every: Optional[int] = None,
-            pred_coef: Optional[torch.Tensor] = None):
+            pred_coef: Optional[torch.Tensor] = None, multistep: Optional[torch.Tensor] = None):
         """x_kp/h_kp/v_kp: the REAL keypoint rows (host or device tensors; pinned host tensors are uploaded straight
         into the capacity buffers); kk_src/kk_dst: kk edges in this batch's own keypoint numbering; init_pos [B_real,3].
         fragment (inpainting samplers): (fixed_mask [N_real] bool, x_fix [N_real,3], h_fix [N_real,F]) or None.
@@ -792,13 +832,16 @@ class CapacitySampler:
         schedule: (coef [n,4], coef2 [n,4] or None) on the device -- run the n rows of that schedule (see
         Sampler.set_schedule; t0 of start then counts its rows) -- or None for the create-time tables.  A run-time
         value like the start: no new capture.  record_every / pred_coef (recording samplers): see Sampler.run; pred_coef
-        has the rows of the schedule run.
+        has the rows of the schedule run.  multistep (multistep samplers, required there): ms_coef [n,4] on the device,
+        schedule.multistep_rows over the grid of `schedule`, whose coef must be its DDIM eta = 0 rows.
         -> (x_lig [N_real,3], h_lig [N_real,F], x_kp [K_real,3][, atom_type int32 [N_real]][, frames]) on the device,
         frames holding the real atoms only ([m+1, N_real, .] and [m, N_real, .])."""
         if plan.key != self.key:
             raise ValueError("CapacitySampler.run: the plan belongs to another capacity bucket")
         if fragment is not None and not self.sampler.resamplings:
             raise ValueError("CapacitySampler.run: a fragment needs an inpainting sampler")
+        if (multistep is not None) != self.sampler.multistep:
+            raise ValueError("CapacitySampler.run: multistep rows go with a multistep sampler, and only there")
         B_r, N_r, K_r = plan.n_real, plan.n_lig_real, plan.n_kp_real
         self.batch.set_layout(plan.lig_n, plan.kp_n)
         if self.sampler.resamplings:     # rows past the real atoms stay zero: fillers are never fixed
@@ -816,6 +859,8 @@ class CapacitySampler:
         else:
             self.sampler.set_start(None)
         self.sampler.set_schedule(*(schedule or ()))
+        if multistep is not None:
+            self.sampler.set_multistep(multistep)
         self.x_kp[:K_r].copy_(x_kp, non_blocking=True)
         self.h_kp[:K_r].copy_(h_kp, non_blocking=True)
         if self.v_kp is not None:

@@ -9,7 +9,8 @@ inpaint_table [T,4] = (alpha_s, sigma_s, alpha_t|s, sigma_t|s) is the second tab
 fragment-conditioned sampling reads (DESIGN.md section 6.1); start_coefficients gives (alpha_t0, sigma_t0), the
 forward noising of a start ligand in ligand optimisation (section 6.2).  Both tables are the unit-step case of
 coefficient_rows / inpaint_rows over a step grid (step_grid), which also give the strided ancestral and DDIM rows of
-fewer-step sampling (section 6.3).  prediction_rows and frame_levels serve recorded trajectories (section 6.4).
+fewer-step sampling (section 6.3).  prediction_rows and frame_levels serve recorded trajectories (section 6.4);
+multistep_rows the second-order DPM-Solver++(2M) steps (section 6.5).
 """
 import numpy as np
 import torch
@@ -165,6 +166,37 @@ def prediction_rows(gamma: torch.Tensor, T: int, grid) -> torch.Tensor:
 def prediction_table(gamma: torch.Tensor, T: int) -> torch.Tensor:
     """fp32 [T,2] on the CPU: prediction_rows over the unit grid (row s: t = s+1)."""
     return prediction_rows(gamma, T, list(range(T + 1)))
+
+
+SOLVERS = ("dpmpp_2m",)
+
+
+def multistep_rows(gamma: torch.Tensor, T: int, grid) -> torch.Tensor:
+    """fp32 [n,4] on the CPU over a step grid; row k = (c_k, alpha_t, sigma_t, 0) with t = tau_{k+1}: the second-order
+    correction z_s += c_k (x^_k - x^_prev) of a DPM-Solver++(2M) run on top of the DDIM eta = 0 row k (DESIGN.md section
+    6.5), and the level its clean-ligand estimate x^_k = (z - sigma_t eps) / alpha_t divides by.  Columns 1-2 are
+    prediction_rows' bit for bit.  With h_k = (gamma[tau_{k+1}] - gamma[tau_k]) / 2, the log-SNR step of row k,
+        c_k = alpha_{tau_k} (-expm1(-h_k)) h_k / (2 h_{k+1})
+    evaluated in fp64 from the fp32 gammas and rounded once to fp32, like _ddim_columns.  c is 0 on the top row k = n-1
+    (no history) and on row 0 (the large log-SNR jump into tau_0 = 0, where a second-order correction does harm)."""
+    g = gamma.detach().float().cpu()
+    n = len(grid) - 1
+    gam, rows = [], []
+    for s_int, t_int in zip(grid[:-1], grid[1:]):
+        gs, gt, _ = _row_gammas(g, T, s_int, t_int)
+        gam.append((float(gs[0]), float(gt[0])))
+        rows.append([alpha(gt)[0], sigma(gt)[0]])
+    out = torch.zeros(n, 4, dtype=torch.float32)
+    for k in range(n):
+        out[k, 1], out[k, 2] = rows[k]
+        if 1 <= k <= n - 2:
+            gs, gt = gam[k]
+            h = 0.5 * (torch.tensor(gt, dtype=torch.float64) - torch.tensor(gs, dtype=torch.float64))
+            h_prev = 0.5 * (torch.tensor(gam[k + 1][1], dtype=torch.float64) - torch.tensor(gam[k + 1][0],
+                                                                                              dtype=torch.float64))
+            a_s = torch.sqrt(torch.sigmoid(-torch.tensor(gs, dtype=torch.float64)))
+            out[k, 0] = (a_s * -torch.expm1(-h) * h / (2 * h_prev)).float()
+    return out.contiguous()
 
 
 def frame_levels(grid, n: int, every: int) -> torch.Tensor:

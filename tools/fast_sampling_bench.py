@@ -11,6 +11,13 @@ Prints one JSON line per workload (and writes them to --out), with cold_captures
 variants) and the card's name and power limit read in the same run.
 
     python tools/fast_sampling_bench.py --out profiles/r06_fast_sampling_bench.jsonl
+
+--solvers times the second-order solver instead (DESIGN.md section 6.5): DDIM eta = 0 (ddim0_n) and DPM-Solver++(2M)
+(2m_n) calls at timesteps = 10, 20, 25, 50 and 100 with steps_per_graph 50, and at 10 and 20 with steps_per_graph = n
+(suffix _spg), the two solvers alternating in one loop.  It also reports, for information only, the RMS distance of each
+call's positions to a 1000-step DDIM eta = 0 call from the same seed (seeded random weights: not a sample-quality claim).
+
+    python tools/fast_sampling_bench.py --solvers --out profiles/r09_multistep_bench.jsonl
 """
 import argparse
 import json
@@ -82,12 +89,68 @@ def run_workload(name, steps, warmup):
     return res
 
 
+SOLVER_STEPS = (10, 20, 25, 50, 100)
+
+
+def _timed(call, steps, warmup):
+    for _ in range(warmup):
+        call()
+    torch.cuda.synchronize()
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    ev0.record()
+    for _ in range(steps):
+        call()
+    ev1.record()
+    torch.cuda.synchronize()
+    return ev0.elapsed_time(ev1) / steps
+
+
+def run_solver_sweep(name, steps, warmup):
+    from keypoint_diffusion_b200 import HeteroBatch, synthetic
+    wl = bench.WORKLOADS[name]
+    dev = torch.device("cuda:0")
+    cfg = bench.load_config(wl["cfg"], dense_ll=True)
+    arch = cfg["diffusion"].get("architecture", "egnn")
+    model = bench.build_model(cfg, dev)
+    model.dynamics.set_precision("bf16x3")
+    F = model.n_lig_features
+    pocket = bench.make_pocket(synthetic, wl, 0, cfg, arch)
+    B, n_at = wl["ligands"], wl["atoms"]
+    g = HeteroBatch.from_pockets([pocket], [n_at] * B, F, pin=True)
+    init = torch.zeros(B, 3).pin_memory()
+    variants = {}
+    for n in SOLVER_STEPS:
+        variants[f"ddim0_{n}"] = dict(timesteps=n, eta=0.0, steps_per_graph=STEPS_PER_GRAPH)
+        variants[f"2m_{n}"] = dict(timesteps=n, solver="dpmpp_2m", steps_per_graph=STEPS_PER_GRAPH)
+    for n in (10, 20):
+        variants[f"ddim0_{n}_spg"] = dict(timesteps=n, eta=0.0, steps_per_graph=n)
+        variants[f"2m_{n}_spg"] = dict(timesteps=n, solver="dpmpp_2m", steps_per_graph=n)
+
+    def call(kw):
+        return model.sample_from_encoded_receptors(g, init_lig_pos=init, seed=1234, return_device_tensors=True, **kw)
+    ref, _ = call(dict(timesteps=1000, eta=0.0, steps_per_graph=STEPS_PER_GRAPH))
+    ref = ref.clone()
+    res = {"workload": f"{name}: {B} ligands x {n_at} atoms, 1 pocket ({wl['n_kp']} keypoints), dense ll, bf16x3, "
+                       f"seeded random weights; ddim0_n = n DDIM eta 0 steps, 2m_n = n DPM-Solver++(2M) steps, "
+                       f"steps_per_graph {STEPS_PER_GRAPH} (_spg: steps_per_graph = n)", "ms_per_call": {},
+           "ligands_per_s": {}, "pos_rms_to_ddim1000": {}}
+    for tag, kw in variants.items():
+        ms = _timed(lambda: call(kw), steps, warmup)
+        x, _ = call(kw)
+        res["ms_per_call"][tag] = round(ms, 2)
+        res["ligands_per_s"][tag] = round(B / (ms / 1e3), 2)
+        res["pos_rms_to_ddim1000"][tag] = round(float((x - ref).pow(2).sum(1).mean().sqrt()), 4)
+    res["cold_captures"] = model.cold_captures
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--workloads", nargs="+", default=["gvp_20kp", "egnn_20kp"], choices=["gvp_20kp", "egnn_20kp"])
     ap.add_argument("--steps", type=int, default=5, help="timed calls per variant")
     ap.add_argument("--warmup", type=int, default=1, help="untimed calls per variant (the first one captures)")
     ap.add_argument("--out", default=None, help="also write the JSON lines to this file")
+    ap.add_argument("--solvers", action="store_true", help="time DDIM eta = 0 against DPM-Solver++(2M) instead")
     args = ap.parse_args()
     if args.steps < 1 or args.warmup < 1:
         ap.error("--steps and --warmup must be >= 1 (the warm-up call captures the graphs)")
@@ -97,7 +160,7 @@ def main():
         raise SystemExit("fast_sampling_bench.py needs a CUDA device")
     lines = []
     for name in args.workloads:
-        r = run_workload(name, args.steps, args.warmup)
+        r = (run_solver_sweep if args.solvers else run_workload)(name, args.steps, args.warmup)
         r.update(card())
         r["steps"], r["warmup"] = args.steps, args.warmup
         lines.append(json.dumps(r))
